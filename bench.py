@@ -1,6 +1,9 @@
 """bench.py -- images/sec of TPDM adaptive sampling, SD3-medium 1024^2 (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config2|config3|config4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config2|config3|config4] [--dump-outputs DIR]
+
+The bench loads the library that build() (python -m tpdm_b200.build) left in tpdm_b200/; it compiles nothing and writes
+nothing under the repository, which may be read-only where it runs.
 
 Default workload (config2, the one the metric is quoted on): a "step" is one full adaptive trajectory for one prompt (MMDiT
 forward with CFG at every denoising step, TimePredictor head, schedule update, Euler update) on synthetic text embeddings
@@ -28,6 +31,11 @@ value = all images / max-over-ranks device time.
   that is EXECUTED, not extrapolated: `blocks_per_sample` consecutive joint blocks of the running denoising step (plus the
   step's embedders / norm_out / proj_out / TimePredictor / Euler when the slice holds them); consecutive steps continue the
   same denoising step, so K samples are K * blocks_per_sample / 24 complete denoising steps.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the timed path returned in its last step as DIR/<name>.npy
+  (config2: the output of the last trajectory; config3: of the last drain; config4: scores, advantages and the TimePredictor
+  parameters after the last update).  Inputs and weights are seeded, so two builds run with the same arguments can be
+  compared output for output.
 """
 from __future__ import annotations
 
@@ -165,13 +173,31 @@ class Dist:
         return out
 
 
-def build_model(local_rank, world, sample_size=128):
-    from tpdm_b200 import build as _build
+DUMP_BYTES = 60 * 10**6      # the .npy headers stay within 64 MB as well
 
-    if local_rank == 0:
-        _build.build()      # no-op when tpdm_b200/libtpdm_b200.so is newer than its sources; the CUDA library is the only path
-    if world > 1:
-        torch.distributed.barrier()
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each tensor as out_dir/<name>.npy, float64 as float64 and every other dtype as float32.  When the arrays exceed
+    DUMP_BYTES together, each one is cut to its share of that budget: a sample of its flattened elements at fixed, seeded
+    positions, the same from run to run."""
+    import numpy as np
+
+    arrays = {k: v.detach().cpu().to(torch.float64 if v.dtype == torch.float64 else torch.float32) for k, v in arrays.items()}
+    total = sum(t.numel() * t.element_size() for t in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        keep = max(1, t.numel() * DUMP_BYTES // total) if total > DUMP_BYTES else t.numel()
+        if keep < t.numel():
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t.flatten()[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+
+
+def tensors_of(out) -> dict:
+    return {k: v for k, v in out.items() if torch.is_tensor(v)}
+
+
+def build_model(local_rank, world, sample_size=128):
     from tpdm_b200 import _lib as L
     from tpdm_b200.modeling_sd3_pnt import SD3_MEDIUM_TRANSFORMER_CONFIG, SD3PredictNextTimeStepModel
 
@@ -225,6 +251,7 @@ def run_ours(args, rank, world, local_rank):
     D.barrier()
     ms_value = D.max(e0.elapsed_time(e1))
     launches = int(lib.tpdm_launch_count(0))
+    timed_out = out
 
     # ---- per-kernel sample: one more trajectory of the same workload with CUDA-event brackets around every GEMM / attention
     # / LayerNorm / adaLN launch (kept out of region 1: ~250 extra event records per denoising step perturb it by a few %)
@@ -275,6 +302,8 @@ def run_ours(args, rank, world, local_rank):
 
     if rank != 0:
         return None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, tensors_of(timed_out))
     eager = torch_eager_bf16_step(dev) if world == 1 else None
     pk = peaks()
     steps_per_image = n_denoise / K
@@ -595,6 +624,8 @@ def run_config3(args, rank, world, local_rank):
     ms_step1 = e0.elapsed_time(e1) / o1.sigmas.shape[1]
     if rank != 0:
         return None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, tensors_of(out))
     st = steps.tolist()
     assert all(s > 0 for s in st), "a prompt was not processed"
     assert sum(mine) == P, "a prompt was processed twice"
@@ -693,6 +724,8 @@ def run_config4(args, rank, world, local_rank):
                  f"parameters bit-identical on all ranks after {K + W} updates")
     if rank != 0:
         return None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(scores=last["scores"], advantages=last["advantages"], tpm_params=trainer.params))
     rollouts = prompts * rloo_k
     return {
         "metric": "rollouts/sec/box, SD3-M 512^2 RLOO update (BASELINE configs[3])", "value": world * K * rollouts / (ms / 1e3), "unit": "rollouts/s",
@@ -719,11 +752,15 @@ def main():
     ap.add_argument("--slots", type=int, default=2, help="config3: prompts in flight per GPU")
     ap.add_argument("--prompts-per-gpu", type=int, default=8, help="config3")
     ap.add_argument("--schedule", default="fifo", choices=["fifo", "lpt"], help="config3: ticket order (lpt: longest expected trajectory first)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, at most 64 MB in all)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = {"config2": 8, "config3": 2, "config4": 2}[args.workload]
     rank, world, local_rank = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the CUDA path; --impl reference has none")
         line = run_reference(args, rank, world)
         if line is not None:
             print(json.dumps(line), flush=True)
