@@ -358,11 +358,11 @@ int tpdm_gemm_bf16(const void* A, const void* W, const float* bias, const float*
                    int N, int K, int epi, void* stream);
 /* qkv bf16 [Bt][S][3*H*dp] -> out bf16 [Bt][S][H*dp] */
 int tpdm_joint_attention(const void* qkv, void* out, int Bt, int S, int H, int dp, int head_dim, int q_rows, void* stream);
-/* Diagnostic (synchronises the device): how many 128-row query tiles of the LAST attention launch the fast kernel handed to the
- * exact kernel (scores more than ~2^64 above everything their row had seen before); -1 when only the exact kernel ran
- * (TPDM_ATTN_EXACT=1).  0 on ordinary activations: the exact pass then costs one empty launch. */
+/* Diagnostic (synchronises the device): how many 128-row query tiles of the LAST attention launch were recomputed with the exact
+ * softmax (scores more than ~2^64 above everything their row had seen before); -1 when the launch had no flag buffer (its
+ * allocation failed).  0 on ordinary activations. */
 int tpdm_attention_redo_count(void);
-/* the same, summed over every attention launch since the library was loaded (exact-only mode: 0) */
+/* the same, summed over every attention launch since the library was loaded */
 long long tpdm_attention_redo_total(void);
 /* conv3x3 pad 1 over NHWC bf16 x [batch][g][g][C], w bf16 [N][9][C] -> out fp32 [batch][g*g][N] */
 int tpdm_conv3x3_nhwc(const void* x, const void* w, const float* bias, float* out, int batch, int g, int C, int N,

@@ -1,7 +1,6 @@
-"""Timeline of ONE attention CTA from the instrumented build (python -m tpdm_b200.build --variant trace TPDM_ATTN_TRACE,TPDM_ATTN_SPLIT=0
--- the per-tile stamps of the softmax warp live in the four-softmax-warp fast path and in the exact path (TPDM_ATTN_TRACE=2);
-the CTA-level stamps and the MMA-issuer stamps also work with the default eight-warp build):
-clock64() stamps of softmax warp 4 and of the two MMA-issuing warps, per 128-key tile.  Run on the GPU box:
+"""Timeline of ONE attention CTA from the instrumented build (python -m tpdm_b200.build --variant trace TPDM_ATTN_TRACE):
+clock64() stamps of softmax warp 4 (keys [0,64) of every tile) and of the two MMA-issuing warps, per 128-key tile, plus CTA-level
+stamps of an early and a late CTA.  Run on the GPU box:
     TPDM_B200_LIB=tpdm_b200/_build/libtpdm_trace.so python tools/attn_trace.py"""
 import ctypes as C
 import os
@@ -24,9 +23,7 @@ lib.tpdm_attn_trace_read.argtypes = [C.POINTER(C.c_longlong), C.c_int]
 assert lib.tpdm_attn_trace_read(buf, 3 * 2048) == 0
 sm, qk, pv = ([buf[r * 2048 + i] for i in range(2048)] for r in range(3))
 n_kv = (S + 127) // 128
-names = (["guard + wait s_full", "ld chunks 0-1", "chunk 0 (pv_done wait, st)", "chunk 1 + p_full[0] + s_free", "chunks 2-3 + p_full[1]"]
-         if os.environ.get("TPDM_ATTN_EXACT") != "1" else
-         ["wait s_full", "ld chunk 0", "max + chunk 0 (pv_done wait, st)", "chunks 1-2 (+ p_full half 0)", "chunk 3 + p_full"])
+names = ["wait s_full", "checkpoint + ld chunks 0-1", "chunk 0 (pv_done wait, st)", "chunk 1 + s_free", "chunks 2-3 + p_full"]
 print("softmax warp 4 of one CTA, cycles per phase of a 128-key tile (period = top(j+1) - top(j))")
 tot = [0.0] * 6
 cnt = 0
@@ -42,11 +39,6 @@ for j in range(4, n_kv - 2):
     if 10 <= j < 16:
         print(f"  j={j:3d}: " + "  ".join(f"{names[k]}={ph[k]:4d}" for k in range(5)) + f"  | period={ph[5]}")
 print("mean over", cnt, "tiles: " + "  ".join(f"{names[k]}={tot[k] / cnt:6.1f}" for k in range(5)) + f"  | period={tot[5] / cnt:.1f}")
-sub = [(sm[8 * j + 6] - sm[8 * j + 2], sm[8 * j + 7] - sm[8 * j + 6], sm[8 * j + 3] - sm[8 * j + 7]) for j in range(4, n_kv - 2)
-       if sm[8 * j + 2] and sm[8 * j + 6] and sm[8 * j + 7] and sm[8 * j + 3]]
-if sub:
-    m = [sum(x[k] for x in sub) / len(sub) for k in range(3)]
-    print(f"inside 'max + chunk 0': max of chunk 0 + vote {m[0]:.0f}, exponentials up to the end of the pv_done wait {m[1]:.0f}, P store + next load + vote {m[2]:.0f}")
 for role, name, arr in ((1, "QK issuer", qk), (2, "PV issuer", pv)):
     w = s_ = c = 0.0
     for j in range(4, n_kv - 2):

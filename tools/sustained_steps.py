@@ -53,6 +53,6 @@ stop[0] = True
 ms = e0.elapsed_time(e1)
 clk = sorted(s[0] for s in samples)
 pw = sorted(s[1] for s in samples)
-print(f"{os.environ.get('TPDM_B200_LIB', 'product')}{' exact-only' if os.environ.get('TPDM_ATTN_EXACT') == '1' else ''}: {images} images, {steps} steps, "
+print(f"{os.environ.get('TPDM_B200_LIB', 'product')}: {images} images, {steps} steps, "
       f"{ms / steps:.3f} ms per denoising step, {images / ms * 1e3:.3f} images/s; median SM clock {clk[len(clk) // 2]:.0f} MHz, "
       f"median power {pw[len(pw) // 2]:.0f} W; attention CTAs that took the exact pass: {_L.load().tpdm_attention_redo_total()}", flush=True)

@@ -6,15 +6,16 @@
 // [Bt][S][3*H*dp] through 4-D TMA tensor maps (no head permute, no concat copy); O is written token-major [Bt][S][H*dp]
 // so the output projection consumes it as-is.
 //
-// One CTA = one 128-row query tile of one (batch, head); 256 threads (384 in the default fast kernel: warps 8-11 are four more softmax
-// warps on the same rows); two CTAs co-resident per SM (dp = 64).
+// One CTA = one 128-row query tile of one (batch, head); 384 threads; two CTAs co-resident per SM (dp = 64).
 //   warp 0      TMA producer  (Q once, K/V tiles of 128 keys through a 2-stage smem ring)
 //   warp 1      MMA issuer for S = Q K^T: one 128 x 128 score tile per K tile (SS, dp/16 instructions of N = 128)
 //   warp 3      MMA issuer for O += P V (A = P from TMEM, B = V MN-major from smem, 8 instructions of N = dp)
 //   warp 2      TMEM allocator
-//   warps 4-7   softmax, one thread per query row.
+//   warps 4-11  softmax, two threads per query row: warps 4-7 take keys [0,64) of every tile, warps 8-11 keys [64,128) of the same
+//               rows (a warp reaches the TMEM lanes 32 * (warp % 4) ..., so the pairs (4,8), (5,9), ... share rows).  Four softmax
+//               warps per scheduler: with two the kernel was bound by the latency of each warp's own instruction stream.
 // TMEM per CTA: S 128 fp32 columns, P 64 columns (128 keys of packed bf16), O dp columns -- ONE buffer each.  Overlap inside a
-// CTA comes from releasing S as soon as its last 32-column chunk is in registers (Q K^T of the next tile then runs under the
+// CTA comes from releasing S as soon as its last chunk is in registers (Q K^T of the next tile then runs under the
 // last quarter of this tile's exponentials and under P V), overlap on the SM from the second co-resident CTA.
 //
 // Why 128-key tiles (round 2; measurements in profiles/r02_*.txt):
@@ -29,19 +30,19 @@
 //  * tools/microbench/tmem_read_rate.cu: tcgen05.ld moves 490-1050 B/clk/SM, so reading S back in fp32 is NOT a floor (round 1
 //    assumed 64 B/clk/SM); the floor of this kernel is the MUFU: 16 ex2 / clk / SM = 1024 cycles per 128 x 128 scores.
 // Softmax: fp32, exp2 with log2(e)/sqrt(d) folded into one FFMA2, in two flavours (attn_cta<DP, kFast>):
-//  * FAST (what joint_attention_fast_kernel runs first).  No maximum inside the key loop: the reference m_ref only has to keep
+//  * FAST (what every CTA runs first, on warps 4-11).  No maximum inside the key loop: the reference m_ref only has to keep
 //    exp2(s - m_ref) inside the fp32 / bf16 exponent range.  It starts as the row maximum of the first key tile and is guarded by
-//    the ROW SUM the loop computes anyway: at the top of a tile, l > 2^32 moves it up by floor(log2 l) (O and l rescaled by that
-//    power of two; no P of the new tile exists yet).  A row the guard cannot keep in range (l > 2^64, inf, NaN, or an argument
-//    > 127 reaching the polynomial, which would wrap instead of overflowing) flags the CTA.
-//  * EXACT (a flagged CTA reruns its tile with it before it exits; TPDM_ATTN_EXACT=1 runs it alone).  Reference maximum m_used raised
-//    lazily: every 32-column chunk computes its own maximum (FMNMX3 trees, issued under the MUFU work of the previous chunk) and
-//    only when that exceeds m_used by more than 2^kRescaleThreshold does the row take the (rare, exact) path that moves the
-//    reference and rescales what was accumulated under the old one -- O, l and the P chunks of this tile already stored.
-// fp32 sums and bf16 P carry 8 exponent bits, so running up to 2^32 above the reference costs no precision, and the final 1/l cancels
-// the reference.  Round-2 measurements (B200, S = 4429, H = 24, Bt = 2): exact 320-327 us, fast 288-292 us with four softmax warps per
-// CTA and 276 us with eight (TPDM_ATTN_SPLIT=1, the default: two threads per row, see the split branch of attn_cta); cuDNN SDPA: 283 us;
-// everything tried on the way is in profiles/r02_attention_experiments.txt.
+//    the ROW SUM the loop computes anyway, at a checkpoint every 4th tile: a half whose partial sum has passed 2^24 proposes a
+//    shift by floor(log2 l) through shared memory, and both halves of the row apply it at the next checkpoint (O and l rescaled
+//    by that power of two; see `tile` in the fast branch of attn_cta).  A row the guard cannot keep in range (l > 2^64, inf, NaN,
+//    or an argument > 127 reaching the polynomial, which would wrap instead of overflowing) flags the CTA.
+//  * EXACT (a flagged CTA reruns its tile with it on warps 4-7 before it exits).  Reference maximum m_used raised lazily: every
+//    32-column chunk computes its own maximum (FMNMX3 trees, issued under the MUFU work of the previous chunk) and only when that
+//    exceeds m_used by more than 2^kRescaleThreshold does the row take the (rare, exact) path that moves the reference and
+//    rescales what was accumulated under the old one -- O, l and the P chunks of this tile already stored.
+// fp32 sums and bf16 P carry 8 exponent bits, so running far above the reference costs no precision, and the final 1/l cancels
+// the reference.  Round-2 measurements (B200, S = 4429, H = 24, Bt = 2): exact 320-327 us, fast 276 us; cuDNN SDPA: 283 us;
+// everything tried on the way (four softmax warps per CTA: 288-292 us) is in profiles/r02_attention_experiments.txt.
 #include <cuda_bf16.h>
 
 #include <stdlib.h>
@@ -55,52 +56,30 @@ namespace tpdm {
 
 namespace {
 
-// Fast path experiment: 1 = EIGHT softmax warps per CTA (384 threads, 80 registers): warps 4-7 take keys [0,64) of every tile, warps
-// 8-11 keys [64,128) of the same rows (a warp reaches the TMEM lanes 32 * (warp % 4) ..., so the pairs (4,8), (5,9), ... share rows).
-// Four softmax warps per scheduler instead of two.  Both halves of a row must use ONE reference: every 4th tile a half whose partial
-// row sum has passed 2^24 proposes a shift through shared memory and both apply it at the next checkpoint (see `tile` in the split branch).  16-column chunks
-// (two buffers of 16 registers).
-#ifndef TPDM_ATTN_SPLIT
-#define TPDM_ATTN_SPLIT 1
-#endif
-constexpr int kAttnThreads = 256;
-constexpr bool kSplit = TPDM_ATTN_SPLIT != 0;
-constexpr int kFastThreads = kSplit ? 384 : 256;   // fast kernel: 4 control warps + 4 or 8 softmax warps
+constexpr int kFastThreads = 384;   // 4 control warps + 8 softmax warps (the exact redo pass uses softmax warps 4-7 only)
 constexpr int kQT = 128;   // query rows per CTA
 constexpr int kKT = 128;   // keys per K/V smem tile = keys per S tile
-constexpr int kChunk = 32; // S columns per tcgen05.ld
+constexpr int kChunk = 32; // S columns per tcgen05.ld of the exact softmax
 constexpr int kKVStages = 2;
 constexpr float kRescaleThreshold = 32.0f;  // log2 units
 // Every kPolyEvery-th pair of exponentials is computed on the FMA/ALU pipes (Cody-Waite range reduction + cubic minimax
-// polynomial, max relative error 7.5e-5 -- P is rounded to bf16 anyway) instead of MUFU.EX2; 0 disables the emulation.
-// Measured on B200 with this kernel (S = 4429, H = 24, Bt = 2; profiles/r02_attention_experiments.txt): 0 -> 343 us, every 8th ->
+// polynomial, max relative error 7.5e-5 -- P is rounded to bf16 anyway) instead of MUFU.EX2.
+// Measured on B200 with this kernel (S = 4429, H = 24, Bt = 2; profiles/r02_attention_experiments.txt): none -> 343 us, every 8th ->
 // 328 us, every 4th -> 324 us, every 2nd -> 325 us.  (Round 1's 64-key kernel was latency bound and got SLOWER with it.)
 // Packing P with integer adds + PRMT instead of F2FP (which shares the XU pipe with MUFU) was measured too: 358 us, rejected.
-#ifndef TPDM_POLY_EVERY
-#define TPDM_POLY_EVERY 4
-#endif
-constexpr int kPolyEvery = TPDM_POLY_EVERY;
-// Fast path, polynomial pairs: 0 = clamp the argument below and track its maximum (3 instructions per pair), 1 = only CHECK
-// |x| <= 126 with one FMNMX3 per pair and send the CTA to the exact pass otherwise.  Measured (profiles/r02_attention_experiments.txt):
-// 289.3 vs 291.1 us, 21.41 vs 21.44 ms per sustained denoising step -- no gain worth a performance cliff for rows that hold a
-// score 87 nats below their reference, so the clamp stays.
-#ifndef TPDM_ATTN_POLY_ABS
-#define TPDM_ATTN_POLY_ABS 0
-#endif
-// Fast path experiment: 1 = P is converted to bf16 by TRUNCATION (one PRMT per pair on the ALU pipe) instead of F2FP.BF16.PACK_AB,
-// which runs on the XU pipe next to MUFU.EX2, with the mean loss of 2^-10 / ln 2 per element (log-uniform mantissas) divided out of
-// the row sum in the epilogue.  Takes a quarter of the XU work away and gains 1.7 % (287.0 vs 292.0 us; 21.13 vs 21.21 ms per
-// sustained step) at a rel-L2 error of 2.78e-3 instead of 2.34e-3: the XU pipe is not the bound either, and the rounding stays.
-#ifndef TPDM_ATTN_TRUNC_P
-#define TPDM_ATTN_TRUNC_P 0
-#endif
-// -DTPDM_ATTN_TRACE: clock64() time stamps of one CTA's softmax warp 4 (role 0, 8 slots per key tile) and of the two MMA-issuing
-// warps (roles 1 and 2, 4 slots per key tile), read back with tpdm_attn_trace_read (tools/attn_trace.py).  Diagnostic builds only.
+constexpr int kPolyEvery = 4;
+// -DTPDM_ATTN_TRACE: clock64() time stamps of one CTA's fast pass: softmax warp 4 (role 0, 8 slots per key tile, STRACE) and the two
+// MMA-issuing warps (roles 1 and 2, 4 slots per key tile), read back with tpdm_attn_trace_read (tools/attn_trace.py).  Diagnostic
+// builds only.
 #ifdef TPDM_ATTN_TRACE
 __device__ long long g_attn_trace[3][2048];
 #define ATRACE(role, idx)                                                                       \
   do {                                                                                          \
     if (trace_on && lane == 0 && (idx) < 2048) g_attn_trace[role][idx] = clock64();             \
+  } while (0)
+#define STRACE(e)                                                                               \
+  do {                                                                                          \
+    if (warp == 4) ATRACE(0, 8 * j + (e));                                                      \
   } while (0)
 // CTA-level stamps of two CTAs (an early and a late one): [0] kernel entry, [1] past pdl_wait, [2] TMEM allocated, [3] first score
 // tile ready, [4] last tile's P handed over, [5] O stored, [6] exit; [7] = %globaltimer at entry, [8] at exit
@@ -111,6 +90,7 @@ __device__ long long g_cta_trace[2][16];
   } while (0)
 #else
 #define ATRACE(role, idx)
+#define STRACE(e)
 #define CTRACE(idx)
 #endif
 
@@ -149,8 +129,9 @@ struct AttnBars {
     tmem_slot = reinterpret_cast<uint32_t*>(pv_done + 1);
   }
   static constexpr int kCount = 1 + 4 * kKVStages + 5;
-  // one thread; `again`: the barriers carry the phases of a finished tile (persistent exact kernel) and are invalidated first
-  __device__ void init(bool again, uint32_t s_free_count = 4) const {
+  // one thread; `again`: the barriers carry the phases of a finished tile (before the exact redo pass) and are invalidated first;
+  // s_free completes with one arrival per softmax warp
+  __device__ void init(bool again, uint32_t s_free_count) const {
     if (again) {
       for (int i = 0; i < kCount; ++i) mbar_inval(q_full + i);
     }
@@ -175,6 +156,57 @@ __device__ __forceinline__ uint8_t* attn_smem_base() {
   return reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
 }
 
+// (p0, p1) = 2^(x0, x1) through MUFU.EX2, or with `poly` on the FMA/ALU pipes: 2^x = 2^n * 2^f, n = rint(x) read from the mantissa
+// of x + 1.5*2^23, f = x - n in [-0.5, 0.5].  Below -126 the clamp flushes the result to ~0; an argument above 127 would wrap the
+// exponent instead of overflowing, so the callers keep x <= kRescaleThreshold (exact softmax) or check it (fast softmax: pmax).
+// (An |x| check instead of the clamp was measured and rejected: profiles/r02_attention_experiments.txt.)
+__device__ __forceinline__ void exp2_pair(const float x0, const float x1, const bool poly, float& p0, float& p1) {
+  if (poly) {
+    const uint64_t magic2 = pack_f32x2(12582912.f, 12582912.f), nmagic2 = pack_f32x2(-12582912.f, -12582912.f);
+    const uint64_t mone2 = pack_f32x2(-1.f, -1.f);
+    const uint64_t c0 = pack_f32x2(0.9999280572f, 0.9999280572f), c1 = pack_f32x2(0.6932609677f, 0.6932609677f),
+                   c2 = pack_f32x2(0.2426111251f, 0.2426111251f), c3 = pack_f32x2(0.0551716499f, 0.0551716499f);
+    const uint64_t xp = pack_f32x2(fmaxf(x0, -126.f), fmaxf(x1, -126.f));
+    const uint64_t t = fadd2(xp, magic2);
+    const uint64_t fr = ffma2(fadd2(t, nmagic2), mone2, xp);
+    uint64_t pp = ffma2(c3, fr, c2);
+    pp = ffma2(pp, fr, c1);
+    pp = ffma2(pp, fr, c0);
+    float t0, t1;
+    unpack_f32x2(t, t0, t1);
+    unpack_f32x2(pp, p0, p1);
+    p0 = __int_as_float(__float_as_int(p0) + (__float_as_int(t0) << 23));
+    p1 = __int_as_float(__float_as_int(p1) + (__float_as_int(t1) << 23));
+  } else {
+    p0 = exp2_approx(x0);
+    p1 = exp2_approx(x1);
+  }
+}
+
+// Epilogue: kCols columns of O (TMEM, from o_tmem on) times inv_l, as bf16 to out[0, kCols) of a token-major row; the TMEM loads are
+// warp-wide, the stores only for rows < S (row_valid).
+template <int kCols>
+__device__ __forceinline__ void store_o(const uint32_t o_tmem, const float inv_l, __nv_bfloat16* out, const bool row_valid) {
+#pragma unroll
+  for (int c = 0; c < kCols / 32; ++c) {
+    uint32_t o[32];
+    tmem_ld_32x32(o_tmem + c * 32, o);
+    tmem_wait_ld();
+    if (row_valid) {
+      uint4* dst = reinterpret_cast<uint4*>(out + c * 32);
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        uint4 w;
+        w.x = pack_bf16x2(__uint_as_float(o[8 * e + 0]) * inv_l, __uint_as_float(o[8 * e + 1]) * inv_l);
+        w.y = pack_bf16x2(__uint_as_float(o[8 * e + 2]) * inv_l, __uint_as_float(o[8 * e + 3]) * inv_l);
+        w.z = pack_bf16x2(__uint_as_float(o[8 * e + 4]) * inv_l, __uint_as_float(o[8 * e + 5]) * inv_l);
+        w.w = pack_bf16x2(__uint_as_float(o[8 * e + 6]) * inv_l, __uint_as_float(o[8 * e + 7]) * inv_l);
+        dst[e] = w;
+      }
+    }
+  }
+}
+
 // One 128-row query tile (qt) of one (batch b, head h): the whole CTA, from initialised mbarriers and an allocated TMEM block to
 // the stores of O.  kFast selects the guarded softmax without per-chunk maxima (redo_smem: set when the tile must be recomputed exactly).
 template <int DP, bool kFast>
@@ -189,7 +221,8 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
   const int q0 = qt * kQT;
   const int n_kv = (A.S + kKT - 1) / kKT;
 #ifdef TPDM_ATTN_TRACE
-  const bool trace_on = kFast == (TPDM_ATTN_TRACE != 2) && qt == 5 && h == 3 && b == 0;
+  const int ctr = !kFast ? -1 : (qt == 5 && h == 3 && b == 0) ? 0 : (qt == 7 && h == 20 && b == 1) ? 1 : -1;   // see g_cta_trace
+  const bool trace_on = ctr == 0;
 #endif
   const uint32_t tmem_base = *B.tmem_slot;
 
@@ -279,8 +312,13 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
       __syncwarp();
     }
   }
-  } else if (kFast && kSplit) {
-    // ---------------------------------------------------------------- split fast softmax: warps 4-7 keys [0,64), warps 8-11 keys [64,128)
+  } else if (kFast) {
+    // ---------------------------------------------------------------- fast softmax: warps 4-7 keys [0,64), warps 8-11 keys [64,128)
+    // The reference m_ref only has to keep exp2(s - m_ref) inside the fp32 / bf16 exponent range; it does not have to be the maximum.
+    // It starts as the row maximum of the first key tile and is then guarded by the ROW SUM, which the loop computes anyway (see
+    // `tile`).  What the guard cannot repair -- a score more than ~2^64 above everything the row has seen (l > 2^64, inf or NaN at the
+    // next check; or an argument > 127 reaching the polynomial) -- sets this CTA's redo flag, and the CTA then runs its tile a second
+    // time with the exact softmax (per-chunk maxima, the branch below) before it exits.
     __shared__ float xch[2][kQT];
     __shared__ int bump[2][kQT];   // see `tile`: total reference shift (float bits, >= 0) in force from the tiles of one parity on
     const int q = warp & 3, half = (warp - 4) >> 2;
@@ -291,9 +329,9 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
     const int rowi = q * 32 + lane;
     const float scale = A.scale_log2;
     const uint64_t scale2 = pack_f32x2(scale, scale);
-    constexpr float kSoft = 4294967296.f, kHard = 1.8446744073709552e19f, kPolyMax = 127.f;
-    uint64_t la = pack_f32x2(0.f, 0.f), lb = pack_f32x2(0.f, 0.f);
-    float pmax = -INFINITY;
+    constexpr float kHard = 1.8446744073709552e19f, kPolyMax = 127.f;
+    uint64_t la = pack_f32x2(0.f, 0.f), lb = pack_f32x2(0.f, 0.f);   // this half's row sum as four partial sums
+    float pmax = -INFINITY;   // largest argument that went through the polynomial
     bool hard = false;
     float applied = 0.f;   // total shift applied to this thread's reference
     if (half == 0) {
@@ -328,33 +366,17 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
       m_ref = fmaxf(xch[0][rowi], xch[1][rowi]);
       asm volatile("bar.sync 1, 256;" ::: "memory");   // xch is reused for the row sums
     }
+    CTRACE(3);
     uint64_t negm2 = pack_f32x2(-m_ref, -m_ref);
+    // exponentials of one 16-column chunk, packed to bf16
     auto exp16 = [&](const uint32_t (&v)[16], uint32_t (&pk)[8]) {
-      const uint64_t magic2 = pack_f32x2(12582912.f, 12582912.f), nmagic2 = pack_f32x2(-12582912.f, -12582912.f);
-      const uint64_t mone2 = pack_f32x2(-1.f, -1.f);
-      const uint64_t c0 = pack_f32x2(0.9999280572f, 0.9999280572f), c1 = pack_f32x2(0.6932609677f, 0.6932609677f),
-                     c2 = pack_f32x2(0.2426111251f, 0.2426111251f), c3 = pack_f32x2(0.0551716499f, 0.0551716499f);
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
         float x0, x1, p0, p1;
         unpack_f32x2(ffma2(pack_f32x2(__uint_as_float(v[2 * i]), __uint_as_float(v[2 * i + 1])), scale2, negm2), x0, x1);
-        if (kPolyEvery > 0 && (i % (kPolyEvery > 0 ? kPolyEvery : 1)) == (kPolyEvery - 1)) {
-          pmax = fmax3(pmax, x0, x1);
-          const uint64_t xp = pack_f32x2(fmaxf(x0, -126.f), fmaxf(x1, -126.f));
-          const uint64_t t = fadd2(xp, magic2);
-          const uint64_t fr = ffma2(fadd2(t, nmagic2), mone2, xp);
-          uint64_t pp = ffma2(c3, fr, c2);
-          pp = ffma2(pp, fr, c1);
-          pp = ffma2(pp, fr, c0);
-          float t0, t1;
-          unpack_f32x2(t, t0, t1);
-          unpack_f32x2(pp, p0, p1);
-          p0 = __int_as_float(__float_as_int(p0) + (__float_as_int(t0) << 23));
-          p1 = __int_as_float(__float_as_int(p1) + (__float_as_int(t1) << 23));
-        } else {
-          p0 = exp2_approx(x0);
-          p1 = exp2_approx(x1);
-        }
+        const bool poly = i % kPolyEvery == kPolyEvery - 1;
+        if (poly) pmax = fmax3(pmax, x0, x1);
+        exp2_pair(x0, x1, poly, p0, p1);
         if (i & 1) lb = fadd2(lb, pack_f32x2(p0, p1));
         else la = fadd2(la, pack_f32x2(p0, p1));
         pk[i] = pack_bf16x2(p0, p1);
@@ -376,11 +398,14 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
       // passed 2^24, proposes applied + floor(log2 l) into slot (c + 1) & 1.  All of this sits BEHIND the wait for s_full(j): that
       // wait is ordered after every softmax warp's s_free arrivals of the earlier tiles, so the proposals of the last checkpoint
       // are visible and nobody still reads the slot that is written now.  A proposal takes effect 4 tiles later and up to 8 tiles
-      // after the sum started to grow: the 2^40 between the proposal threshold and the exact-pass threshold cover that.
+      // after the sum started to grow: the 2^40 between the proposal threshold and the exact-pass threshold cover that.  (A vote
+      // per tile between the two halves costs the whole gain of the second four warps.)
+      STRACE(0);
       hard = hard || pmax > kPolyMax;
       mbar_wait(s_full, j & 1);
       tc_fence_after();
-      if (warp == 4 && lane == 0) mbar_arrive(&k_empty[j % kKVStages]);
+      if (warp == 4 && lane == 0) mbar_arrive(&k_empty[j % kKVStages]);   // Q K(j)^T has completed: the K stage is free
+      STRACE(1);
       uint32_t va[16], vb[16], pk[8];
       tmem_ld_32x16(s_tmem, va);
       tmem_ld_32x16(s_tmem + 16, vb);
@@ -417,6 +442,7 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
         }
       }
       tmem_wait_ld();
+      STRACE(2);
       if (kMasked) {
         mask16(0, va, valid);
         mask16(1, vb, valid);
@@ -425,10 +451,11 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
       if (j > 0) {  // P is single-buffered: P(j-1) V must be done before P(j) lands
         mbar_wait(pv_done, (j - 1) & 1);
         tc_fence_after();
-        if (warp == 4 && lane == 0) mbar_arrive(&v_empty[(j - 1) % kKVStages]);
+        if (warp == 4 && lane == 0) mbar_arrive(&v_empty[(j - 1) % kKVStages]);   // ... and its V stage is free
       }
       tmem_st_32x8(p_tmem, pk);
       tmem_ld_32x16(s_tmem + 32, va);
+      STRACE(3);
       exp16(vb, pk);
       tmem_st_32x8(p_tmem + 8, pk);
       tmem_ld_32x16(s_tmem + 48, vb);
@@ -436,6 +463,7 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(s_free);   // this warp's half of S(j) is in registers (8 arrivals complete the phase)
+      STRACE(4);
       if (kMasked) {
         mask16(2, va, valid);
         mask16(3, vb, valid);
@@ -448,9 +476,11 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&p_full[half]);   // keys [0,64) from warps 4-7, keys [64,128) from warps 8-11: 4 arrivals each
+      STRACE(5);
     };
     for (int j = 0; j < n_kv - 1; ++j) tile(j, std::false_type{});
     tile(n_kv - 1, std::true_type{});
+    CTRACE(4);
     const float lh = row_sum();
     if (!(lh <= kHard) || pmax > kPolyMax) hard = true;
     if (hard) *redo_smem = 1;
@@ -460,27 +490,10 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
     mbar_wait(pv_done, (n_kv - 1) & 1);
     tc_fence_after();
     const int row = q0 + rowi;
-    __nv_bfloat16* out = A.out + (static_cast<long long>(b) * A.S + row) * (static_cast<long long>(A.H) * DP) + h * DP + half * (DP / 2);
-#pragma unroll
-    for (int c = 0; c < DP / 64; ++c) {
-      uint32_t o[32];
-      tmem_ld_32x32(o_tmem + c * 32, o);
-      tmem_wait_ld();
-      if (row < A.S) {
-        uint4* dst = reinterpret_cast<uint4*>(out + c * 32);
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          uint4 w;
-          w.x = pack_bf16x2(__uint_as_float(o[8 * e + 0]) * inv_l, __uint_as_float(o[8 * e + 1]) * inv_l);
-          w.y = pack_bf16x2(__uint_as_float(o[8 * e + 2]) * inv_l, __uint_as_float(o[8 * e + 3]) * inv_l);
-          w.z = pack_bf16x2(__uint_as_float(o[8 * e + 4]) * inv_l, __uint_as_float(o[8 * e + 5]) * inv_l);
-          w.w = pack_bf16x2(__uint_as_float(o[8 * e + 6]) * inv_l, __uint_as_float(o[8 * e + 7]) * inv_l);
-          dst[e] = w;
-        }
-      }
-    }
+    store_o<DP / 2>(o_tmem, inv_l,
+                    A.out + (static_cast<long long>(b) * A.S + row) * (static_cast<long long>(A.H) * DP) + h * DP + half * (DP / 2), row < A.S);
   } else if (warp < 8) {
-    // ---------------------------------------------------------------- softmax / correction / epilogue
+    // ---------------------------------------------------------------- exact softmax (the redo pass): warps 4-7, one thread per row
     const int q = warp & 3;
     const uint32_t lane_off = static_cast<uint32_t>(q * 32) << 16;
     const uint32_t s_tmem = tmem_base + lane_off + L::kSCol;
@@ -490,37 +503,16 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
     const uint64_t scale2 = pack_f32x2(scale, scale);
     float m_used = -INFINITY;            // reference max of the running sums (log2 domain); may lag the true max by 2^kRescaleThreshold
     uint64_t l2 = pack_f32x2(0.f, 0.f);  // row sum as two partial sums
-    float l = 0.f;                       // final row sum
 
-    // p = exp2(s * scale - m_used) for one half (16 columns) of a 32-column chunk, packed to bf16; accumulates the row sum
+    // p = exp2(s * scale - m_used) for one half (16 columns) of a 32-column chunk, packed to bf16; accumulates the row sum.
+    // x <= kRescaleThreshold by construction of m_used, so the polynomial pairs need no check.
     auto exp_half = [&](const uint32_t (&v)[32], uint32_t (&pk)[16], uint64_t negm2, const int half) {
-      const uint64_t magic2 = pack_f32x2(12582912.f, 12582912.f), nmagic2 = pack_f32x2(-12582912.f, -12582912.f);
-      const uint64_t mone2 = pack_f32x2(-1.f, -1.f);
-      const uint64_t c0 = pack_f32x2(0.9999280572f, 0.9999280572f), c1 = pack_f32x2(0.6932609677f, 0.6932609677f),
-                     c2 = pack_f32x2(0.2426111251f, 0.2426111251f), c3 = pack_f32x2(0.0551716499f, 0.0551716499f);
 #pragma unroll
       for (int ii = 0; ii < 8; ++ii) {
         const int i = half * 8 + ii;
         float x0, x1, p0, p1;
         unpack_f32x2(ffma2(pack_f32x2(__uint_as_float(v[2 * i]), __uint_as_float(v[2 * i + 1])), scale2, negm2), x0, x1);
-        if (kPolyEvery > 0 && (i % (kPolyEvery > 0 ? kPolyEvery : 1)) == (kPolyEvery - 1)) {
-          // 2^x = 2^n * 2^f, n = rint(x) read from the mantissa of x + 1.5*2^23, f = x - n in [-0.5, 0.5].  x <= kRescaleThreshold
-          // by construction of m_used (no wrap of the exponent on the high side); below -126 the clamp flushes the result to ~0.
-          const uint64_t xp = pack_f32x2(fmaxf(x0, -126.f), fmaxf(x1, -126.f));
-          const uint64_t t = fadd2(xp, magic2);
-          const uint64_t fr = ffma2(fadd2(t, nmagic2), mone2, xp);
-          uint64_t pp = ffma2(c3, fr, c2);
-          pp = ffma2(pp, fr, c1);
-          pp = ffma2(pp, fr, c0);
-          float t0, t1;
-          unpack_f32x2(t, t0, t1);
-          unpack_f32x2(pp, p0, p1);
-          p0 = __int_as_float(__float_as_int(p0) + (__float_as_int(t0) << 23));
-          p1 = __int_as_float(__float_as_int(p1) + (__float_as_int(t1) << 23));
-        } else {
-          p0 = exp2_approx(x0);
-          p1 = exp2_approx(x1);
-        }
+        exp2_pair(x0, x1, i % kPolyEvery == kPolyEvery - 1, p0, p1);
         l2 = fadd2(l2, pack_f32x2(p0, p1));
         pk[i] = pack_bf16x2(p0, p1);
       }
@@ -571,192 +563,11 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
       return fmax3(m0, fmax3(m2, __uint_as_float(v[23]), __uint_as_float(v[31])), m0) * scale;
     };
 
-#ifdef TPDM_ATTN_TRACE
-    const bool tr4 = trace_on && warp == 4;
-#define STRACE(e) do { if (tr4 && lane == 0 && 8 * j + (e) < 2048) g_attn_trace[0][8 * j + (e)] = clock64(); } while (0)
-#else
-#define STRACE(e)
-#endif
-    if constexpr (kFast) {
-      // ------------------------------------------------------------ fast path: no maximum inside the loop
-      // The reference m_ref only has to keep exp2(s - m_ref) inside the fp32 / bf16 exponent range; it does not have to be the
-      // maximum.  It starts as the row maximum of the first key tile and is then guarded by the ROW SUM, which the loop computes
-      // anyway: at the top of every tile, l > 2^32 moves the reference up by floor(log2 l) (O and l rescaled by the same power of
-      // two; nothing of the new tile exists yet and P(j-1) V has drained by then, so no P is ever touched).  One tile can add at
-      // most a factor 2^32 per element before the next check, far inside the range.  What the guard cannot repair -- a score more
-      // than ~2^64 above everything the row has seen (l > 2^64, inf or NaN at the next check; or an argument > 127 reaching the
-      // polynomial, which would wrap instead of overflowing) -- sets this CTA's redo flag, and the CTA then runs its tile a second time with the
-      // exact softmax (per-chunk maxima, the `else` branch below) before it exits.  Per 128 keys this removes 64 FMNMX3, four votes and the
-      // serial "load chunk 0 -> maximum -> vote" prefix of every tile from the softmax warps.
-      constexpr float kSoft = 4294967296.f, kHard = 1.8446744073709552e19f, kPolyMax = 126.f;
-      uint64_t la = pack_f32x2(0.f, 0.f), lb = pack_f32x2(0.f, 0.f);   // row sum as four partial sums
-      float pmax = -INFINITY;   // largest argument that went through the polynomial since the last guard
-      bool hard = false;
-      float m_ref;
-      mbar_wait(s_full, 0);
-      tc_fence_after();
-      {
-        const int valid0 = A.S < kKT ? A.S : kKT;
-        float mx = -INFINITY;
-#pragma unroll 1
-        for (int c = 0; c < kKT / kChunk; ++c) {
-          uint32_t v[32];
-          tmem_ld_32x32(s_tmem + c * kChunk, v);
-          tmem_wait_ld();
-          mask_chunk(c, v, valid0);
-          mx = fmaxf(mx, chunk_max(v));
-        }
-        m_ref = mx;
-      }
-#ifdef TPDM_ATTN_TRACE
-      if (threadIdx.x == 128) {
-        const int ctr2 = (qt == 5 && h == 3 && b == 0) ? 0 : (qt == 7 && h == 20 && b == 1) ? 1 : -1;
-        if (ctr2 >= 0) g_cta_trace[ctr2][3] = clock64();
-      }
-#endif
-      // exponentials of one 32-column chunk, packed to bf16
-      auto exp_chunk = [&](const uint32_t (&v)[32], uint32_t (&pk)[16], const uint64_t negm2, auto clamp_tag) {
-        constexpr bool kClamp = decltype(clamp_tag)::value || !TPDM_ATTN_POLY_ABS;   // the masked tail tile holds -inf scores
-        const uint64_t magic2 = pack_f32x2(12582912.f, 12582912.f), nmagic2 = pack_f32x2(-12582912.f, -12582912.f);
-        const uint64_t mone2 = pack_f32x2(-1.f, -1.f);
-        const uint64_t c0 = pack_f32x2(0.9999280572f, 0.9999280572f), c1 = pack_f32x2(0.6932609677f, 0.6932609677f),
-                       c2 = pack_f32x2(0.2426111251f, 0.2426111251f), c3 = pack_f32x2(0.0551716499f, 0.0551716499f);
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-          float x0, x1, p0, p1;
-          unpack_f32x2(ffma2(pack_f32x2(__uint_as_float(v[2 * i]), __uint_as_float(v[2 * i + 1])), scale2, negm2), x0, x1);
-          if (kPolyEvery > 0 && (i % (kPolyEvery > 0 ? kPolyEvery : 1)) == (kPolyEvery - 1)) {
-            // Unmasked tiles, no clamp: |x| <= 126 is CHECKED (one FMNMX3 with |.| modifiers per pair instead of two clamps and a
-            // maximum); an argument outside -- a score 87 nats below the reference, or one the row-sum guard could not keep in
-            // range -- flags the CTA for the exact pass.  The masked tail tile clamps (its -inf scores are legitimate).
-            pmax = kClamp ? fmax3(pmax, x0, x1) : fmax3(pmax, fabsf(x0), fabsf(x1));
-            const uint64_t xp = kClamp ? pack_f32x2(fmaxf(x0, -126.f), fmaxf(x1, -126.f)) : pack_f32x2(x0, x1);
-            const uint64_t t = fadd2(xp, magic2);
-            const uint64_t fr = ffma2(fadd2(t, nmagic2), mone2, xp);
-            uint64_t pp = ffma2(c3, fr, c2);
-            pp = ffma2(pp, fr, c1);
-            pp = ffma2(pp, fr, c0);
-            float t0, t1;
-            unpack_f32x2(t, t0, t1);
-            unpack_f32x2(pp, p0, p1);
-            p0 = __int_as_float(__float_as_int(p0) + (__float_as_int(t0) << 23));
-            p1 = __int_as_float(__float_as_int(p1) + (__float_as_int(t1) << 23));
-          } else {
-            p0 = exp2_approx(x0);
-            p1 = exp2_approx(x1);
-          }
-          if (i & 1) lb = fadd2(lb, pack_f32x2(p0, p1));
-          else la = fadd2(la, pack_f32x2(p0, p1));
-#if TPDM_ATTN_TRUNC_P
-          pk[i] = __byte_perm(__float_as_uint(p0), __float_as_uint(p1), 0x7632);   // upper halves: bf16 by truncation (one PRMT, ALU pipe)
-#else
-          pk[i] = pack_bf16x2(p0, p1);
-#endif
-        }
-      };
-      auto row_sum = [&]() {
-        float a0, a1, b0, b1;
-        unpack_f32x2(la, a0, a1);
-        unpack_f32x2(lb, b0, b1);
-        return (a0 + a1) + (b0 + b1);
-      };
-      // rare: move the reference (whole warp; rows that do not need it use alpha = 1)
-      auto renorm = [&](const int j, const float lsum) {
-        if (!(lsum <= kHard) || pmax > kPolyMax) hard = true;
-        float alpha = 1.f;
-        if (lsum > kSoft && !hard) {
-          const float m_new = m_ref + static_cast<float>((__float_as_int(lsum) >> 23) - 127);
-          alpha = exp2_approx(m_ref - m_new);
-          m_ref = m_new;
-        }
-        if (j > 0) {
-          mbar_wait(pv_done, (j - 1) & 1);   // every P V issued so far has drained: O may be touched
-          tc_fence_after();
-          rescale_o(alpha);
-        }
-        const uint64_t alpha2 = pack_f32x2(alpha, alpha);
-        la = fmul2(la, alpha2);
-        lb = fmul2(lb, alpha2);
-        pmax = -INFINITY;
-      };
-      auto tile = [&](const int j, auto masked_tag) {
-        constexpr bool kMasked = decltype(masked_tag)::value;
-        const int valid = A.S - j * kKT;
-        STRACE(0);
-        {
-          const float lsum = row_sum();
-          if (__any_sync(0xffffffffu, !(lsum <= kSoft) || pmax > kPolyMax)) renorm(j, lsum);
-        }
-        const uint64_t negm2 = pack_f32x2(-m_ref, -m_ref);
-        mbar_wait(s_full, j & 1);
-        tc_fence_after();
-        if (warp == 4 && lane == 0) mbar_arrive(&k_empty[j % kKVStages]);   // Q K(j)^T has completed: the K stage is free
-        STRACE(1);
-        uint32_t va[32], vb[32], pk[16];
-        tmem_ld_32x32(s_tmem, va);
-        tmem_ld_32x32(s_tmem + kChunk, vb);
-        tmem_wait_ld();
-        STRACE(2);
-        if (kMasked) {
-          mask_chunk(0, va, valid);
-          mask_chunk(1, vb, valid);
-        }
-        exp_chunk(va, pk, negm2, masked_tag);
-        if (j > 0) {  // P is single-buffered: P(j-1) V must be done before P(j) lands
-          mbar_wait(pv_done, (j - 1) & 1);
-          tc_fence_after();
-          if (warp == 4 && lane == 0) mbar_arrive(&v_empty[(j - 1) % kKVStages]);   // ... and its V stage is free
-        }
-        tmem_st_32x16(p_tmem, pk);
-        tmem_ld_32x32(s_tmem + 2 * kChunk, va);
-        STRACE(3);
-        exp_chunk(vb, pk, negm2, masked_tag);
-        tmem_st_32x16(p_tmem + 16, pk);
-        tmem_ld_32x32(s_tmem + 3 * kChunk, vb);
-        // keys [0,64) of P(j) go to the MMA warp
-        tmem_wait_st();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&p_full[0]);
-        // all of S(j) is in registers: Q K^T of the next tile may overwrite it
-        tmem_wait_ld();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(s_free);
-        STRACE(4);
-        if (kMasked) {
-          mask_chunk(2, va, valid);
-          mask_chunk(3, vb, valid);
-        }
-        exp_chunk(va, pk, negm2, masked_tag);
-        tmem_st_32x16(p_tmem + 32, pk);
-        exp_chunk(vb, pk, negm2, masked_tag);
-        tmem_st_32x16(p_tmem + 48, pk);
-        tmem_wait_st();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&p_full[1]);
-        STRACE(5);
-      };
-      for (int j = 0; j < n_kv - 1; ++j) tile(j, std::false_type{});
-      tile(n_kv - 1, std::true_type{});
-#ifdef TPDM_ATTN_TRACE
-      if (threadIdx.x == 128) {
-        const int ctr2 = (qt == 5 && h == 3 && b == 0) ? 0 : (qt == 7 && h == 20 && b == 1) ? 1 : -1;
-        if (ctr2 >= 0) g_cta_trace[ctr2][4] = clock64();
-      }
-#endif
-      l = row_sum();
-      if (!(l <= kHard) || pmax > kPolyMax) hard = true;
-      if (hard) *redo_smem = 1;
-    } else {
     for (int j = 0; j < n_kv; ++j) {
       const int valid = A.S - j * kKT;  // keys valid in this tile (>= 1)
-      STRACE(0);
       mbar_wait(s_full, j & 1);
       tc_fence_after();
       if (warp == 4 && lane == 0) mbar_arrive(&k_empty[j % kKVStages]);   // Q K(j)^T has completed: the K stage is free
-      STRACE(1);
       uint32_t va[32], vb[32];
       tmem_ld_32x32(s_tmem, va);
       // rare path, entered by the whole warp when any row's chunk maximum runs more than 2^kRescaleThreshold above its reference
@@ -786,14 +597,12 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
       // S released at 10 % of the tile and P chunk 0 held in registers instead of waiting for P(j-1) V -- no wait on data left, yet
       // 375 us against 339 us: every mbarrier / tcgen05.wait placed between the halves of a chunk drains the warp's MUFU queue.)
       tmem_wait_ld();
-      STRACE(2);
       tmem_ld_32x32(s_tmem + kChunk, vb);
       mask_chunk(0, va, valid);
       {
         const float mc = chunk_max(va);
         if (__any_sync(0xffffffffu, mc > m_used + kRescaleThreshold)) raise_reference(0, mc);
       }
-      STRACE(6);
       auto do_chunk = [&](const int c, uint32_t (&cur)[32], uint32_t (&nxt)[32]) {
         constexpr int kLast = kKT / kChunk - 1;
         uint32_t pk[16];
@@ -816,7 +625,6 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
           mbar_wait(pv_done, (j - 1) & 1);
           tc_fence_after();
           if (warp == 4 && lane == 0) mbar_arrive(&v_empty[(j - 1) % kKVStages]);   // ... and its V stage is free
-          STRACE(7);
         }
         tmem_st_32x16(p_tmem + c * 16, pk);
         if (c + 2 <= kLast) tmem_ld_32x32(s_tmem + (c + 2) * kChunk, cur);
@@ -829,43 +637,19 @@ __device__ __forceinline__ void attn_cta(const AttnOp& A, uint8_t* smem, const i
           __syncwarp();
           if (lane == 0) mbar_arrive(&p_full[c == kLast ? 1 : 0]);
         }
-        if (c == 0) STRACE(3);
       };
       do_chunk(0, va, vb);
       do_chunk(1, vb, va);
       do_chunk(2, va, vb);
-      STRACE(4);
       do_chunk(3, vb, va);
-      STRACE(5);
     }
     float l_lo, l_hi;
     unpack_f32x2(l2, l_lo, l_hi);
-    l = l_lo + l_hi;
-    }
-    // epilogue: O / l -> bf16, token-major
     mbar_wait(pv_done, (n_kv - 1) & 1);
     tc_fence_after();
     const int row = q0 + q * 32 + lane;
-    const float inv_l = (kFast && TPDM_ATTN_TRUNC_P) ? 1.0f / (l * (1.0f - 0.00140887f)) : 1.0f / l;
-    __nv_bfloat16* out = A.out + (static_cast<long long>(b) * A.S + row) * (static_cast<long long>(A.H) * DP) + h * DP;
-#pragma unroll
-    for (int c = 0; c < DP / 32; ++c) {
-      uint32_t o[32];
-      tmem_ld_32x32(o_tmem + c * 32, o);
-      tmem_wait_ld();
-      if (row < A.S) {
-        uint4* dst = reinterpret_cast<uint4*>(out + c * 32);
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          uint4 w;
-          w.x = pack_bf16x2(__uint_as_float(o[8 * e + 0]) * inv_l, __uint_as_float(o[8 * e + 1]) * inv_l);
-          w.y = pack_bf16x2(__uint_as_float(o[8 * e + 2]) * inv_l, __uint_as_float(o[8 * e + 3]) * inv_l);
-          w.z = pack_bf16x2(__uint_as_float(o[8 * e + 4]) * inv_l, __uint_as_float(o[8 * e + 5]) * inv_l);
-          w.w = pack_bf16x2(__uint_as_float(o[8 * e + 6]) * inv_l, __uint_as_float(o[8 * e + 7]) * inv_l);
-          dst[e] = w;
-        }
-      }
-    }
+    store_o<DP>(o_tmem, 1.0f / (l_lo + l_hi), A.out + (static_cast<long long>(b) * A.S + row) * (static_cast<long long>(A.H) * DP) + h * DP,
+                row < A.S);
   }
 
   __syncwarp();
@@ -898,7 +682,7 @@ __global__ void __launch_bounds__(kFastThreads, DP == 64 ? 2 : 1) joint_attentio
     tma_prefetch_desc(&A.tmK);
     tma_prefetch_desc(&A.tmV);
   }
-  if (warp == 1 && lane == 0) B.init(false, kSplit ? 8 : 4);
+  if (warp == 1 && lane == 0) B.init(false, 8);
   if (threadIdx.x == 0) redo_smem = 0;
   pdl_wait();
   CTRACE(1);
@@ -939,46 +723,8 @@ __global__ void __launch_bounds__(kFastThreads, DP == 64 ? 2 : 1) joint_attentio
 #endif
 }
 
-// Exact kernel alone (TPDM_ATTN_EXACT=1): per-chunk maxima from the first tile on, as in round 1 / early round 2.
-template <int DP>
-__global__ void __launch_bounds__(kAttnThreads, DP == 64 ? 2 : 1) joint_attention_exact_kernel(const __grid_constant__ AttnOp A) {
-  using L = AttnSmem<DP>;
-  pdl_launch_dependents();
-  uint8_t* smem = attn_smem_base();
-  const AttnBars<DP> B(smem);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&A.tmQ);
-    tma_prefetch_desc(&A.tmK);
-    tma_prefetch_desc(&A.tmV);
-  }
-  if (warp == 1 && lane == 0) B.init(false);
-  pdl_wait();
-  if (A.skip != nullptr && *A.skip != 0) return;
-  if (A.bmask != nullptr && A.bmask[blockIdx.z % A.bslots] == 0) return;  // emptied queue slot
-  if (warp == 2) {
-    tmem_alloc<L::kTmemCols>(B.tmem_slot);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  attn_cta<DP, false>(A, smem, blockIdx.x, blockIdx.y, blockIdx.z, nullptr);
-  if (warp == 2) tmem_dealloc<L::kTmemCols>(*B.tmem_slot);
-}
-
-// TPDM_ATTN_EXACT=1: only the exact kernel (per-chunk maxima), as in round 1 / early round 2 -- for A/B timing and tests
-bool exact_only() {
-  static const bool v = [] {
-    const char* e = getenv("TPDM_ATTN_EXACT");
-    return e != nullptr && e[0] == '1';
-  }();
-  return v;
-}
-
-// Redo flags of the fast kernel, one int per CTA: slices of one device buffer handed out round-robin at attn_op_init time (an op
-// keeps its slice; after a wrap two ops may share one, which is harmless on one stream: the fast kernel rewrites every flag of its
-// grid before the exact kernel behind it reads them).
+// Redo flags, one int per CTA: slices of one device buffer handed out round-robin at attn_op_init time (an op keeps its slice; after
+// a wrap two ops may share one, which is harmless on one stream: every launch rewrites every flag of its grid).
 constexpr size_t kRedoCapacity = size_t(1) << 20;
 int* redo_slice(size_t n) {
   static int* buf = nullptr;
@@ -995,7 +741,7 @@ int* redo_slice(size_t n) {
   return p;
 }
 
-const int* g_last_redo = nullptr;   // slice and grid size of the last launch (tpdm_attention_redo_count)
+const int* g_last_redo = nullptr;   // slice and grid size of the last launch (tpdm_attention_redo_count; nullptr: no slice)
 int g_last_redo_n = 0;
 
 template <int DP>
@@ -1003,18 +749,14 @@ int attn_launch_impl(const AttnOp& op, cudaStream_t stream) {
   static bool attr_set = false;
   if (!attr_set) {
     TPDM_CUDA_OK(cudaFuncSetAttribute(joint_attention_fast_kernel<DP>, cudaFuncAttributeMaxDynamicSharedMemorySize, AttnSmem<DP>::kTotal));
-    TPDM_CUDA_OK(cudaFuncSetAttribute(joint_attention_exact_kernel<DP>, cudaFuncAttributeMaxDynamicSharedMemorySize, AttnSmem<DP>::kTotal));
     attr_set = true;
   }
   dim3 grid(op.q_tiles, op.H, op.Bt);
-  g_last_redo = exact_only() ? nullptr : op.redo;
+  g_last_redo = op.redo;
   g_last_redo_n = op.q_tiles * op.H * op.Bt;
   const double q_rows = op.q_tiles * kQT < op.S ? op.q_tiles * kQT : op.S;
   prof_begin(1, 4.0 * op.Bt * op.H * q_rows * op.S * op.head_dim, stream);
-  if (exact_only())
-    TPDM_CUDA_OK(launch_pdl(joint_attention_exact_kernel<DP>, grid, dim3(kAttnThreads), AttnSmem<DP>::kTotal, stream, op));
-  else
-    TPDM_CUDA_OK(launch_pdl(joint_attention_fast_kernel<DP>, grid, dim3(kFastThreads), AttnSmem<DP>::kTotal, stream, op));
+  TPDM_CUDA_OK(launch_pdl(joint_attention_fast_kernel<DP>, grid, dim3(kFastThreads), AttnSmem<DP>::kTotal, stream, op));
   prof_end(stream);
   count_launch();
   TPDM_CUDA_OK(cudaGetLastError());

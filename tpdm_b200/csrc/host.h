@@ -140,11 +140,11 @@ struct alignas(64) AttnOp {
   const int* bmask = nullptr; // see set_batch_mask
   int bslots = 1;
   __nv_bfloat16* out;         // [Bt][S][H*dp]
-  int* redo = nullptr;        // [Bt*H*q_tiles] flags: CTAs of the fast kernel that must be recomputed by the exact kernel
+  int* redo = nullptr;        // [Bt*H*q_tiles] flags: CTAs that recomputed their tile with the exact softmax
 };
 int attn_op_init(AttnOp* op, const void* qkv, int Bt, int S, int H, int dp, int head_dim, void* out);
 int attn_launch(const AttnOp* op, cudaStream_t stream);
 long long attn_redo_total();  // diagnostic, synchronises: CTAs that took the exact pass since the library was loaded
-int attn_redo_count();  // diagnostic, synchronises: CTAs of the last launch recomputed by the exact kernel (-1: exact only)
+int attn_redo_count();  // diagnostic, synchronises: CTAs of the last launch recomputed with the exact softmax (-1: no flag buffer)
 
 }  // namespace tpdm
