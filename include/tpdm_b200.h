@@ -270,6 +270,15 @@ int tpdm_queue_begin(tpdm_plan* plan, int n_prompts, const float* latents_all, c
                      float guidance_scale, void* queue_workspace, size_t queue_workspace_bytes, int* ticket,
                      float* out_latents, int* out_steps, float* out_sigmas, const int* order, int n_queued,
                      const float* init_sigma, int init_step, void* stream);
+/* Switch a begun queue to sampled rollouts (predict = 0): call after tpdm_queue_begin, before its first tpdm_queue_step.
+ * Every prompt then follows the trajectory tpdm_sample_* with predict = 0 gives row `prompt` of one batch of all P prompts.
+ * ratios_all [P][max_steps] (NULL: device Beta draws from `seed`, keyed by (prompt, trajectory step) exactly as
+ * tpdm_sample_begin keys sample b); records, each [P][max_steps] row-major and each optional: alphas, betas, logprobs (raw),
+ * tembs [P][max_steps][D], tpm_inputs bf16 [P][max_steps][g][g][2D].  Entries past a prompt's last step are not written.
+ * TPDM_ERR_STATE before tpdm_queue_begin or after one with init_step > 0 (the probe step ran the Beta mode).  A captured
+ * queue-step graph is dropped; the seed stays fixed for the drain, so tpdm_queue_step_graph captures the rollout step once. */
+int tpdm_queue_set_rollout(tpdm_plan* plan, unsigned long long seed, const float* ratios_all, float* alphas, float* betas,
+                           float* logprobs, float* tembs, void* tpm_inputs);
 /* one denoising step of every occupied slot, then retire / refill.  No host synchronisation. */
 int tpdm_queue_step(tpdm_plan* plan, void* stream);
 /* the same step replayed from a CUDA graph captured on the first call (stream must not be the legacy default stream) */

@@ -91,6 +91,7 @@ EXPORTS = {
     "tpdm_tpm_train_backward": (C.c_int, [vp, vp, vp]),
     "tpdm_queue_workspace_bytes": (C.c_size_t, [vp, C.c_int]),
     "tpdm_queue_begin": (C.c_int, [vp, C.c_int, vp, vp, vp, vp, vp, C.c_float, vp, C.c_size_t, vp, vp, vp, vp, vp, C.c_int, vp, C.c_int, vp]),
+    "tpdm_queue_set_rollout": (C.c_int, [vp, C.c_ulonglong, vp, vp, vp, vp, vp, vp]),
     "tpdm_queue_step": (C.c_int, [vp, vp]),
     "tpdm_queue_step_graph": (C.c_int, [vp, vp]),
     "tpdm_queue_status": (C.c_int, [vp, C.POINTER(vp), C.POINTER(vp)]),

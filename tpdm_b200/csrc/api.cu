@@ -81,6 +81,12 @@ struct tpdm_plan {
     const int* order = nullptr;
     const float* init_sigma = nullptr;
     int init_step = 0, n_queued = 0;
+    // sampled rollouts (tpdm_queue_set_rollout); tpdm_queue_begin resets the queue to predict mode
+    int predict = 1;
+    unsigned long long seed = 0;
+    const float* ratios_all = nullptr;
+    float *rec_alphas = nullptr, *rec_betas = nullptr, *rec_logprobs = nullptr, *rec_tembs = nullptr;
+    bf16* rec_tpm = nullptr;
     cudaGraphExec_t graph = nullptr;   // one captured queue step (every pointer of a queue step is fixed between steps)
     long long graph_launches = 0;
   } q;
@@ -658,6 +664,12 @@ QueueArgs queue_args(const tpdm_plan* p, int init) {
   a.init = init;
   a.min_sigma = p->ctx->cfg.min_sigma;
   a.epsilon = p->ctx->cfg.epsilon;
+  a.predict = q.predict;
+  a.seed = q.seed;
+  a.ratios_all = q.ratios_all;
+  a.rec_alphas = q.rec_alphas;
+  a.rec_betas = q.rec_betas;
+  a.rec_logprobs = q.rec_logprobs;
   return a;
 }
 int queue_move(tpdm_plan* p, cudaStream_t s) {
@@ -720,6 +732,11 @@ int tpdm_queue_begin(tpdm_plan* p, int n_prompts, const float* latents_all, cons
   q.out_latents = out_latents;
   q.out_steps = out_steps;
   q.out_sigmas = out_sigmas;
+  q.predict = 1;
+  q.seed = 0;
+  q.ratios_all = nullptr;
+  q.rec_alphas = q.rec_betas = q.rec_logprobs = q.rec_tembs = nullptr;
+  q.rec_tpm = nullptr;
   p->guidance = guidance_scale;
   p->predict = 1;
   // sigma-independent text branch of every prompt, B prompts at a time through the plan's own buffers
@@ -760,6 +777,10 @@ int tpdm_queue_step(tpdm_plan* p, void* stream) {
   if (st_mm == 0) st_mm = run_tpm(p, B, p->temb_cfg, p->alpha_beta, s);
   set_batch_mask(nullptr, 1);
   TPDM_TRY(st_mm);
+  const tpdm_plan::Queue& q = p->q;
+  if (q.rec_tembs || q.rec_tpm)  // before queue_advance moves the slots on
+    TPDM_TRY(k_queue_record(q.slot_prompt, q.slot_step, B, p->max_steps, ctx->D, p->temb_cfg, q.rec_tembs, p->tpm_x, q.rec_tpm,
+                            static_cast<long long>(p->g) * p->g * 2 * ctx->D, s));
   TPDM_TRY(k_queue_schedule(queue_args(p, 0), s));
   TPDM_TRY(k_unpatchify(p->pout, B, 1, p->guidance, ctx->cfg.out_channels, p->Hl, p->Wl, nullptr, p->latents, p->q.sigma_cur,
                         p->q.sigma_next, 1, nullptr, s));
@@ -768,12 +789,35 @@ int tpdm_queue_step(tpdm_plan* p, void* stream) {
   return 0;
 }
 
+int tpdm_queue_set_rollout(tpdm_plan* p, unsigned long long seed, const float* ratios_all, float* alphas, float* betas, float* logprobs,
+                           float* tembs, void* tpm_inputs) {
+  TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_queue_set_rollout: null plan");
+  TPDM_CHECK(p->q.begun, TPDM_ERR_STATE, "tpdm_queue_set_rollout: call tpdm_queue_begin first");
+  // the probe step of longest-first scheduling ran the Beta mode, so such a queue cannot start sampled trajectories
+  TPDM_CHECK(p->q.init_step == 0, TPDM_ERR_STATE, "tpdm_queue_set_rollout: the queue began after %d probe steps (init_step > 0)", p->q.init_step);
+  tpdm_plan::Queue& q = p->q;
+  if (q.graph) {  // the captured step holds the predict-mode arguments
+    cudaGraphExecDestroy(q.graph);
+    q.graph = nullptr;
+  }
+  q.predict = 0;
+  q.seed = seed;
+  q.ratios_all = ratios_all;
+  q.rec_alphas = alphas;
+  q.rec_betas = betas;
+  q.rec_logprobs = logprobs;
+  q.rec_tembs = tembs;
+  q.rec_tpm = static_cast<bf16*>(tpm_inputs);
+  return 0;
+}
+
 int tpdm_queue_step_graph(tpdm_plan* p, void* stream) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_queue_step_graph: null plan");
   TPDM_CHECK(p->q.begun, TPDM_ERR_STATE, "tpdm_queue_step_graph: call tpdm_queue_begin first");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (p->q.graph == nullptr) {
-    // a queue step has no host-side argument that changes between steps: capture it once, replay it every step
+    // a queue step has no host-side argument that changes between steps (a rollout's seed is fixed for the whole drain):
+    // capture it once, replay it every step
     const long long before = launches_so_far();
     cudaGraph_t g = nullptr;
     TPDM_CUDA_OK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));

@@ -711,52 +711,69 @@ __device__ float gamma_draw(curandStatePhilox4_32_10_t* st, float shape) {
   return boost * d;
 }
 
-// schedule update (modeling_sd3_pnt.py:557-590, 608)
+// One sample's schedule update (modeling_sd3_pnt.py:557-590) from the raw TimePredictor outputs (p1, p2) at `sigma`.  The ratio
+// is the Beta mode (predict), `given` (an injected draw) or Beta.sample() from the Philox stream (seed, sample, step * 1024);
+// tpdm_sample_* and the device queue both key that stream by (sample or prompt, trajectory step), so both draw the same ratio.
+enum RatioSource { kRatioMode, kRatioGiven, kRatioDraw };
+struct ScheduleStep {
+  float alpha, beta, ratio, sigma_next;
+  double logprob;
+};
+__device__ __forceinline__ ScheduleStep schedule_step(float p1, float p2, float sigma, RatioSource src, float given, unsigned long long seed,
+                                                      int sample, int step, int prediction_type, int relative, float epsilon) {
+  ScheduleStep r;
+  if (prediction_type == 0) {
+    r.alpha = p1;
+    r.beta = p2;
+  } else {
+    r.alpha = p1 * (p2 - 2.f) + 1.f;
+    r.beta = (1.f - p1) * (p2 - 2.f) + 1.f;
+  }
+  float ratio;
+  if (src == kRatioMode) {
+    ratio = (r.alpha - 1.f) / (r.alpha + r.beta - 2.f);  // Beta.mode (:567)
+  } else if (src == kRatioGiven) {
+    ratio = given;
+  } else {  // Beta.sample() (:569) = Ga / (Ga + Gb)
+    curandStatePhilox4_32_10_t st;
+    curand_init(seed, static_cast<unsigned long long>(sample), static_cast<unsigned long long>(step) * 1024ull, &st);
+    const float ga = gamma_draw(&st, r.alpha), gb = gamma_draw(&st, r.beta);
+    ratio = ga / (ga + gb);
+  }
+  if (relative) {
+    ratio = fminf(fmaxf(ratio, epsilon), 1.f - epsilon);
+    r.sigma_next = sigma * ratio;
+  } else {
+    ratio = fminf(fmaxf(ratio, epsilon), sigma);
+    ratio = fminf(fmaxf(ratio, 0.f), 1.f - epsilon);
+    r.sigma_next = sigma - ratio;
+  }
+  r.ratio = ratio;
+  const double A = r.alpha, Bq = r.beta, rr = ratio;
+  r.logprob = (A - 1.0) * log(rr) + (Bq - 1.0) * log1p(-rr) + lgamma(A + Bq) - lgamma(A) - lgamma(Bq);
+  return r;
+}
+
+// schedule update of the lockstep batch (modeling_sd3_pnt.py:557-590, 608)
 __global__ void schedule_kernel(const ScheduleArgs a) {
   const int i = threadIdx.x;
   int done = 1;
   if (i < a.B) {
-    const float p1 = a.alpha_beta[2 * i], p2 = a.alpha_beta[2 * i + 1];
-    float alpha, beta;
-    if (a.prediction_type == 0) {
-      alpha = p1;
-      beta = p2;
-    } else {
-      alpha = p1 * (p2 - 2.f) + 1.f;
-      beta = (1.f - p1) * (p2 - 2.f) + 1.f;
-    }
     const float sigma = a.sigma_hist[i * (a.T + 1) + a.step];
-    float ratio;
-    if (a.predict) {
-      ratio = (alpha - 1.f) / (alpha + beta - 2.f);  // Beta.mode (:567)
-    } else if (a.ratios) {
-      ratio = a.ratios[i * a.T + a.step];
-    } else {  // Beta.sample() (:569) = Ga / (Ga + Gb)
-      curandStatePhilox4_32_10_t st;
-      curand_init(a.seed, static_cast<unsigned long long>(i), static_cast<unsigned long long>(a.step) * 1024ull, &st);
-      const float ga = gamma_draw(&st, alpha), gb = gamma_draw(&st, beta);
-      ratio = ga / (ga + gb);
-    }
-    float sigma_next;
-    if (a.relative) {
-      ratio = fminf(fmaxf(ratio, a.epsilon), 1.f - a.epsilon);
-      sigma_next = sigma * ratio;
-    } else {
-      ratio = fminf(fmaxf(ratio, a.epsilon), sigma);
-      ratio = fminf(fmaxf(ratio, 0.f), 1.f - a.epsilon);
-      sigma_next = sigma - ratio;
-    }
-    const double A = alpha, Bq = beta, r = ratio;
-    const double lp = (A - 1.0) * log(r) + (Bq - 1.0) * log1p(-r) + lgamma(A + Bq) - lgamma(A) - lgamma(Bq);
+    const RatioSource src = a.predict ? kRatioMode : (a.ratios ? kRatioGiven : kRatioDraw);
+    const ScheduleStep r = schedule_step(a.alpha_beta[2 * i], a.alpha_beta[2 * i + 1], sigma, src,
+                                         src == kRatioGiven ? a.ratios[i * a.T + a.step] : 0.f, a.seed, i, a.step, a.prediction_type,
+                                         a.relative, a.epsilon);
+    float sigma_next = r.sigma_next;
     int mask = 0;
     if (sigma < a.min_sigma) {
       mask = 1;
       if (a.predict) sigma_next = 0.f;
     }
     const int o = i * a.T + a.step;
-    a.alphas[o] = alpha;
-    a.betas[o] = beta;
-    a.logprobs[o] = static_cast<float>(lp);
+    a.alphas[o] = r.alpha;
+    a.betas[o] = r.beta;
+    a.logprobs[o] = static_cast<float>(r.logprob);
     a.masks[o] = mask;
     a.sigma_hist[i * (a.T + 1) + a.step + 1] = sigma_next;
     done = sigma_next < a.min_sigma ? 1 : 0;
@@ -778,30 +795,49 @@ __global__ void __launch_bounds__(256) sum_partials_kernel(const float* __restri
 }
 
 // ---- device-side prompt queue ---------------------------------------------------------------------------------
-// predict-mode schedule update per slot (modeling_sd3_pnt.py:557-590 with ratio = Beta mode), sigma kept per slot
+// schedule update per slot (modeling_sd3_pnt.py:557-590), sigma kept per slot.  predict: ratio = Beta mode.  Rollouts
+// (predict == 0): the prompt's injected ratio or a Philox draw keyed by (prompt, the slot's own trajectory step), recorded per
+// prompt and step.
 __global__ void queue_schedule_kernel(const QueueArgs a) {
   const int i = threadIdx.x;
   if (i >= a.B) return;
-  const float p1 = a.alpha_beta[2 * i], p2 = a.alpha_beta[2 * i + 1];
-  float alpha = p1, beta = p2;
-  if (a.prediction_type != 0) {
-    alpha = p1 * (p2 - 2.f) + 1.f;
-    beta = (1.f - p1) * (p2 - 2.f) + 1.f;
-  }
   const float sigma = a.sigma_cur[i];
-  float ratio = (alpha - 1.f) / (alpha + beta - 2.f);
-  float sigma_next;
-  if (a.relative) {
-    ratio = fminf(fmaxf(ratio, a.epsilon), 1.f - a.epsilon);
-    sigma_next = sigma * ratio;
-  } else {
-    ratio = fminf(fmaxf(ratio, a.epsilon), sigma);
-    ratio = fminf(fmaxf(ratio, 0.f), 1.f - a.epsilon);
-    sigma_next = sigma - ratio;
+  const int prompt = a.slot_prompt[i];
+  if (prompt < 0) {  // idle slot: the Euler step is a no-op
+    a.sigma_next[i] = sigma;
+    return;
   }
-  if (sigma < a.min_sigma) sigma_next = 0.f;
-  if (a.slot_prompt[i] < 0) sigma_next = sigma;  // idle slot: the Euler step is a no-op
+  const int step = a.slot_step[i];
+  const long long o = static_cast<long long>(prompt) * a.max_steps + step;
+  const RatioSource src = a.predict ? kRatioMode : (a.ratios_all ? kRatioGiven : kRatioDraw);
+  const ScheduleStep r = schedule_step(a.alpha_beta[2 * i], a.alpha_beta[2 * i + 1], sigma, src, src == kRatioGiven ? a.ratios_all[o] : 0.f,
+                                       a.seed, prompt, step, a.prediction_type, a.relative, a.epsilon);
+  float sigma_next = r.sigma_next;
+  if (a.predict && sigma < a.min_sigma) sigma_next = 0.f;
   a.sigma_next[i] = sigma_next;
+  if (a.rec_alphas) a.rec_alphas[o] = r.alpha;
+  if (a.rec_betas) a.rec_betas[o] = r.beta;
+  if (a.rec_logprobs) a.rec_logprobs[o] = static_cast<float>(r.logprob);
+}
+
+// rollout records of every occupied slot at its own (prompt, step): the CFG-combined temb [D] and the NHWC bf16 TimePredictor
+// input [g][g][2D] (6.3 MB per slot at 512^2), 16-byte vector copies spread over gridDim.x blocks per slot
+__global__ void __launch_bounds__(256) queue_record_kernel(const int* __restrict__ slot_prompt, const int* __restrict__ slot_step, int max_steps,
+                                                           int D, const float* __restrict__ temb_cfg, float* __restrict__ tembs_all,
+                                                           const uint4* __restrict__ tpm_x, uint4* __restrict__ tpm_all, long long tpm_vecs) {
+  const int b = blockIdx.y;
+  const int prompt = slot_prompt[b];
+  if (prompt < 0) return;
+  const long long o = static_cast<long long>(prompt) * max_steps + slot_step[b];
+  const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
+  const long long t0 = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (tembs_all)
+    for (long long k = t0 * 4; k < D; k += stride * 4) *reinterpret_cast<float4*>(tembs_all + o * D + k) = ld4(temb_cfg + static_cast<long long>(b) * D + k);
+  if (tpm_all) {
+    const uint4* src = tpm_x + b * tpm_vecs;
+    uint4* dst = tpm_all + o * tpm_vecs;
+    for (long long k = t0; k < tpm_vecs; k += stride) dst[k] = __ldg(src + k);
+  }
 }
 
 // after the Euler step: count the step, retire finished trajectories, hand the freed slots their next ticket
@@ -1169,6 +1205,18 @@ int k_queue_schedule(const QueueArgs& a, cudaStream_t s) {
 int k_queue_advance(const QueueArgs& a, cudaStream_t s) {
   TPDM_CHECK(a.B <= 1024, TPDM_ERR_SHAPE, "queue: %d slots > 1024", a.B);
   queue_advance_kernel<<<1, ((a.B + 31) / 32) * 32, 0, s>>>(a);
+  count_launch();
+  TPDM_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
+int k_queue_record(const int* slot_prompt, const int* slot_step, int B, int max_steps, int D, const float* temb_cfg, float* tembs_all,
+                   const bf16* tpm_x, bf16* tpm_all, long long tpm_elems, cudaStream_t s) {
+  TPDM_CHECK(D % 4 == 0 && tpm_elems % 8 == 0, TPDM_ERR_SHAPE, "queue_record: D and the TimePredictor input must be whole 16-byte vectors");
+  TPDM_CHECK((reinterpret_cast<uintptr_t>(tembs_all) & 15) == 0 && (reinterpret_cast<uintptr_t>(tpm_all) & 15) == 0, TPDM_ERR_ARG,
+             "queue_record: record buffers must be 16-byte aligned");
+  queue_record_kernel<<<dim3(64, B), 256, 0, s>>>(slot_prompt, slot_step, max_steps, D, temb_cfg, tembs_all, reinterpret_cast<const uint4*>(tpm_x),
+                                                  reinterpret_cast<uint4*>(tpm_all), tpm_elems / 8);
   count_launch();
   TPDM_CUDA_OK(cudaGetLastError());
   return 0;

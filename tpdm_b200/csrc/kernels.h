@@ -101,9 +101,18 @@ struct QueueArgs {
   int init_step;             // denoising steps every prompt has already made when it enters the queue (0 without a probe)
   int B, n_prompts, max_steps, relative, prediction_type, init;
   float min_sigma, epsilon;
+  // sampled rollouts (predict == 0): ratios_all [P][max_steps] or null (Philox draws from `seed`); records [P][max_steps], each optional
+  int predict;
+  unsigned long long seed;
+  const float* ratios_all;
+  float *rec_alphas, *rec_betas, *rec_logprobs;
 };
 int k_queue_schedule(const QueueArgs& a, cudaStream_t s);
 int k_queue_advance(const QueueArgs& a, cudaStream_t s);
+// per occupied slot b at (prompt, step) = (slot_prompt[b], slot_step[b]): tembs_all[prompt][step] = temb_cfg[b] ([D]) and
+// tpm_all[prompt][step] = tpm_x[b] (tpm_elems bf16); either destination may be null
+int k_queue_record(const int* slot_prompt, const int* slot_step, int B, int max_steps, int D, const float* temb_cfg, float* tembs_all,
+                   const bf16* tpm_x, bf16* tpm_all, long long tpm_elems, cudaStream_t s);
 // per slot b: flush -> out_latents[flush] = latents[b]; load -> latents[b] = noise_all[prompt], ctx0 / text_part rows b and B + b
 // = ctx0_all / text_all [prompt][0 | 1]
 int k_queue_move(const int* slot_prompt, const int* slot_flush, const int* slot_load, int B, long long lat, long long ctx, int D,

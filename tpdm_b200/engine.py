@@ -443,20 +443,40 @@ class Engine:
 
     def sample_queue(self, latents, prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds, negative_pooled_prompt_embeds,
                      slots: int, max_inference_steps: int, guidance_scale: float, ticket: Optional[torch.Tensor] = None,
-                     out_latents: Optional[torch.Tensor] = None, use_graph: bool = True, schedule: str = "fifo"):
+                     out_latents: Optional[torch.Tensor] = None, use_graph: bool = True, schedule: str = "fifo", predict: bool = True,
+                     seed: int = 0, ratios: Optional[torch.Tensor] = None, record: bool = True):
         """Device-side prompt queue (``tpdm_queue_*``): all P prompts are resident, ``slots`` of them are in flight; a slot
         whose trajectory ends takes the next ticket on the device.  ``ticket`` (int32 device tensor of one element, zeroed by
         its owner) may be shared between GPUs, which then split one prompt list between them.  Returns device tensors:
-        latents (P, C, h, w), steps (P,) (0 for prompts another GPU processed), sigmas (P, max_steps + 1)."""
+        latents (P, C, h, w), steps (P,) (0 for prompts another GPU processed), sigmas (P, max_steps + 1).
+        ``predict=False`` samples rollouts (``tpdm_queue_set_rollout``): prompt p follows row p of one lockstep
+        ``sample(..., predict=False)`` of all P prompts -- the injected ``ratios`` (P, max_steps) or the device draws of ``seed``.
+        The result then also holds alphas, betas, logprobs_raw (P, max_steps), tembs (P, max_steps, D) and, with ``record``,
+        tpm_inputs_nhwc (P, max_steps, g, g, 2D) bf16.  They are zero past each prompt's last step: the PPO replay runs the
+        TimePredictor on every (prompt, step) and multiplies those inputs by a zero gradient, which a stray NaN would poison."""
         lib = L.load()
         P, Cc, h, w = latents.shape
         dev, f32 = self.device, torch.float32
         if schedule not in ("fifo", "lpt"):
             raise ValueError(f"unknown queue schedule {schedule!r} ('fifo': tickets in prompt order, 'lpt': longest expected trajectory first)")
+        if schedule == "lpt" and not predict:
+            raise ValueError("schedule='lpt' probes step 0 with the Beta mode and cannot start sampled rollouts (predict=False)")
         if not 1 <= slots <= P:
             raise ValueError(f"slots must be in [1, {P}]")
         cvt = lambda t: t.to(device=dev, dtype=f32).contiguous()
         lat, pe, ne, pp, npp = cvt(latents), cvt(prompt_embeds), cvt(negative_prompt_embeds), cvt(pooled_prompt_embeds), cvt(negative_pooled_prompt_embeds)
+        rt, rec = None, {}
+        if not predict:
+            if ratios is not None:
+                rt = cvt(ratios)
+                if rt.shape != (P, max_inference_steps):
+                    raise ValueError(f"ratios must have shape {(P, max_inference_steps)}, got {tuple(rt.shape)}")
+            z = lambda *s, dtype=f32: torch.zeros(*s, device=dev, dtype=dtype)
+            rec = dict(alphas=z(P, max_inference_steps), betas=z(P, max_inference_steps), logprobs_raw=z(P, max_inference_steps))
+            rec["tembs"] = z(P, max_inference_steps, self.D)
+            if record:
+                g = h // 2
+                rec["tpm_inputs_nhwc"] = z(P, max_inference_steps, g, g, 2 * self.D, dtype=torch.bfloat16)
         if ticket is None:
             ticket = torch.zeros(1, dtype=torch.int32, device=dev)
         out_lat = torch.zeros(P, Cc, h, w, device=dev, dtype=f32) if out_latents is None else out_latents
@@ -486,6 +506,9 @@ class Engine:
                                          nbytes, ticket.data_ptr(), L.ptr(out_lat), L.ptr(out_steps), L.ptr(out_sig),
                                          L.ptr(order) if order is not None else None, int(n_queued),
                                          L.ptr(init_sigma) if init_sigma is not None else None, int(init_step), stream))
+            if not predict:
+                L.check(lib.tpdm_queue_set_rollout(plan.handle, int(seed) & (2**64 - 1), L.ptr(rt), L.ptr(rec["alphas"]), L.ptr(rec["betas"]),
+                                                   L.ptr(rec["logprobs_raw"]), L.ptr(rec.get("tembs")), L.ptr(rec.get("tpm_inputs_nhwc"))))
             act_p, slot_p = L.vp(), L.vp()
             L.check(lib.tpdm_queue_status(plan.handle, C.byref(act_p), C.byref(slot_p)))
             off = act_p.value - ws.data_ptr()          # the counters live in the queue workspace
@@ -513,5 +536,5 @@ class Engine:
                     raise RuntimeError("sample_queue: the queue did not drain within the step bound")
             torch.cuda.current_stream().synchronize()
         torch.cuda.current_stream(dev).wait_stream(qs)
-        self._queue_keepalive = (ws, lat, pe, ne, pp, npp, ticket, order, init_sigma)
-        return dict(latents=out_lat, steps=out_steps, sigmas=out_sig, device_steps=steps_run + (1 if init_step else 0))
+        self._queue_keepalive = (ws, lat, pe, ne, pp, npp, ticket, order, init_sigma, rt)
+        return dict(latents=out_lat, steps=out_steps, sigmas=out_sig, device_steps=steps_run + (1 if init_step else 0), **rec)

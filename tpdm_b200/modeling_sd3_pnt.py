@@ -317,13 +317,8 @@ class SD3PredictNextTimeStepModel(nn.Module):
             for i in range(batch_size):
                 steps_i = self.vae.decode_latents(hist[i].to(out_dtype), output_type)   # (T, ...) all recorded steps
                 images.append(list(steps_i) if output_type == "pil" else steps_i)
-        elif self.vae is not None and hasattr(self.vae, "decode_latents"):        # :645-655 on the native decoder, one call
-            decoded = self.vae.decode_latents(finals, output_type)
-            images = [[im] for im in decoded] if output_type == "pil" else [decoded[i:i + 1] for i in range(batch_size)]
-        elif self.vae is not None and hasattr(self.vae, "decode"):                 # a caller-supplied module
-            for i in range(batch_size):
-                lat = (finals[i] / self.vae.config.scaling_factor) + self.vae.config.shift_factor
-                images.append(self.vae.decode(lat.unsqueeze(0).to(self.vae.dtype), return_dict=False)[0].detach())
+        else:
+            images = self._final_images(finals, output_type)
         hcs = None
         if "tpm_inputs_nhwc" in res:  # (B, T, g, g, 2D) bf16 -> reference layout (B, T, 2D, g, g) as a zero-copy view
             hcs = res["tpm_inputs_nhwc"].permute(0, 1, 4, 2, 3)
@@ -335,7 +330,60 @@ class SD3PredictNextTimeStepModel(nn.Module):
             out["velocities"] = res["velocities"]
         return out
 
+    def _final_images(self, finals, output_type):
+        """:645-655: the final latent of every prompt through the native decoder (one call) or a caller-supplied module;
+        [] without a VAE."""
+        images = []
+        if self.vae is not None and hasattr(self.vae, "decode_latents"):
+            decoded = self.vae.decode_latents(finals, output_type)
+            images = [[im] for im in decoded] if output_type == "pil" else [decoded[i:i + 1] for i in range(finals.shape[0])]
+        elif self.vae is not None and hasattr(self.vae, "decode"):
+            for i in range(finals.shape[0]):
+                lat = (finals[i] / self.vae.config.scaling_factor) + self.vae.config.shift_factor
+                images.append(self.vae.decode(lat.unsqueeze(0).to(self.vae.dtype), return_dict=False)[0].detach())
+        return images
+
     # ---------------------------------------------------------------------------------------------------------------
+    @torch.no_grad()
+    def sample_rollouts(self, prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds, negative_pooled_prompt_embeds, latents=None, *,
+                        slots: int, max_inference_steps: int = 28, guidance_scale: float = 7.0, generator=None, ratios=None,
+                        return_hidden_states: bool = True, output_type: str = "pil", use_graph: bool = True) -> CustomDiffusionModelOutput:
+        """Sampled rollouts (``forward(predict=False)``) through the device-side prompt queue: ``slots`` prompts are in flight and
+        a prompt leaves its slot when its own trajectory ends, where the lockstep batch of ``forward`` keeps stepping every
+        sample until the longest one is done.  ``generator`` is consumed as ``forward`` consumes it (initial latents, then one
+        Philox seed), so with equal generator states prompt p gets the rollout ``forward`` gives row p of one batch of all
+        prompts: the same Beta draws (or the injected ``ratios`` (P, max_inference_steps)), per-step records and output
+        container, with T the longest rollout's step count.  Records past a prompt's last step are zero.  Adds ``steps`` (P,)
+        and ``device_steps`` (queue steps executed)."""
+        if guidance_scale is None:
+            raise ValueError("guidance_scale=None is unsupported (as in the reference, whose sigma.repeat(2) is unconditional, :526)")
+        P = prompt_embeds.shape[0]
+        side = self.default_sample_size * self.vae_scale_factor
+        if latents is None:
+            latents = self.prepare_latents(P, self.transformer.config.in_channels, side, side, prompt_embeds.dtype, self.device, generator, None)
+        init_noise_latents = latents.clone()
+        seed = 0
+        if ratios is None:      # the draw forward(predict=False) makes (:292-296)
+            gen = generator[0] if isinstance(generator, (list, tuple)) else generator
+            seed = int(torch.randint(0, 2**62, (1,), generator=gen, device=gen.device if gen is not None else "cpu").item())
+        res = self.get_engine().sample_queue(latents, prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds, negative_pooled_prompt_embeds,
+                                             int(slots), int(max_inference_steps), float(guidance_scale), use_graph=use_graph, predict=False,
+                                             seed=seed, ratios=ratios, record=bool(return_hidden_states))
+        steps = res["steps"]
+        T = int(steps.max())
+        out_dtype = latents.dtype
+        prob_masks = torch.arange(T, device=steps.device)[None, :] >= steps[:, None]
+        logprobs = torch.masked_fill(res["logprobs_raw"][:, :T], prob_masks, 1.0)          # INVALID_LOGPROB (:615-621)
+        finals = res["latents"].to(out_dtype)
+        hcs = None
+        if "tpm_inputs_nhwc" in res:  # (P, T, g, g, 2D) bf16 -> reference layout (P, T, 2D, g, g) as a zero-copy view
+            hcs = res["tpm_inputs_nhwc"][:, :T].permute(0, 1, 4, 2, 3)
+        return CustomDiffusionModelOutput(
+            init_noise_latents=init_noise_latents, hidden_states_combineds=hcs, tembs=res["tembs"][:, :T].to(out_dtype).contiguous(),
+            images=self._final_images(finals, output_type), last_valid_indices=list(steps.long() - 1),
+            alphas=res["alphas"][:, :T].contiguous(), betas=res["betas"][:, :T].contiguous(), sigmas=res["sigmas"][:, 1:T + 1].contiguous(),
+            logprobs=logprobs, prob_masks=prob_masks, latents=finals, steps=steps, device_steps=res["device_steps"])
+
     @torch.no_grad()
     def sample_queue(self, prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds, negative_pooled_prompt_embeds, latents=None,
                      slots: int = 2, max_inference_steps: int = 28, guidance_scale: float = 7.0, generator=None, ticket=None,

@@ -47,19 +47,27 @@ def rloo_advantages(rlhf_reward: torch.Tensor, rloo_k: int) -> torch.Tensor:
 
 def rloo_update(wrapper, trainer: TimePredictorTrainer, data: Dict, reward_fn: Callable, rloo_k: int = 2, num_ppo_epochs: int = 4,
                 micro_batch_size: int = 8, cliprange: float = 0.2, gamma: float = 0.97, kl_coef: float = 0.0, seed: int = 0,
-                generator: Optional[torch.Generator] = None) -> Dict:
+                generator: Optional[torch.Generator] = None, slots: Optional[int] = None) -> Dict:
     """`wrapper`: SD3PredictNextTimeStepModelRLOOWrapper; `data`: dict with the four embedding tensors (and optionally
     'prompt'); `reward_fn(latents (B,C,h,w), outputs) -> (B,)` stands in for the reward model.  Randomness (initial noise, Beta
     draws, micro-batch permutations) comes from ``generator``, or from one generator per trainer that is seeded with ``seed`` on
     the FIRST update and then keeps advancing, so successive updates see independent rollouts (the reference's global RNG does
-    the same, rloo_trainer.py:133)."""
+    the same, rloo_trainer.py:133).  ``slots=None`` samples the rollouts as one lockstep batch (``wrapper.sample``, the
+    reference's semantics: finished samples keep stepping until the longest is done); an integer samples the same rollouts
+    through the device-side prompt queue with that many in flight (``sample_rollouts``), where each leaves its slot when it ends."""
     agent = wrapper.agent_model
     data = wrapper.rloo_repeat(dict(data), rloo_k)
     if generator is None:
         generator = getattr(trainer, "_rollout_generator", None)
         if generator is None:
             generator = trainer._rollout_generator = torch.Generator().manual_seed(seed)
-    outputs = wrapper.sample({**data, "predict": False, "generator": generator})
+    if slots is None:
+        outputs = wrapper.sample({**data, "predict": False, "generator": generator})
+    else:
+        guidance = 3.5 if "3.5" in wrapper.pretrained_model_name_or_path else data.get("guidance_scale", 7.0)     # as wrapper.sample
+        outputs = agent.sample_rollouts(data["prompt_embeds"], data["negative_prompt_embeds"], data["pooled_prompt_embeds"],
+                                        data["negative_pooled_prompt_embeds"], data.get("latents"), slots=slots,
+                                        max_inference_steps=wrapper.max_inference_steps, guidance_scale=guidance, generator=generator)
     prob_masks = outputs["prob_masks"]
     last_reward = reward_fn(outputs["latents"], outputs).float()
     shaped = shape_rollout(outputs, last_reward, relative=agent.relative, gamma=gamma, kl_coef=kl_coef, rloo_k=rloo_k)
