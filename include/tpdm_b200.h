@@ -137,6 +137,26 @@ int tpdm_destroy(tpdm_ctx* ctx);
  * (modeling_sd3_pnt.py:144-157, gradio_sd3_inference.py:20-21). */
 int tpdm_set_weights(tpdm_ctx* ctx, const tpdm_weights* w);
 
+/* Opt-in FP8 (E4M3) mode of the MMDiT's QKV and FF1 projections.  Per block (host array [num_layers]): E4M3 codes
+ * [N][K] of the bf16 matrices of the same name in tpdm_block_weights, quantized per output channel by tpdm_quantize_fp8_rows,
+ * and their fp32 scales [N]; cff1_w / cff1_s are null in the last block.  Borrowed for the lifetime of the ctx. */
+typedef struct tpdm_fp8_block_weights {
+  const void* qkv_w;    /* E4M3 [3*Dp][D] */
+  const float* qkv_s;   /* [3*Dp] */
+  const void* cqkv_w;   /* E4M3 [3*Dp][D] */
+  const float* cqkv_s;
+  const void* ff1_w;    /* E4M3 [4D][D] */
+  const float* ff1_s;
+  const void* cff1_w;   /* E4M3 [4D][D] (null in the last block) */
+  const float* cff1_s;
+} tpdm_fp8_block_weights;
+/* Call after tpdm_set_weights and before the first tpdm_plan_create of the ctx (TPDM_ERR_STATE once a plan has been created).
+ * Every plan of the ctx then runs QKV / context QKV and FF1 / context FF1 as E4M3 x E4M3 -> fp32 GEMMs: ln_modulate writes the
+ * modulated token rows as E4M3 codes with one scale per row, and the GEMM epilogue applies row scale x channel scale before the
+ * bias.  Out-projections, FF2, attention, qk-RMSNorm, SD3.5 attn2, context_embedder, proj_out and the TimePredictor stay bf16.
+ * tpdm_plan_workspace_bytes then includes the E4M3 activations and their row scales. */
+int tpdm_set_fp8_weights(tpdm_ctx* ctx, const tpdm_fp8_block_weights* blocks);
+
 /* A plan fixes the shapes: `batch` prompts (transformer batch Bt = 2*batch when cfg_pairs != 0, i.e. the loop's
  * cat([latents]*2) at modeling_sd3_pnt.py:524; else Bt = batch), latent side, text tokens, recorded steps. */
 size_t tpdm_plan_workspace_bytes(const tpdm_ctx* ctx, int batch, int cfg_pairs, int latent_h, int latent_w, int n_text,
@@ -382,6 +402,17 @@ int tpdm_conv3x3_wgrad(const void* dyt, const void* x_shifted_nchw, float* dw, i
 /* LayerNorm(eps 1e-6, no affine) * (1 + scale[b]) + shift[b] : x fp32 [batch][rows][D] -> bf16 */
 int tpdm_ln_modulate(const float* x, const float* shift, const float* scale, int mod_stride, void* out_bf16, int batch,
                      int rows, int D, void* stream);
+/* E4M3 row quantization, the rounding every FP8 operand of the library uses: per row, amax = max |x|, codes =
+ * cvt.rn.satfinite.e4m3(x * (448 / amax)), scale = amax / 448 (IEEE fp32 divisions), so x ~= code * scale; a zero row gets
+ * scale 1 and zero codes.  x fp32 [rows][K] (K % 4 == 0) -> codes E4M3 [rows][K], scales fp32 [rows]. */
+int tpdm_quantize_fp8_rows(const float* x, int rows, int K, void* codes, float* scales, void* stream);
+/* tpdm_ln_modulate with the result quantized per row as above: codes E4M3 [batch][rows][D], scales fp32 [batch][rows] */
+int tpdm_ln_modulate_fp8(const float* x, const float* shift, const float* scale, int mod_stride, void* out_codes, float* out_scales,
+                         int batch, int rows, int D, void* stream);
+/* out = epilogue((A8[batch][rows][K] . W8[N][K]^T) * a_scale[batch][rows] * w_scale[N] + bias), E4M3 operands, fp32
+ * accumulation; epi 0 -> bf16, 1 -> f32, 2 gelu -> bf16.  N > 128, K % 16 == 0. */
+int tpdm_gemm_fp8(const void* A8, const float* a_scale, const void* W8, const float* w_scale, const float* bias, void* out, int batch,
+                  int rows, int N, int K, int epi, void* stream);
 
 #ifdef __cplusplus
 }

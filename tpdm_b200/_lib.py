@@ -30,6 +30,13 @@ class TpdmBlockWeights(C.Structure):
     _fields_ = [(n, vp) for n in BLOCK_FIELDS]
 
 
+FP8_BLOCK_FIELDS = ("qkv_w", "qkv_s", "cqkv_w", "cqkv_s", "ff1_w", "ff1_s", "cff1_w", "cff1_s")
+
+
+class TpdmFp8BlockWeights(C.Structure):
+    _fields_ = [(n, vp) for n in FP8_BLOCK_FIELDS]
+
+
 GLOBAL_FIELDS_A = ("patch_w", "patch_b", "pos_table", "t_w1", "t_b1", "t_w2", "t_b2", "p_w1", "p_b1", "p_w2", "p_b2",
                    "ctx_w", "ctx_b", "adaln_w", "adaln_b", "proj_w", "proj_b")
 GLOBAL_FIELDS_B = ("tpm_conv1_w", "tpm_conv1_b", "tpm_lin_w", "tpm_lin_b", "tpm_gn_w", "tpm_gn_b", "tpm_conv2_w",
@@ -72,6 +79,7 @@ EXPORTS = {
     "tpdm_create": (C.c_int, [C.POINTER(TpdmConfig), C.POINTER(vp)]),
     "tpdm_destroy": (C.c_int, [vp]),
     "tpdm_set_weights": (C.c_int, [vp, C.POINTER(TpdmWeights)]),
+    "tpdm_set_fp8_weights": (C.c_int, [vp, C.POINTER(TpdmFp8BlockWeights)]),
     "tpdm_plan_workspace_bytes": (C.c_size_t, [vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     "tpdm_plan_create": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, C.c_size_t, C.POINTER(vp)]),
     "tpdm_plan_destroy": (C.c_int, [vp]),
@@ -119,6 +127,9 @@ EXPORTS = {
     "tpdm_conv3x3_nhwc": (C.c_int, [vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
     "tpdm_conv3x3_wgrad": (C.c_int, [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
     "tpdm_ln_modulate": (C.c_int, [vp, vp, vp, C.c_int, vp, C.c_int, C.c_int, C.c_int, vp]),
+    "tpdm_quantize_fp8_rows": (C.c_int, [vp, C.c_int, C.c_int, vp, vp, vp]),
+    "tpdm_ln_modulate_fp8": (C.c_int, [vp, vp, vp, C.c_int, vp, vp, C.c_int, C.c_int, C.c_int, vp]),
+    "tpdm_gemm_fp8": (C.c_int, [vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
 }
 
 _lib = None

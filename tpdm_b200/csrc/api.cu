@@ -21,6 +21,8 @@ struct tpdm_ctx {
   int D = 0, dp = 0, Dp = 0, R = 0, device = 0;
   std::vector<int> mod_off;  // first adaLN row of block i (norm1 rows, then norm1_context rows)
   bool any_dual = false;
+  std::vector<tpdm_fp8_block_weights> fp8;  // tpdm_set_fp8_weights; empty = bf16 everywhere
+  bool planned = false;                     // a plan was created: the GEMM operand types are fixed from then on
   bool dual(int i) const { return i < 64 && ((cfg.dual_attention_mask >> i) & 1ull) != 0; }
   int norm1_rows(int i) const { return (dual(i) ? 9 : 6) * D; }
 };
@@ -58,6 +60,8 @@ struct tpdm_plan {
   float *x_img, *x_ctx, *ctx0, *mod, *temb, *tproj, *thid, *text_part, *phid, *pout;
   bf16 *xn_img, *xn_ctx, *qkv, *attn_o, *ff_img, *ff_ctx, *enc_bf16;
   bf16 *xn2_img = nullptr, *qkv2 = nullptr, *attn_o2 = nullptr;  // dual-attention blocks only
+  uint8_t *xn8_img = nullptr, *xn8_ctx = nullptr;  // FP8 mode: E4M3 QKV / FF1 inputs and their row scales
+  float *xs_img = nullptr, *xs_ctx = nullptr;
   // TimePredictor
   bf16* tpm_x;
   float *y1, *y1p, *a2, *y2, *tpm_emb, *temb_cfg, *alpha_beta;
@@ -134,6 +138,12 @@ void carve(tpdm_plan* p, Carver& c) {
     p->qkv2 = c.take<bf16>(Bt * N * 3 * Dp);
     p->attn_o2 = c.take<bf16>(Bt * N * Dp);
   }
+  if (!ctx->fp8.empty()) {
+    p->xn8_img = c.take<uint8_t>(Bt * N * D);
+    p->xn8_ctx = c.take<uint8_t>(Bt * T * D);
+    p->xs_img = c.take<float>(Bt * N);
+    p->xs_ctx = c.take<float>(Bt * T);
+  }
   p->ff_img = c.take<bf16>(Bt * N * 4 * D);
   p->ff_ctx = c.take<bf16>(Bt * T * 4 * D);
   p->enc_bf16 = c.take<bf16>(Bt * T * ctx->cfg.joint_attention_dim);
@@ -201,18 +211,31 @@ int build_ops(tpdm_plan* p) {
     float* mod_img = p->mod + ctx->mod_off[i];
     float* mod_ctx = mod_img + ctx->norm1_rows(i);
     o.dual = ctx->dual(i);
+    const bool fp8 = !ctx->fp8.empty();
     // fused QKV: image rows land at tokens [0,N), text rows at [N,S) of the joint qkv buffer
-    TPDM_TRY(gemm_op_init(&o.qkv[0], p->xn_img, D, static_cast<long long>(N) * D, N, Bt, D, bw.qkv_w, 3 * Dp, EPI_BIAS_BF16, p->qkv,
-                          static_cast<long long>(S) * 3 * Dp, 3 * Dp, bw.qkv_b, nullptr, 0));
-    TPDM_TRY(gemm_op_init(&o.qkv[1], p->xn_ctx, D, static_cast<long long>(T) * D, T, Bt, D, bw.cqkv_w, 3 * Dp, EPI_BIAS_BF16,
-                          p->qkv + static_cast<size_t>(N) * 3 * Dp, static_cast<long long>(S) * 3 * Dp, 3 * Dp, bw.cqkv_b, nullptr, 0));
+    if (fp8) {
+      const tpdm_fp8_block_weights& fw = ctx->fp8[i];
+      TPDM_TRY(gemm_op_init_fp8(&o.qkv[0], p->xn8_img, D, static_cast<long long>(N) * D, p->xs_img, N, Bt, D, fw.qkv_w, fw.qkv_s, 3 * Dp,
+                                EPI_BIAS_BF16, p->qkv, static_cast<long long>(S) * 3 * Dp, 3 * Dp, bw.qkv_b));
+      TPDM_TRY(gemm_op_init_fp8(&o.qkv[1], p->xn8_ctx, D, static_cast<long long>(T) * D, p->xs_ctx, T, Bt, D, fw.cqkv_w, fw.cqkv_s, 3 * Dp,
+                                EPI_BIAS_BF16, p->qkv + static_cast<size_t>(N) * 3 * Dp, static_cast<long long>(S) * 3 * Dp, 3 * Dp, bw.cqkv_b));
+    } else {
+      TPDM_TRY(gemm_op_init(&o.qkv[0], p->xn_img, D, static_cast<long long>(N) * D, N, Bt, D, bw.qkv_w, 3 * Dp, EPI_BIAS_BF16, p->qkv,
+                            static_cast<long long>(S) * 3 * Dp, 3 * Dp, bw.qkv_b, nullptr, 0));
+      TPDM_TRY(gemm_op_init(&o.qkv[1], p->xn_ctx, D, static_cast<long long>(T) * D, T, Bt, D, bw.cqkv_w, 3 * Dp, EPI_BIAS_BF16,
+                            p->qkv + static_cast<size_t>(N) * 3 * Dp, static_cast<long long>(S) * 3 * Dp, 3 * Dp, bw.cqkv_b, nullptr, 0));
+    }
     TPDM_TRY(attn_op_init(&o.attn, p->qkv, Bt, S, ctx->cfg.num_heads, ctx->dp, ctx->cfg.head_dim, p->attn_o));
     if (last) o.attn.q_tiles = (N + 127) / 128;  // context_pre_only: text-query rows are never used
     // output projections: x += gate_msa * (o W^T + b)
     TPDM_TRY(gemm_op_init(&o.out[0], p->attn_o, Dp, static_cast<long long>(S) * Dp, N, Bt, Dp, bw.out_w, D, EPI_GATE_RESIDUAL, p->x_img,
                           static_cast<long long>(N) * D, D, bw.out_b, mod_img + 2 * D, R));
-    TPDM_TRY(gemm_op_init(&o.ff1[0], p->xn_img, D, static_cast<long long>(N) * D, N, Bt, D, bw.ff1_w, 4 * D, EPI_BIAS_GELU_BF16,
-                          p->ff_img, static_cast<long long>(N) * 4 * D, 4 * D, bw.ff1_b, nullptr, 0));
+    if (fp8)
+      TPDM_TRY(gemm_op_init_fp8(&o.ff1[0], p->xn8_img, D, static_cast<long long>(N) * D, p->xs_img, N, Bt, D, ctx->fp8[i].ff1_w, ctx->fp8[i].ff1_s,
+                                4 * D, EPI_BIAS_GELU_BF16, p->ff_img, static_cast<long long>(N) * 4 * D, 4 * D, bw.ff1_b));
+    else
+      TPDM_TRY(gemm_op_init(&o.ff1[0], p->xn_img, D, static_cast<long long>(N) * D, N, Bt, D, bw.ff1_w, 4 * D, EPI_BIAS_GELU_BF16,
+                            p->ff_img, static_cast<long long>(N) * 4 * D, 4 * D, bw.ff1_b, nullptr, 0));
     TPDM_TRY(gemm_op_init(&o.ff2[0], p->ff_img, 4 * D, static_cast<long long>(N) * 4 * D, N, Bt, 4 * D, bw.ff2_w, D, EPI_GATE_RESIDUAL,
                           p->x_img, static_cast<long long>(N) * D, D, bw.ff2_b, mod_img + 5 * D, R));
     if (o.dual) {
@@ -228,8 +251,12 @@ int build_ops(tpdm_plan* p) {
       TPDM_CHECK(bw.cout_w && bw.cff1_w && bw.cff2_w, TPDM_ERR_ARG, "block %d: missing context-stream weights", i);
       TPDM_TRY(gemm_op_init(&o.out[1], p->attn_o + static_cast<size_t>(N) * Dp, Dp, static_cast<long long>(S) * Dp, T, Bt, Dp, bw.cout_w,
                             D, EPI_GATE_RESIDUAL, p->x_ctx, static_cast<long long>(T) * D, D, bw.cout_b, mod_ctx + 2 * D, R));
-      TPDM_TRY(gemm_op_init(&o.ff1[1], p->xn_ctx, D, static_cast<long long>(T) * D, T, Bt, D, bw.cff1_w, 4 * D, EPI_BIAS_GELU_BF16,
-                            p->ff_ctx, static_cast<long long>(T) * 4 * D, 4 * D, bw.cff1_b, nullptr, 0));
+      if (fp8)
+        TPDM_TRY(gemm_op_init_fp8(&o.ff1[1], p->xn8_ctx, D, static_cast<long long>(T) * D, p->xs_ctx, T, Bt, D, ctx->fp8[i].cff1_w,
+                                  ctx->fp8[i].cff1_s, 4 * D, EPI_BIAS_GELU_BF16, p->ff_ctx, static_cast<long long>(T) * 4 * D, 4 * D, bw.cff1_b));
+      else
+        TPDM_TRY(gemm_op_init(&o.ff1[1], p->xn_ctx, D, static_cast<long long>(T) * D, T, Bt, D, bw.cff1_w, 4 * D, EPI_BIAS_GELU_BF16,
+                              p->ff_ctx, static_cast<long long>(T) * 4 * D, 4 * D, bw.cff1_b, nullptr, 0));
       TPDM_TRY(gemm_op_init(&o.ff2[1], p->ff_ctx, 4 * D, static_cast<long long>(T) * 4 * D, T, Bt, 4 * D, bw.cff2_w, D,
                             EPI_GATE_RESIDUAL, p->x_ctx, static_cast<long long>(T) * D, D, bw.cff2_b, mod_ctx + 5 * D, R));
     }
@@ -260,6 +287,15 @@ int set_prompts(tpdm_plan* p, const float* enc_a, const float* enc_b, const floa
   return 0;
 }
 
+// FP8 mode: the LN-modulate feeding QKV / FF1 writes E4M3 rows + row scales (image stream seg[0], text stream seg[1])
+void set_fp8_out(const tpdm_plan* p, LnSeg (&seg)[2]) {
+  if (p->xn8_img == nullptr) return;
+  seg[0].out8 = p->xn8_img;
+  seg[0].out_scale = p->xs_img;
+  seg[1].out8 = p->xn8_ctx;
+  seg[1].out_scale = p->xs_ctx;
+}
+
 // CustomSD3Transformer2DModel.forward minus the sigma-independent part
 int run_mmdit(tpdm_plan* p, const float* latents, int Bl, int dup, const float* timestep, int t_stride, float t_scale, int t_rep,
               float* h1_out, float* h2_out, bool tpm_taps, cudaStream_t s) {
@@ -287,6 +323,7 @@ int run_mmdit(tpdm_plan* p, const float* latents, int Bl, int dup, const float* 
     seg[0] = LnSeg{p->x_img, p->xn_img, mi, mi + D, N, Bt, R};
     // last block: AdaLayerNormContinuous chunk order is (scale, shift)
     seg[1] = last ? LnSeg{p->x_ctx, p->xn_ctx, mc + D, mc, T, Bt, R} : LnSeg{p->x_ctx, p->xn_ctx, mc, mc + D, T, Bt, R};
+    set_fp8_out(p, seg);
     TPDM_TRY(k_ln_modulate(seg, 2, D, s));
     if (o.dual) {  // norm_hidden_states2 = LN(x) * (1 + scale_msa2) + shift_msa2, from x BEFORE the first attention is added
       LnSeg seg2{p->x_img, p->xn2_img, mi + 6 * D, mi + 7 * D, N, Bt, R};
@@ -308,6 +345,7 @@ int run_mmdit(tpdm_plan* p, const float* latents, int Bl, int dup, const float* 
     }
     seg[0] = LnSeg{p->x_img, p->xn_img, mi + 3 * D, mi + 4 * D, N, Bt, R};
     seg[1] = LnSeg{p->x_ctx, p->xn_ctx, mc + 3 * D, mc + 4 * D, T, Bt, R};
+    set_fp8_out(p, seg);
     TPDM_TRY(k_ln_modulate(seg, o.n_streams, D, s));
     TPDM_TRY(gemm_launch(o.ff1, o.n_streams, s));
     TPDM_TRY(gemm_launch(o.ff2, o.n_streams, s));
@@ -422,6 +460,20 @@ int tpdm_set_weights(tpdm_ctx* ctx, const tpdm_weights* w) {
   return 0;
 }
 
+int tpdm_set_fp8_weights(tpdm_ctx* ctx, const tpdm_fp8_block_weights* blocks) {
+  TPDM_CHECK(ctx && blocks, TPDM_ERR_ARG, "tpdm_set_fp8_weights: null argument");
+  TPDM_CHECK(ctx->has_mmdit, TPDM_ERR_STATE, "tpdm_set_fp8_weights: call tpdm_set_weights with MMDiT weights first");
+  TPDM_CHECK(!ctx->planned, TPDM_ERR_STATE, "tpdm_set_fp8_weights: a plan of this ctx already exists (set FP8 weights before the first plan)");
+  const int L = ctx->cfg.num_layers;
+  for (int i = 0; i < L; ++i) {
+    const tpdm_fp8_block_weights& b = blocks[i];
+    TPDM_CHECK(b.qkv_w && b.qkv_s && b.cqkv_w && b.cqkv_s && b.ff1_w && b.ff1_s && (i == L - 1 || (b.cff1_w && b.cff1_s)), TPDM_ERR_ARG,
+               "tpdm_set_fp8_weights: block %d is missing FP8 weights or scales", i);
+  }
+  ctx->fp8.assign(blocks, blocks + L);
+  return 0;
+}
+
 size_t tpdm_plan_workspace_bytes(const tpdm_ctx* ctx, int batch, int cfg_pairs, int latent_h, int latent_w, int n_text, int max_steps) {
   if (check_shapes(ctx, batch, latent_h, latent_w, n_text, max_steps) != 0) return 0;
   tpdm_plan p;
@@ -468,6 +520,7 @@ int tpdm_plan_create(tpdm_ctx* ctx, int batch, int cfg_pairs, int latent_h, int 
     delete p;
     return st;
   }
+  ctx->planned = true;
   *out = p;
   return 0;
 }
@@ -887,6 +940,28 @@ int tpdm_ln_modulate(const float* x, const float* shift, const float* scale, int
   TPDM_CHECK(x && shift && scale && out_bf16, TPDM_ERR_ARG, "tpdm_ln_modulate: null argument");
   LnSeg seg{x, reinterpret_cast<bf16*>(out_bf16), shift, scale, rows, batch, mod_stride};
   return k_ln_modulate(&seg, 1, D, static_cast<cudaStream_t>(stream));
+}
+
+int tpdm_quantize_fp8_rows(const float* x, int rows, int K, void* codes, float* scales, void* stream) {
+  TPDM_CHECK(x && codes && scales, TPDM_ERR_ARG, "tpdm_quantize_fp8_rows: null argument");
+  return k_quantize_fp8_rows(x, rows, K, static_cast<uint8_t*>(codes), scales, static_cast<cudaStream_t>(stream));
+}
+
+int tpdm_ln_modulate_fp8(const float* x, const float* shift, const float* scale, int mod_stride, void* out_codes, float* out_scales,
+                         int batch, int rows, int D, void* stream) {
+  TPDM_CHECK(x && shift && scale && out_codes && out_scales, TPDM_ERR_ARG, "tpdm_ln_modulate_fp8: null argument");
+  LnSeg seg{x, nullptr, shift, scale, rows, batch, mod_stride, static_cast<uint8_t*>(out_codes), out_scales};
+  return k_ln_modulate(&seg, 1, D, static_cast<cudaStream_t>(stream));
+}
+
+int tpdm_gemm_fp8(const void* A8, const float* a_scale, const void* W8, const float* w_scale, const float* bias, void* out, int batch,
+                  int rows, int N, int K, int epi, void* stream) {
+  TPDM_CHECK(A8 && a_scale && W8 && w_scale && out, TPDM_ERR_ARG, "tpdm_gemm_fp8: null argument");
+  TPDM_CHECK(epi >= 0 && epi <= 2, TPDM_ERR_ARG, "tpdm_gemm_fp8: epilogue %d unknown", epi);
+  GemmOp op;
+  TPDM_TRY(gemm_op_init_fp8(&op, A8, K, static_cast<long long>(rows) * K, a_scale, rows, batch, K, W8, w_scale, N, epi, out,
+                            static_cast<long long>(rows) * N, N, bias));
+  return gemm_launch(&op, 1, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

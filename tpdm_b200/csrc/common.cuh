@@ -197,6 +197,12 @@ __host__ __device__ constexpr uint32_t make_idesc_bf16(uint32_t M, uint32_t N, b
          | ((b_mn_major ? 1u : 0u) << 16) | ((N >> 3) << 17) | ((M >> 4) << 24);
 }
 
+// kind::f8f6f4 instruction descriptor: fp32 accumulate, E4M3 A/B (format code 0), both K-major.
+__host__ __device__ constexpr uint32_t make_idesc_e4m3(uint32_t M, uint32_t N) {
+  return (1u << 4)  // c_format = F32; a_format = b_format = E4M3 (0)
+         | ((N >> 3) << 17) | ((M >> 4) << 24);
+}
+
 // shared-memory matrix descriptor, 128-byte swizzle.  K-major: rows of 64 bf16 (128 B), 8-row atoms 1024 B apart
 // (SBO = 1024).  MN-major: 64 MN-elements contiguous per K row, 8-K atoms SBO apart, 64-element MN groups LBO apart.
 __device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
@@ -279,6 +285,18 @@ __device__ __forceinline__ float exp2_approx(float x) {
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
   __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
   return *reinterpret_cast<uint32_t*>(&v);
+}
+// The one E4M3 row quantizer of the library (ln_modulate's FP8 output and the load-time weight quantizer both call it, so a
+// torch restatement reproduces the codes bit for bit): amax = max |y| over the row, codes = cvt.rn.satfinite(y * (448 / amax)),
+// stored scale = amax / 448 (both divisions IEEE round-to-nearest), so y ~= code * scale.  A zero row gets scale 1 and zero codes.
+__device__ __forceinline__ float fp8_row_inv_scale(float amax) { return amax > 0.f ? __fdiv_rn(448.f, amax) : 1.f; }
+__device__ __forceinline__ float fp8_row_scale(float amax) { return amax > 0.f ? __fdiv_rn(amax, 448.f) : 1.f; }
+// four values -> four E4M3 codes, first value in the lowest byte
+__device__ __forceinline__ uint32_t pack_e4m3x4(float a, float b, float c, float d, float inv) {
+  uint16_t lo, hi;
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(lo) : "f"(__fmul_rn(b, inv)), "f"(__fmul_rn(a, inv)));
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(hi) : "f"(__fmul_rn(d, inv)), "f"(__fmul_rn(c, inv)));
+  return static_cast<uint32_t>(lo) | (static_cast<uint32_t>(hi) << 16);
 }
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

@@ -29,6 +29,10 @@ constexpr int BN2 = 256;
 #endif
 constexpr int BK = TPDM_GEMM2_BK;   // k-block per pipeline stage: 64 (one 128-byte swizzle atom row) or 128 (two, side by side)
 constexpr int kSub = BK / 64;       // 64-wide TMA boxes per operand and stage
+// E4M3 instantiation: a 128-byte swizzle row holds 128 one-byte elements, so every byte offset, stage size and ring depth below is
+// unchanged and only the element counts along K double (a stage covers 2 * BK elements, each MMA K = 32)
+template <bool kFp8>
+constexpr int kElemsPerRow = kFp8 ? 128 : 64;
 constexpr int kStages2 = BK == 64 ? 5 : 3;
 constexpr int kEpiWarps2 = 8;   // two warps per TMEM lane quarter, each draining half of the tile's columns
 constexpr int kThreads2 = 64 + 32 * kEpiWarps2;
@@ -129,6 +133,15 @@ __device__ __forceinline__ void umma2_ss_elect(uint32_t d_tmem, uint64_t a_desc,
       "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+__device__ __forceinline__ void umma2_ss_elect_e4m3(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p, e;\n\t"
+      "elect.sync _|e, 0xffffffff;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "@e tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(d_tmem),
+      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 __device__ __forceinline__ void umma2_commit_multicast_elect(uint64_t* bar) {
   asm volatile(
       "{\n\t.reg .pred e;\n\t"
@@ -144,7 +157,11 @@ __device__ __forceinline__ void umma2_commit_multicast(uint64_t* bar) {
                : "memory");
 }
 
+// kFp8: E4M3 x E4M3 -> fp32 (kind::f8f6f4) with the scaled epilogue; otherwise bf16 x bf16 -> fp32 (kind::f16)
+template <bool kFp8>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1) gemm2_bf16_tcgen05_kernel(const __grid_constant__ Gemm2Params P) {
+  constexpr int kRowElems = kElemsPerRow<kFp8>;
+  constexpr int kStageK = kSub * kRowElems;  // K elements per stage
   pdl_launch_dependents();
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -197,7 +214,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1) gemm2_
         const PairCoord tc = decode_pair(P, tile);
         if (P.bmask != nullptr && P.bmask[tc.b % P.bslots] == 0) continue;
         const GemmOp& G = P.op[tc.g];
-        const int nkb = (G.K + BK - 1) / BK;
+        const int nkb = (G.K + kStageK - 1) / kStageK;
         const int m0 = tc.mtp * 2 * BM + static_cast<int>(rank) * BM;
         const int nb0 = tc.nt * BN2 + static_cast<int>(rank) * (BN2 / 2);
         for (int kb = 0; kb < nkb; ++kb) {
@@ -208,8 +225,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1) gemm2_
           mbar_arrive_expect_tx_cluster(leader_full, kStageBytes2);
 #pragma unroll
           for (int h = 0; h < kSub; ++h) {
-            tma2_load_3d(sA + h * (BM * 128), &G.tmA, leader_full, kb * BK + h * 64, m0, tc.b);
-            tma2_load_2d(sB + h * ((BN2 / 2) * 128), &G.tmB2, leader_full, kb * BK + h * 64, nb0);
+            tma2_load_3d(sA + h * (BM * 128), &G.tmA, leader_full, kb * kStageK + h * kRowElems, m0, tc.b);
+            tma2_load_2d(sB + h * ((BN2 / 2) * 128), &G.tmB2, leader_full, kb * kStageK + h * kRowElems, nb0);
           }
           if (++stage == kStages2) {
             stage = 0;
@@ -221,7 +238,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1) gemm2_
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer (leader CTA only)
     if (rank == 0) {
-      constexpr uint32_t idesc = make_idesc_bf16(2 * BM, BN2);
+      constexpr uint32_t idesc = kFp8 ? make_idesc_e4m3(2 * BM, BN2) : make_idesc_bf16(2 * BM, BN2);
       int stage = 0;
       uint32_t phase = 0;
       int acc = 0;
@@ -230,7 +247,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1) gemm2_
         const PairCoord tc = decode_pair(P, tile);
         if (P.bmask != nullptr && P.bmask[tc.b % P.bslots] == 0) continue;
         const GemmOp& G = P.op[tc.g];
-        const int nkb = (G.K + BK - 1) / BK;
+        const int nkb = (G.K + kStageK - 1) / kStageK;
 #ifdef TPDM_GEMM_TRACE
         const bool tr = cluster_id == 0 && lane == 0;
         long long tq0 = 0;
@@ -260,12 +277,16 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1) gemm2_
           {
             const uint32_t a_base = smem_u32(smem + stage * kStageBytes2);
             const uint32_t b_base = a_base + kABytes2;
-            // descriptors of the stage once; the sixteen-element k steps advance the 14-bit start-address field (units of 16 B)
+            // descriptors of the stage once; the 32-byte k steps (16 bf16 or 32 E4M3 elements) advance the 14-bit start-address
+            // field (units of 16 B)
             const uint64_t adesc0 = make_smem_desc_sw128(a_base, 16, 1024), bdesc0 = make_smem_desc_sw128(b_base, 16, 1024);
 #pragma unroll
             for (int k = 0; k < BK / 16; ++k) {
               const uint32_t ao = ((k / 4) * (BM * 128) + (k % 4) * 32) >> 4, bo = ((k / 4) * ((BN2 / 2) * 128) + (k % 4) * 32) >> 4;
-              umma2_ss_elect(d_tmem, adesc0 + ao, bdesc0 + bo, idesc, (kb | k) != 0 ? 1u : 0u);
+              if constexpr (kFp8)
+                umma2_ss_elect_e4m3(d_tmem, adesc0 + ao, bdesc0 + bo, idesc, (kb | k) != 0 ? 1u : 0u);
+              else
+                umma2_ss_elect(d_tmem, adesc0 + ao, bdesc0 + bo, idesc, (kb | k) != 0 ? 1u : 0u);
             }
             umma2_commit_multicast_elect(&empty_bar[stage]);
             if (kb == nkb - 1) umma2_commit_multicast_elect(&tmem_full[acc]);
@@ -305,7 +326,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1) gemm2_
       const GemmOp& G = P.op[tc.g];
       const int n0 = tc.nt * BN2;
       const int row_base = tc.mtp * 2 * BM + static_cast<int>(rank) * BM + q * 32;
-      gemm_epilogue_tile<BN2>(
+      gemm_epilogue_tile<BN2, kFp8>(
           G, tc.b, row_base, n0, tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * BN2, st, sbias, lane, hh * (BN2 / 64), (hh + 1) * (BN2 / 64),
           [&]() { mbar_wait_backoff(&tmem_full[acc], acc_phase); },
           [&]() {
@@ -350,8 +371,10 @@ int gemm2_launch(const GemmOp* ops, int n_ops, cudaStream_t stream) {
   P.bmask = batch_mask();
   P.bslots = batch_mask_slots();
   double flops = 0;
+  const bool fp8 = ops[0].fp8 != 0;
   for (int i = 0; i < n_ops; ++i) {
     TPDM_CHECK(ops[i].conv == 0 && ops[i].block_n == 256, TPDM_ERR_ARG, "gemm2_launch: plain GEMMs with 256-wide N tiles only");
+    TPDM_CHECK((ops[i].fp8 != 0) == fp8, TPDM_ERR_ARG, "gemm2_launch: grouped ops must share the operand type");
     P.op[i] = ops[i];
     const int tiles_mp = (ops[i].rows_per_batch + 2 * BM - 1) / (2 * BM);
     const int t = ops[i].batch * tiles_mp * ops[i].tiles_n;
@@ -360,15 +383,17 @@ int gemm2_launch(const GemmOp* ops, int n_ops, cudaStream_t stream) {
     flops += 2.0 * ops[i].batch * ops[i].rows_per_batch * static_cast<double>(ops[i].N) * ops[i].K;
   }
   if (n_ops == 1) P.op[1] = ops[0];
-  static bool attr_set = false;
-  if (!attr_set) {
-    TPDM_CUDA_OK(cudaFuncSetAttribute(gemm2_bf16_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem2));
-    attr_set = true;
+  static bool attr_set[2] = {false, false};
+  if (!attr_set[fp8]) {
+    TPDM_CUDA_OK(cudaFuncSetAttribute(fp8 ? gemm2_bf16_tcgen05_kernel<true> : gemm2_bf16_tcgen05_kernel<false>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem2));
+    attr_set[fp8] = true;
   }
   const int max_clusters = num_sms() / 2;
   const int clusters = P.total_tiles < max_clusters ? P.total_tiles : max_clusters;
   prof_begin(0, flops, stream);
-  TPDM_CUDA_OK(launch_pdl(gemm2_bf16_tcgen05_kernel, dim3(2 * clusters), dim3(kThreads2), kSmem2, stream, P));
+  TPDM_CUDA_OK(launch_pdl(fp8 ? gemm2_bf16_tcgen05_kernel<true> : gemm2_bf16_tcgen05_kernel<false>, dim3(2 * clusters), dim3(kThreads2), kSmem2,
+                          stream, P));
   prof_end(stream);
   count_launch();
   TPDM_CUDA_OK(cudaGetLastError());

@@ -20,7 +20,9 @@ constexpr int kStagePad = 36;  // floats per staged row: 16-byte aligned rows, c
 // once its last TMEM load has landed in registers.
 // The warp handles the 32-column chunks [c_begin, c_end) of the tile (all of them in the 1-CTA kernel; half of them in the
 // CTA-pair kernel, where two warps share each TMEM lane quarter).  sbias holds 2 * 32 * (c_end - c_begin) floats.
-template <int BN, typename WaitFn, typename ReleaseFn>
+// kScaled (E4M3 operands): y = acc * a_scale[b][row] * w_scale[col] + bias before the store; w_scale is staged in the gate half
+// of sbias, which the bf16 / plain fp32 modes leave unused, and each lane reads its row's a_scale once per tile.
+template <int BN, bool kScaled = false, typename WaitFn, typename ReleaseFn>
 __device__ __forceinline__ void gemm_epilogue_tile(const GemmOp& G, int batch_idx, int row_base, int n0, uint32_t tmem_acc, float* st,
                                                    float* sbias, int lane, int c_begin, int c_end, WaitFn wait_accumulator,
                                                    ReleaseFn release_accumulator) {
@@ -70,11 +72,19 @@ __device__ __forceinline__ void gemm_epilogue_tile(const GemmOp& G, int batch_id
         if (col < G.N) {
           if (G.bias) b4 = *reinterpret_cast<const float4*>(G.bias + col);
           if (resid) g4 = *reinterpret_cast<const float4*>(gate_row + col);
+          if constexpr (kScaled) g4 = *reinterpret_cast<const float4*>(G.w_scale + col);
         }
         *reinterpret_cast<float4*>(sbias + k) = b4;
         *reinterpret_cast<float4*>(sbias + ncol + k) = g4;
       }
       __syncwarp();
+      // kScaled: a_s = this lane's row scale (bf16 path, lane = row); a_r[it] = the scale of row it * 4 + r_in (fp32 path)
+      float a_s = 0.f, a_r[8];
+      if constexpr (kScaled) {
+        if (lane < rows) a_s = G.a_scale[static_cast<long long>(batch_idx) * G.rows_per_batch + row_base + lane];
+#pragma unroll
+        for (int it = 0; it < 8; ++it) a_r[it] = __shfl_sync(0xffffffffu, a_s, it * 4 + r_in);
+      }
       float4 resv_a[8], resv_b[8];
       if (resid) {
         if (lane < rows) {
@@ -119,6 +129,13 @@ __device__ __forceinline__ void gemm_epilogue_tile(const GemmOp& G, int batch_id
                             __uint_as_float(v[8 * q + 2]) + b0.z, __uint_as_float(v[8 * q + 3]) + b0.w,
                             __uint_as_float(v[8 * q + 4]) + b1.x, __uint_as_float(v[8 * q + 5]) + b1.y,
                             __uint_as_float(v[8 * q + 6]) + b1.z, __uint_as_float(v[8 * q + 7]) + b1.w};
+              if constexpr (kScaled) {
+                const float4 s0 = *reinterpret_cast<const float4*>(sb + ncol + 8 * q);
+                const float4 s1 = *reinterpret_cast<const float4*>(sb + ncol + 8 * q + 4);
+                const float ws[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w}, bs[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+#pragma unroll
+                for (int e = 0; e < 8; ++e) y[e] = fmaf(__uint_as_float(v[8 * q + e]) * a_s, ws[e], bs[e]);
+              }
               if (gelu) {
 #pragma unroll
                 for (int e = 0; e < 8; ++e) y[e] = gelu_tanh(y[e]);
@@ -153,6 +170,9 @@ __device__ __forceinline__ void gemm_epilogue_tile(const GemmOp& G, int batch_id
               if (r < rows) {
                 const float4 x = *reinterpret_cast<const float4*>(st + r * kStagePad + cg * 4);
                 float4 y = make_float4(x.x + bias[0], x.y + bias[1], x.z + bias[2], x.w + bias[3]);
+                if constexpr (kScaled)
+                  y = make_float4(fmaf(x.x * a_r[it], gate[0], bias[0]), fmaf(x.y * a_r[it], gate[1], bias[1]), fmaf(x.z * a_r[it], gate[2], bias[2]),
+                                  fmaf(x.w * a_r[it], gate[3], bias[3]));
                 if (resid)
                   y = make_float4(resv[it].x + gate[0] * y.x, resv[it].y + gate[1] * y.y, resv[it].z + gate[2] * y.z,
                                   resv[it].w + gate[3] * y.w);

@@ -299,6 +299,47 @@ int gemm_op_init(GemmOp* op, const void* A, long long a_row_stride, long long a_
   return finish_op(op, W, N, K, epi, out, out_batch_stride, ldo, bias, gate, gate_stride);
 }
 
+int gemm_op_init_fp8(GemmOp* op, const void* A, long long a_row_stride, long long a_batch_stride, const float* a_scale, int rows_per_batch,
+                     int batch, int K, const void* W, const float* w_scale, int N, int epi, void* out, long long out_batch_stride, int ldo,
+                     const float* bias) {
+  *op = GemmOp{};
+  TPDM_CHECK(rows_per_batch > 0 && batch > 0 && K > 0 && N > 0, TPDM_ERR_SHAPE, "gemm fp8: empty problem");
+  TPDM_CHECK(epi == EPI_BIAS_BF16 || epi == EPI_BIAS_F32 || epi == EPI_BIAS_GELU_BF16, TPDM_ERR_ARG, "gemm fp8: epilogue %d unsupported", epi);
+  TPDM_CHECK(N > 128, TPDM_ERR_SHAPE, "gemm fp8: N=%d must exceed 128 (CTA-pair kernel, 256-wide N tiles)", N);
+  TPDM_CHECK(K % 16 == 0 && a_row_stride % 16 == 0, TPDM_ERR_SHAPE, "gemm fp8: K=%d and the A row stride must be multiples of 16", K);
+  TPDM_CHECK(a_scale != nullptr && w_scale != nullptr && (reinterpret_cast<uintptr_t>(w_scale) & 15) == 0, TPDM_ERR_ARG,
+             "gemm fp8: a_scale and a 16-byte aligned w_scale are required");
+  op->rows_per_batch = rows_per_batch;
+  op->batch = batch;
+  op->tiles_m_per_batch = (rows_per_batch + BM - 1) / BM;
+  op->conv = 0;
+  op->fp8 = 1;
+  op->a_scale = a_scale;
+  op->w_scale = w_scale;
+  op->N = N;
+  op->K = K;
+  op->block_n = 256;
+  op->tiles_n = (N + 255) / 256;
+  op->num_tiles = batch * op->tiles_m_per_batch * op->tiles_n;
+  op->epi = epi;
+  op->out = out;
+  op->out_batch_stride = out_batch_stride;
+  op->ldo = ldo;
+  op->bias = bias;
+  TPDM_CHECK(N % 8 == 0 && ldo % 8 == 0, TPDM_ERR_SHAPE, "gemm fp8: N=%d and ldo=%d must be multiples of 8 (16-byte row segments)", N, ldo);
+  TPDM_CHECK((reinterpret_cast<uintptr_t>(out) & 15) == 0 && (reinterpret_cast<uintptr_t>(bias) & 15) == 0, TPDM_ERR_ARG,
+             "gemm fp8: out / bias must be 16-byte aligned");
+  // a 128-byte swizzle row is 128 E4M3 elements: boxes {128, rows}
+  uint64_t dims[3] = {static_cast<uint64_t>(K), static_cast<uint64_t>(rows_per_batch), static_cast<uint64_t>(batch)};
+  uint64_t strides[2] = {static_cast<uint64_t>(a_row_stride), static_cast<uint64_t>(batch > 1 ? a_batch_stride : a_row_stride * rows_per_batch)};
+  uint32_t box[3] = {128, BM, 1};
+  TPDM_TRY(encode_tmap(&op->tmA, CU_TENSOR_MAP_DATA_TYPE_UINT8, A, 3, dims, strides, box));
+  uint64_t wdims[2] = {static_cast<uint64_t>(K), static_cast<uint64_t>(N)};
+  uint64_t wstrides[1] = {static_cast<uint64_t>(K)};
+  uint32_t wbox[2] = {128, 128};
+  return encode_tmap(&op->tmB2, CU_TENSOR_MAP_DATA_TYPE_UINT8, W, 2, wdims, wstrides, wbox);
+}
+
 int gemm_op_init_conv3x3(GemmOp* op, const void* X, int batch, int g, int C, const void* W, int N, int epi, void* out,
                          int ldo, const float* bias) {
   *op = GemmOp{};
@@ -397,9 +438,10 @@ int gemm_launch(const GemmOp* ops, int n_ops, cudaStream_t stream) {
   for (int i = 0; i < n_ops; ++i) {
     P.op[i] = ops[i];
     P.total_tiles += ops[i].num_tiles;
-    TPDM_CHECK(ops[i].block_n == ops[0].block_n, TPDM_ERR_ARG, "gemm_launch: grouped ops must share the N tile");
+    TPDM_CHECK(ops[i].block_n == ops[0].block_n && ops[i].fp8 == ops[0].fp8, TPDM_ERR_ARG, "gemm_launch: grouped ops must share the N tile and operand type");
   }
   if (n_ops == 1) P.op[1] = ops[0];
+  if (ops[0].fp8) return gemm2_launch(ops, n_ops, stream);  // E4M3 operands exist only in the CTA-pair kernel
   // plain GEMMs with 256-wide N tiles go to the CTA-pair kernel (TPDM_GEMM_2CTA=0 forces the 1-CTA kernel)
   static const bool pair = getenv("TPDM_GEMM_2CTA") == nullptr || atoi(getenv("TPDM_GEMM_2CTA")) != 0;
   bool plain = ops[0].block_n == 256;

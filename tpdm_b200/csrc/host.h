@@ -74,6 +74,9 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
 // bf16 tiled tensor map with 128-byte swizzle.  dims/strides innermost first; strides (bytes) for dims 1..rank-1.
 int encode_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                      const uint32_t* box);
+// the same for any element type (E4M3 operands use CU_TENSOR_MAP_DATA_TYPE_UINT8)
+int encode_tmap(CUtensorMap* out, CUtensorMapDataType dtype, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
+                const uint32_t* box);
 
 // ------------------------------------------------------------------------------------------------------------
 // GEMM  (gemm_tcgen05.cu):  out = epilogue(A[rows x K] * W[N x K]^T)
@@ -96,20 +99,36 @@ struct alignas(64) GemmOp {
   int conv_bx = 0, conv_xt = 1;        // conv 1: pixels per tile row segment, tile segments per image row
   int ksplit = 1;                      // 1-CTA kernel: K is cut into `ksplit` ranges, range s writes out + (s*batch + b)*out_batch_stride
                                        // (partial sums, to be added by the consumer); see gemm_op_set_ksplit
-  const void* res = nullptr;           // EPI_BIAS_ADD_BF16: bf16 addend, indexed exactly like `out` (may alias it)
+  // E4M3 operands (gemm_op_init_fp8, CTA-pair kernel only): out = epilogue(acc * a_scale[b][row] * w_scale[n] + bias).  The two
+  // scale pointers share storage with `res` / `gate`, which no FP8 epilogue reads, so the struct keeps its 512 bytes.
+  int fp8 = 0;
+  union {
+    const void* res = nullptr;         // EPI_BIAS_ADD_BF16: bf16 addend, indexed exactly like `out` (may alias it)
+    const float* w_scale;              // fp8: [N]
+  };
   int wg_px, wg_bpr, wg_ctiles, wg_pad;
   void* out;
   long long out_batch_stride;  // elements between batches of the output
   int ldo;                     // output leading dimension (elements)
   int gate_stride;             // elements between batches of gate
   const float* bias;           // [N] or null
-  const float* gate;           // [batch][gate_stride] (EPI_GATE_RESIDUAL)
+  union {
+    const float* gate;         // [batch][gate_stride] (EPI_GATE_RESIDUAL)
+    const float* a_scale;      // fp8: [batch][rows_per_batch]
+  };
 };
+static_assert(sizeof(GemmOp) == 512, "GemmOp is a kernel parameter: its size sets the indexing of GemmParams::op[]");
 
 // A: bf16, element (b, r, k) at A + b*a_batch_stride + r*a_row_stride + k.   W: bf16 [N][K] row-major.
 int gemm_op_init(GemmOp* op, const void* A, long long a_row_stride, long long a_batch_stride, int rows_per_batch, int batch,
                  int K, const void* W, int N, int epi, void* out, long long out_batch_stride, int ldo, const float* bias,
                  const float* gate, int gate_stride);
+// A: E4M3 codes, element (b, r, k) at A + b*a_batch_stride + r*a_row_stride + k (strides in elements = bytes), a_scale fp32
+// [batch][rows_per_batch];  W: E4M3 [N][K] row-major, w_scale fp32 [N].  epi: EPI_BIAS_BF16, EPI_BIAS_F32 or EPI_BIAS_GELU_BF16;
+// N > 128 (256-wide N tiles of the CTA-pair kernel); K tails beyond a 128-element k-block are zero-filled by TMA.
+int gemm_op_init_fp8(GemmOp* op, const void* A, long long a_row_stride, long long a_batch_stride, const float* a_scale, int rows_per_batch,
+                     int batch, int K, const void* W, const float* w_scale, int N, int epi, void* out, long long out_batch_stride, int ldo,
+                     const float* bias);
 // implicit-GEMM 3x3 / pad 1 / stride 1 convolution over NHWC bf16 X[b][g][g][C]; W packed [N][9*C] (tap-major, tap=ky*3+kx).
 int gemm_op_init_conv3x3(GemmOp* op, const void* X, int batch, int g, int C, const void* W, int N, int epi, void* out,
                          int ldo, const float* bias);

@@ -300,7 +300,8 @@ __device__ __forceinline__ float4 ld4_stream(const float* p) {
   return r;
 }
 
-template <int VPL>
+// kFp8: the modulated row is written as E4M3 codes + one row scale (S.out8 / S.out_scale) instead of bf16
+template <int VPL, bool kFp8 = false>
 __global__ void __launch_bounds__(256) ln_modulate_kernel(const __grid_constant__ LnParams P) {
   pdl_launch_dependents();
   pdl_wait();
@@ -344,24 +345,64 @@ __global__ void __launch_bounds__(256) ln_modulate_kernel(const __grid_constant_
         ss += (a * a + bq * bq) + (c * c + d * d);
       }
       const float rstd = rsqrtf(warp_sum(ss) / P.D + 1e-6f);
+      if constexpr (kFp8) {
+        float am = 0.f;
 #pragma unroll
-      for (int i = 0; i < VPL; ++i) {
-        const int k = (i * 32 + lane) * 4;
-        const float4 h = *reinterpret_cast<const float4*>(ln_mod + k), c = *reinterpret_cast<const float4*>(ln_mod + P.D + k);
-        uint2 w;
-        w.x = pack_bf16x2((v[i].x - mean) * rstd * c.x + h.x, (v[i].y - mean) * rstd * c.y + h.y);
-        w.y = pack_bf16x2((v[i].z - mean) * rstd * c.z + h.z, (v[i].w - mean) * rstd * c.w + h.w);
-        *reinterpret_cast<uint2*>(o + k) = w;
+        for (int i = 0; i < VPL; ++i) {
+          const int k = (i * 32 + lane) * 4;
+          const float4 h = *reinterpret_cast<const float4*>(ln_mod + k), c = *reinterpret_cast<const float4*>(ln_mod + P.D + k);
+          v[i] = make_float4((v[i].x - mean) * rstd * c.x + h.x, (v[i].y - mean) * rstd * c.y + h.y, (v[i].z - mean) * rstd * c.z + h.z,
+                             (v[i].w - mean) * rstd * c.w + h.w);
+          am = fmaxf(am, fmaxf(fmaxf(fabsf(v[i].x), fabsf(v[i].y)), fmaxf(fabsf(v[i].z), fabsf(v[i].w))));
+        }
+        am = warp_max(am);
+        const float inv = fp8_row_inv_scale(am);
+        uint8_t* o8 = S.out8 + lr * P.D;
+#pragma unroll
+        for (int i = 0; i < VPL; ++i)
+          *reinterpret_cast<uint32_t*>(o8 + (i * 32 + lane) * 4) = pack_e4m3x4(v[i].x, v[i].y, v[i].z, v[i].w, inv);
+        if (lane == 0) S.out_scale[lr] = fp8_row_scale(am);
+      } else {
+#pragma unroll
+        for (int i = 0; i < VPL; ++i) {
+          const int k = (i * 32 + lane) * 4;
+          const float4 h = *reinterpret_cast<const float4*>(ln_mod + k), c = *reinterpret_cast<const float4*>(ln_mod + P.D + k);
+          uint2 w;
+          w.x = pack_bf16x2((v[i].x - mean) * rstd * c.x + h.x, (v[i].y - mean) * rstd * c.y + h.y);
+          w.y = pack_bf16x2((v[i].z - mean) * rstd * c.z + h.z, (v[i].w - mean) * rstd * c.w + h.w);
+          *reinterpret_cast<uint2*>(o + k) = w;
+        }
       }
     } else {
       float mean, rstd;
       row_stats(row, P.D, lane, mean, rstd);
-      for (int k = lane * 4; k < P.D; k += 128) {
-        const float4 v = ld4(row + k), h = *reinterpret_cast<const float4*>(ln_mod + k), c = *reinterpret_cast<const float4*>(ln_mod + P.D + k);
-        uint2 w;
-        w.x = pack_bf16x2((v.x - mean) * rstd * c.x + h.x, (v.y - mean) * rstd * c.y + h.y);
-        w.y = pack_bf16x2((v.z - mean) * rstd * c.z + h.z, (v.w - mean) * rstd * c.w + h.w);
-        *reinterpret_cast<uint2*>(o + k) = w;
+      if constexpr (kFp8) {  // generic width: one pass for the amax, one that recomputes the same values and stores the codes
+        auto mod4 = [&](int k) {
+          const float4 v = ld4(row + k), h = *reinterpret_cast<const float4*>(ln_mod + k), c = *reinterpret_cast<const float4*>(ln_mod + P.D + k);
+          return make_float4((v.x - mean) * rstd * c.x + h.x, (v.y - mean) * rstd * c.y + h.y, (v.z - mean) * rstd * c.z + h.z,
+                             (v.w - mean) * rstd * c.w + h.w);
+        };
+        float am = 0.f;
+        for (int k = lane * 4; k < P.D; k += 128) {
+          const float4 y = mod4(k);
+          am = fmaxf(am, fmaxf(fmaxf(fabsf(y.x), fabsf(y.y)), fmaxf(fabsf(y.z), fabsf(y.w))));
+        }
+        am = warp_max(am);
+        const float inv = fp8_row_inv_scale(am);
+        uint8_t* o8 = S.out8 + lr * P.D;
+        for (int k = lane * 4; k < P.D; k += 128) {
+          const float4 y = mod4(k);
+          *reinterpret_cast<uint32_t*>(o8 + k) = pack_e4m3x4(y.x, y.y, y.z, y.w, inv);
+        }
+        if (lane == 0) S.out_scale[lr] = fp8_row_scale(am);
+      } else {
+        for (int k = lane * 4; k < P.D; k += 128) {
+          const float4 v = ld4(row + k), h = *reinterpret_cast<const float4*>(ln_mod + k), c = *reinterpret_cast<const float4*>(ln_mod + P.D + k);
+          uint2 w;
+          w.x = pack_bf16x2((v.x - mean) * rstd * c.x + h.x, (v.y - mean) * rstd * c.y + h.y);
+          w.y = pack_bf16x2((v.z - mean) * rstd * c.z + h.z, (v.w - mean) * rstd * c.w + h.w);
+          *reinterpret_cast<uint2*>(o + k) = w;
+        }
       }
     }
   }
@@ -920,7 +961,7 @@ __device__ __forceinline__ void bulk_load_row(void* smem_dst, const void* gsrc, 
                : "memory");
 }
 
-template <int VPL>
+template <int VPL, bool kFp8 = false>
 __global__ void __launch_bounds__(256, 2) ln_modulate_bulk_kernel(const __grid_constant__ LnParams P) {
   pdl_launch_dependents();
   extern __shared__ __align__(128) float ln_smem[];  // [D] shift, [D] 1 + scale, then 8 warps x kLnSlots rows of D floats
@@ -989,6 +1030,26 @@ __global__ void __launch_bounds__(256, 2) ln_modulate_bulk_kernel(const __grid_c
       ss += (a * a + bq * bq) + (c * c + d * d);
     }
     const float rstd = rsqrtf(warp_sum(ss) / D + 1e-6f);
+    if constexpr (kFp8) {
+      float am = 0.f;
+#pragma unroll
+      for (int i = 0; i < VPL; ++i) {
+        const int k = (i * 32 + lane) * 4;
+        const float4 h = *reinterpret_cast<const float4*>(ln_smem + k), c = *reinterpret_cast<const float4*>(ln_smem + D + k);
+        v[i] = make_float4((v[i].x - mean) * rstd * c.x + h.x, (v[i].y - mean) * rstd * c.y + h.y, (v[i].z - mean) * rstd * c.z + h.z,
+                           (v[i].w - mean) * rstd * c.w + h.w);
+        am = fmaxf(am, fmaxf(fmaxf(fabsf(v[i].x), fabsf(v[i].y)), fmaxf(fabsf(v[i].z), fabsf(v[i].w))));
+      }
+      am = warp_max(am);
+      const float inv = fp8_row_inv_scale(am);
+      const long long lr = row0 + r0 + warp + 8 * j;
+      uint8_t* o8 = S.out8 + lr * D;
+#pragma unroll
+      for (int i = 0; i < VPL; ++i)
+        *reinterpret_cast<uint32_t*>(o8 + (i * 32 + lane) * 4) = pack_e4m3x4(v[i].x, v[i].y, v[i].z, v[i].w, inv);
+      if (lane == 0) S.out_scale[lr] = fp8_row_scale(am);
+      continue;
+    }
     bf16* o = S.out + (row0 + r0 + warp + 8 * j) * D;
 #pragma unroll
     for (int i = 0; i < VPL; ++i) {
@@ -1000,6 +1061,27 @@ __global__ void __launch_bounds__(256, 2) ln_modulate_bulk_kernel(const __grid_c
       *reinterpret_cast<uint2*>(o + k) = w;
     }
   }
+}
+
+// one warp per row: amax pass, then the codes (weights at load time, so the second read of the row is not worth avoiding)
+__global__ void __launch_bounds__(256) quantize_fp8_rows_kernel(const float* __restrict__ x, int rows, int K, uint8_t* __restrict__ codes,
+                                                                float* __restrict__ scales) {
+  const int lane = threadIdx.x & 31;
+  const long long r = static_cast<long long>(blockIdx.x) * 8 + (threadIdx.x >> 5);
+  if (r >= rows) return;
+  const float* row = x + r * K;
+  float am = 0.f;
+  for (int k = lane * 4; k < K; k += 128) {
+    const float4 v = ld4(row + k);
+    am = fmaxf(am, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))));
+  }
+  am = warp_max(am);
+  const float inv = fp8_row_inv_scale(am);
+  for (int k = lane * 4; k < K; k += 128) {
+    const float4 v = ld4(row + k);
+    *reinterpret_cast<uint32_t*>(codes + r * K + k) = pack_e4m3x4(v.x, v.y, v.z, v.w, inv);
+  }
+  if (lane == 0) scales[r] = fp8_row_scale(am);
 }
 
 inline unsigned blocks_for(long long n, int per) { return static_cast<unsigned>((n + per - 1) / per); }
@@ -1058,8 +1140,21 @@ int k_patchify(const float* latents, const float* Wp, const float* bias, const f
   return 0;
 }
 
+int k_quantize_fp8_rows(const float* x, int rows, int K, uint8_t* codes, float* scales, cudaStream_t s) {
+  TPDM_CHECK(rows > 0 && K > 0 && K % 4 == 0, TPDM_ERR_SHAPE, "quantize_fp8_rows: rows=%d, K=%d (K must be a positive multiple of 4)", rows, K);
+  TPDM_CHECK((reinterpret_cast<uintptr_t>(x) & 15) == 0, TPDM_ERR_ARG, "quantize_fp8_rows: the input must be 16-byte aligned");
+  quantize_fp8_rows_kernel<<<blocks_for(rows, 8), 256, 0, s>>>(x, rows, K, codes, scales);
+  count_launch();
+  TPDM_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
 int k_ln_modulate(const LnSeg* segs, int nseg, int D, cudaStream_t s) {
   TPDM_CHECK(nseg >= 1 && nseg <= 2 && D % 4 == 0, TPDM_ERR_ARG, "ln_modulate: bad arguments");
+  const bool fp8 = segs[0].out8 != nullptr;
+  TPDM_CHECK(nseg == 1 || (segs[1].out8 != nullptr) == fp8, TPDM_ERR_ARG, "ln_modulate: segments of one launch share the output type");
+  for (int i = 0; i < nseg; ++i)
+    TPDM_CHECK(!fp8 || segs[i].out_scale != nullptr, TPDM_ERR_ARG, "ln_modulate: an E4M3 output needs its row scales");
   LnParams P;
   P.nseg = nseg;
   P.D = D;
@@ -1074,11 +1169,26 @@ int k_ln_modulate(const LnSeg* segs, int nseg, int D, cudaStream_t s) {
   const unsigned grid = static_cast<unsigned>(P.blocks_total);
   const size_t smem = static_cast<size_t>(2) * D * sizeof(float);
   TPDM_CHECK(smem <= 48 * 1024, TPDM_ERR_SHAPE, "ln_modulate: D=%d too large", D);
-  double bytes = 0;  // profile class 2: algorithmic bytes = one fp32 read + one bf16 write per element
-  for (int i = 0; i < nseg; ++i) bytes += 6.0 * segs[i].batch * segs[i].rows * D;
+  double bytes = 0;  // profile class 2: algorithmic bytes = one fp32 read + one bf16 (E4M3) write per element
+  for (int i = 0; i < nseg; ++i) bytes += (fp8 ? 5.0 : 6.0) * segs[i].batch * segs[i].rows * D;
   prof_begin(2, bytes, s);
   static const bool bulk = getenv("TPDM_LN_BULK") == nullptr || atoi(getenv("TPDM_LN_BULK")) != 0;
-  if (D == 1536 && bulk) {
+  if (fp8) {
+    if (D == 1536 && bulk) {
+      const size_t smem_b = (2 + 8 * kLnSlots) * static_cast<size_t>(D) * sizeof(float);
+      static bool attr = false;
+      if (!attr) {
+        TPDM_CUDA_OK(cudaFuncSetAttribute(ln_modulate_bulk_kernel<12, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem_b)));
+        attr = true;
+      }
+      TPDM_CUDA_OK(launch_pdl(ln_modulate_bulk_kernel<12, true>, dim3(grid), dim3(256), smem_b, s, P));
+    } else if (D == 1536)
+      TPDM_CUDA_OK(launch_pdl(ln_modulate_kernel<12, true>, dim3(grid), dim3(256), smem, s, P));
+    else if (D == 384)
+      TPDM_CUDA_OK(launch_pdl(ln_modulate_kernel<3, true>, dim3(grid), dim3(256), smem, s, P));
+    else
+      TPDM_CUDA_OK(launch_pdl(ln_modulate_kernel<0, true>, dim3(grid), dim3(256), smem, s, P));
+  } else if (D == 1536 && bulk) {
     const size_t smem_b = (2 + 8 * kLnSlots) * static_cast<size_t>(D) * sizeof(float);
     static bool attr = false;
     if (!attr) {

@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
+#include <stdint.h>
 
 namespace tpdm {
 
@@ -28,9 +29,15 @@ struct LnSeg {
   const float* shift;  // [batch] rows of the modulation buffer, stride mod_stride
   const float* scale;
   int rows, batch, mod_stride;
+  // E4M3 output instead of `out` (every segment of a launch or none): codes [batch][rows][D] and row scales [batch][rows],
+  // quantized per token row by the library's one row quantizer (pack_e4m3x4 in common.cuh)
+  uint8_t* out8 = nullptr;
+  float* out_scale = nullptr;
 };
 // LayerNorm(eps 1e-6, no affine) * (1 + scale) + shift for up to two streams in one launch
 int k_ln_modulate(const LnSeg* segs, int nseg, int D, cudaStream_t s);
+// per row r of x fp32 [rows][K] (K % 4 == 0): codes[r] = E4M3 row quantization of x[r], scales[r] = its scale
+int k_quantize_fp8_rows(const float* x, int rows, int K, uint8_t* codes, float* scales, cudaStream_t s);
 
 // norm_out for the sampling loop: LN-modulate both CFG halves (bf16 -> xn for proj_out) and write
 // h2 = u + guidance*(c - u), scrambled to pixel order, into tpm_x[bl][pix][D:2D];  optional fp32 h2 [2B][N][D]

@@ -105,6 +105,11 @@ static EncodeTiledFn get_encode_fn() {
 
 int encode_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                      const uint32_t* box) {
+  return encode_tmap(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, base, rank, dims, strides_bytes, box);
+}
+
+int encode_tmap(CUtensorMap* out, CUtensorMapDataType dtype, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
+                const uint32_t* box) {
   EncodeTiledFn fn = get_encode_fn();
   TPDM_CHECK(fn != nullptr, TPDM_ERR_CUDA, "cuTensorMapEncodeTiled unavailable (no CUDA driver / device?)");
   TPDM_CHECK((reinterpret_cast<uintptr_t>(base) & 15) == 0, TPDM_ERR_ARG, "TMA base pointer must be 16-byte aligned");
@@ -121,7 +126,7 @@ int encode_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_
       TPDM_CHECK(gstr[i] % 16 == 0, TPDM_ERR_SHAPE, "TMA stride %llu not a multiple of 16 bytes", (unsigned long long)gstr[i]);
     }
   }
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, static_cast<cuuint32_t>(rank), const_cast<void*>(base), gdim, gstr, bx, estr,
+  CUresult r = fn(out, dtype, static_cast<cuuint32_t>(rank), const_cast<void*>(base), gdim, gstr, bx, estr,
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   TPDM_CHECK(r == CUDA_SUCCESS, TPDM_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d (rank %d, dims %llu %llu, box %u %u)",

@@ -31,6 +31,35 @@ def _pad_heads_rows(w: torch.Tensor, heads: int, d: int, dp: int) -> torch.Tenso
     return out.reshape((heads * dp,) + tuple(rest))
 
 
+MMDIT_PRECISIONS = ("bf16", "fp8")
+
+
+def check_mmdit_precision(precision: str) -> str:
+    """``"bf16"`` (every MMDiT GEMM in bf16, the default) or ``"fp8"`` (QKV and FF1 of both streams as E4M3 GEMMs)."""
+    if precision not in MMDIT_PRECISIONS:
+        raise ValueError(f"mmdit_precision must be one of {MMDIT_PRECISIONS}, got {precision!r}")
+    return precision
+
+
+def _fused_rows(g, p: str, names, attn: str, H: int, d: int, dp: int):
+    """Fused projection of a block, [len(names) * H * dp, D] weight and bias, each head padded to dp rows (zeros)."""
+    w = torch.cat([_pad_heads_rows(g(p + f"{attn}.{n}.weight"), H, d, dp) for n in names], 0)
+    bias = torch.cat([_pad_heads_rows(g(p + f"{attn}.{n}.bias"), H, d, dp) for n in names], 0)
+    return w, bias
+
+
+def quantize_fp8_rows(w: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """E4M3 codes (uint8, [rows, K]) and fp32 scales ([rows]) of each row of ``w``, by the library kernel
+    ``tpdm_quantize_fp8_rows``: w ~= codes.view(torch.float8_e4m3fn).float() * scales[:, None]."""
+    lib = L.load()
+    x = _f32(w)
+    codes = torch.empty(x.shape, dtype=torch.uint8, device=x.device)
+    scales = torch.empty(x.shape[0], dtype=torch.float32, device=x.device)
+    with torch.cuda.device(x.device):
+        L.check(lib.tpdm_quantize_fp8_rows(L.ptr(x), x.shape[0], x.shape[1], L.ptr(codes), L.ptr(scales), L.stream_ptr()))
+    return codes, scales
+
+
 class PackedWeights:
     """Device tensors in the layout include/tpdm_b200.h documents, plus the ctypes structs pointing at them."""
 
@@ -39,6 +68,7 @@ class PackedWeights:
         self.by_name = {}
         self.struct = L.TpdmWeights()
         self.blocks = None
+        self.fp8_blocks = None
 
     def _set(self, struct, name, tensor):
         if struct is self.struct and name in self.by_name:   # refresh: same storage, same pointers (plans stay valid)
@@ -81,8 +111,7 @@ def pack_transformer(pw: PackedWeights, sd: Dict[str, torch.Tensor], cfg, device
         b = blocks[i]
 
         def fused(names, attn="attn"):
-            w = torch.cat([_pad_heads_rows(g(p + f"{attn}.{n}.weight"), H, d, dp) for n in names], 0)
-            bias = torch.cat([_pad_heads_rows(g(p + f"{attn}.{n}.bias"), H, d, dp) for n in names], 0)
+            w, bias = _fused_rows(g, p, names, attn, H, d, dp)
             return _bf16(w), _f32(bias)
 
         def out_proj(name, attn="attn"):
@@ -129,6 +158,28 @@ def pack_transformer(pw: PackedWeights, sd: Dict[str, torch.Tensor], cfg, device
     assert pw.keep[-1].numel() == 12 * D * Lyr - 2 * D + 3 * D * len(dual_layers)
     pw.blocks = blocks
     s.blocks = C.cast(blocks, C.POINTER(L.TpdmBlockWeights))
+
+
+def pack_fp8_blocks(pw: PackedWeights, sd: Dict[str, torch.Tensor], cfg, device) -> None:
+    """tpdm_fp8_block_weights: E4M3 codes + per-output-channel scales of the fused QKV / context QKV and FF1 / context FF1
+    matrices, quantized on the device from the state dict's values."""
+    H, d = cfg.num_attention_heads, cfg.attention_head_dim
+    dp = 64 if d <= 64 else 128
+    Lyr = cfg.num_layers
+    g = lambda k: sd[k].to(device)
+    blocks = (L.TpdmFp8BlockWeights * Lyr)()
+    for i in range(Lyr):
+        p = f"transformer_blocks.{i}."
+        mats = [("qkv", _fused_rows(g, p, ("to_q", "to_k", "to_v"), "attn", H, d, dp)[0]),
+                ("cqkv", _fused_rows(g, p, ("add_q_proj", "add_k_proj", "add_v_proj"), "attn", H, d, dp)[0]),
+                ("ff1", g(p + "ff.net.0.proj.weight"))]
+        if i != Lyr - 1:
+            mats.append(("cff1", g(p + "ff_context.net.0.proj.weight")))
+        for field, w in mats:
+            codes, scales = quantize_fp8_rows(w)
+            pw._set(blocks[i], field + "_w", codes)
+            pw._set(blocks[i], field + "_s", scales)
+    pw.fp8_blocks = blocks
 
 
 def pack_time_predictor(pw: PackedWeights, sd: Dict[str, torch.Tensor], device) -> None:
@@ -208,13 +259,19 @@ class Engine:
 
     def __init__(self, cfg: dict, device: torch.device, transformer_sd: Optional[Dict[str, torch.Tensor]] = None, transformer_cfg=None,
                  tpm_sd: Optional[Dict[str, torch.Tensor]] = None, min_sigma: float = 0.001, relative: bool = True,
-                 prediction_type: str = "alpha_beta", epsilon: float = 1e-3, tpm_epsilon: float = 1.0, tpm_channels: int = 128):
+                 prediction_type: str = "alpha_beta", epsilon: float = 1e-3, tpm_epsilon: float = 1.0, tpm_channels: int = 128,
+                 mmdit_precision: str = "bf16"):
+        """``mmdit_precision="fp8"`` runs the QKV and FF1 projections of both streams as E4M3 GEMMs (per-token activation
+        scales, per-channel weight scales); every other GEMM stays bf16."""
+        check_mmdit_precision(mmdit_precision)
+        if mmdit_precision == "fp8" and transformer_sd is None:
+            raise ValueError("mmdit_precision='fp8' needs the transformer weights")
         lib = L.load()
         if device.type != "cuda":
             raise RuntimeError("tpdm_b200 runs on CUDA (sm_100a) only; there is no CPU path")
         if prediction_type not in ("alpha_beta", "mode_concentration"):
             raise ValueError(f"unknown prediction_type {prediction_type!r}")
-        self.cfg, self.device = dict(cfg), device
+        self.cfg, self.device, self.mmdit_precision = dict(cfg), device, mmdit_precision
         self.D = cfg["num_attention_heads"] * cfg["attention_head_dim"]
         c = L.TpdmConfig(
             num_layers=cfg["num_layers"], num_heads=cfg["num_attention_heads"], head_dim=cfg["attention_head_dim"],
@@ -236,6 +293,9 @@ class Engine:
             if self.has_tpm:
                 pack_time_predictor(self.weights, tpm_sd, device)
             L.check(lib.tpdm_set_weights(self.ctx, C.byref(self.weights.struct)))
+            if mmdit_precision == "fp8":
+                pack_fp8_blocks(self.weights, transformer_sd, transformer_cfg, device)
+                L.check(lib.tpdm_set_fp8_weights(self.ctx, self.weights.fp8_blocks))
         self.plans: Dict[Tuple, Plan] = {}
         self.min_sigma = min_sigma
 

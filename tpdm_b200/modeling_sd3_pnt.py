@@ -125,9 +125,11 @@ class SD3PredictNextTimeStepModel(nn.Module):
         transformer_config: Optional[dict] = None,
         device=None,
         vae_config: Optional[dict] = None,
+        mmdit_precision: str = "bf16",
     ):
         """Reference kwargs (modeling_sd3_pnt.py:130-140) plus ``transformer_config`` / ``device`` for offline random-init
-        construction (the reference only has ``from_pretrained``)."""
+        construction (the reference only has ``from_pretrained``) and ``mmdit_precision`` ("bf16" or "fp8", see
+        CustomSD3Transformer2DModel), which is the transformer's attribute of that name."""
         super().__init__()
         cfg = transformer_config
         weights_file = None
@@ -162,7 +164,7 @@ class SD3PredictNextTimeStepModel(nn.Module):
                 from safetensors.torch import load_file
 
                 _check_loaded("vae", self.vae.load_state_dict(load_file(vae_weights), strict=False), ("encoder.", "quant_conv.", "post_quant_conv."))
-        self.transformer = CustomSD3Transformer2DModel(**cfg, device=device, dtype=torch_dtype)
+        self.transformer = CustomSD3Transformer2DModel(**cfg, device=device, dtype=torch_dtype, mmdit_precision=mmdit_precision)
         if weights_file is not None and os.path.isfile(weights_file):
             from safetensors.torch import load_file
 
@@ -194,15 +196,23 @@ class SD3PredictNextTimeStepModel(nn.Module):
     def dtype(self):
         return self.transformer.dtype
 
+    @property
+    def mmdit_precision(self) -> str:
+        return self.transformer.mmdit_precision
+
+    @mmdit_precision.setter
+    def mmdit_precision(self, value: str) -> None:
+        self.transformer.mmdit_precision = value
+
     def get_engine(self) -> Engine:
-        key_t = (self.transformer._weights_key(), self.min_sigma, self.relative, self.prediction_type)
+        key_t = (self.transformer._weights_key(), self.min_sigma, self.relative, self.prediction_type, self.mmdit_precision)
         key_p = self.time_predictor._weights_key()
         if self._engine is None or key_t != self._engine_key[0]:
             self._engine = Engine(self.transformer.engine_config(), self.device, transformer_sd=self.transformer.state_dict(),
                                   transformer_cfg=self.transformer.config, tpm_sd=self.time_predictor.state_dict(),
                                   min_sigma=self.min_sigma, relative=self.relative, prediction_type=self.prediction_type,
                                   epsilon=self.epsilon, tpm_epsilon=self.time_predictor.epsilon,
-                                  tpm_channels=self.time_predictor.conv_out_channels)
+                                  tpm_channels=self.time_predictor.conv_out_channels, mmdit_precision=self.mmdit_precision)
         elif key_p != self._engine_key[1]:
             # only the TimePredictor changed (an optimizer step): refresh its packed tensors in place, keep the 4 GB MMDiT pack
             self._engine.refresh_time_predictor(self.time_predictor.state_dict())
@@ -470,13 +480,14 @@ class SD3PredictNextTimeStepModelRLOOWrapper(nn.Module):
         max_inference_steps: int = 28,
         transformer_config: Optional[dict] = None,
         device=None,
+        mmdit_precision: str = "bf16",
     ):
         super().__init__()
         self.pretrained_model_name_or_path = pretrained_model_name_or_path or ""
         self.agent_model = SD3PredictNextTimeStepModel(
             pretrained_model_name_or_path, torch_dtype=torch_dtype, init_alpha=init_alpha, init_beta=init_beta, min_sigma=min_sigma,
             pre_process=pre_process, relative=relative, prediction_type=prediction_type, transformer_config=transformer_config,
-            device=device).eval()
+            device=device, mmdit_precision=mmdit_precision).eval()
         self.relative = relative
         self.fsdp = fsdp
         self.max_inference_steps = max_inference_steps

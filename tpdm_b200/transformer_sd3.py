@@ -14,7 +14,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from .engine import Engine
+from .engine import Engine, check_mmdit_precision
 
 
 class BaseOutput(dict):
@@ -177,8 +177,13 @@ class CustomSD3Transformer2DModel(nn.Module):
         qk_norm: Optional[str] = None,
         device=None,
         dtype=None,
+        mmdit_precision: str = "bf16",
     ):
+        """``mmdit_precision``: ``"bf16"`` (default) or ``"fp8"``, which runs the QKV and FF1 projections of both streams as
+        E4M3 GEMMs with per-token activation and per-channel weight scales (INTEGRATION.md states the accuracy); the
+        attribute of the same name may be changed later, the next forward then builds a matching engine."""
         super().__init__()
+        self.mmdit_precision = mmdit_precision
         dual_attention_layers = tuple(int(i) for i in dual_attention_layers)
         if any(i < 0 or i >= num_layers or i >= 64 for i in dual_attention_layers):
             raise ValueError(f"dual_attention_layers {dual_attention_layers} must name layers below min(num_layers, 64)")
@@ -208,6 +213,14 @@ class CustomSD3Transformer2DModel(nn.Module):
         self._engine: Optional[Engine] = None
         self._engine_key = None
 
+    @property
+    def mmdit_precision(self) -> str:
+        return self._mmdit_precision
+
+    @mmdit_precision.setter
+    def mmdit_precision(self, value: str) -> None:
+        self._mmdit_precision = check_mmdit_precision(value)
+
     # -- engine management: repack whenever a parameter tensor was replaced / modified in place ---------------------
     def _weights_key(self):
         return tuple((p.data_ptr(), p._version, p.device) for p in list(self.parameters()) + list(self.buffers()))
@@ -220,10 +233,11 @@ class CustomSD3Transformer2DModel(nn.Module):
                     pos_embed_max_size=c.pos_embed_max_size, qk_norm=c.qk_norm, dual_attention_layers=c.dual_attention_layers)
 
     def get_engine(self) -> Engine:
-        key = self._weights_key()
+        key = (self._weights_key(), self.mmdit_precision)
         if self._engine is None or key != self._engine_key:
             dev = self.proj_out.weight.device
-            self._engine = Engine(self.engine_config(), dev, transformer_sd=self.state_dict(), transformer_cfg=self.config)
+            self._engine = Engine(self.engine_config(), dev, transformer_sd=self.state_dict(), transformer_cfg=self.config,
+                                  mmdit_precision=self.mmdit_precision)
             self._engine_key = key
         return self._engine
 
