@@ -308,6 +308,40 @@ int tpdm_queue_step_graph(tpdm_plan* plan, void* stream);
 int tpdm_queue_status(tpdm_plan* plan, const int** active_slots, const int** slot_prompts);
 
 /* ----------------------------------------------------------------------------------------------------------------
+ * Open prompt stream: the device-side prompt queue with admission while it runs (continuous batching for serving).  The
+ * plan's `batch` entries are the in-flight slots; prompts live in a ring of `capacity` ENTRIES inside the caller's
+ * workspace, each holding the noise latents, the context_embedder output [2][T][D] and pooled-text part [2][D] (uncond, cond),
+ * the output latents, step count and sigmas [max_steps + 1] of one request.  The caller owns the free list: an entry is
+ * handed to tpdm_stream_submit, and free again once its id was read from the completion log and its outputs were copied.
+ * Counters (device int[4]): submitted, claimed, completed, executed steps.  Every stream call and every step is enqueued on
+ * ONE stream, so ordering is by stream order; nothing synchronises the host.
+ * Steps are tpdm_queue_step / tpdm_queue_step_graph on the plan (one captured graph: the ring, counters and staging never move).
+ * A slot without a prompt -- its trajectory just ended, or it was idle -- takes the next submitted ticket in slot order (no
+ * atomics, deterministic); a step of a stream with no active slot is skipped on the device.  Each request follows exactly the
+ * trajectory tpdm_sample_* gives it with batch 1 and predict = 1.  TPDM_ERR_STATE: open on a plan whose queue has begun or whose
+ * stream is open; tpdm_queue_begin / tpdm_sample_begin / tpdm_queue_set_rollout while the stream is open; the other stream
+ * calls without an open stream.
+ * ---------------------------------------------------------------------------------------------------------------- */
+size_t tpdm_stream_workspace_bytes(const tpdm_plan* plan, int capacity);
+/* workspace: 1 KiB aligned, >= tpdm_stream_workspace_bytes; borrowed until tpdm_stream_close.  Encodes the TMA maps of the
+ * stream's own context_embedder GEMM (2 * batch rows of staging). */
+int tpdm_stream_open(tpdm_plan* plan, int capacity, float guidance_scale, void* workspace, size_t workspace_bytes, void* stream);
+/* Admit n prompts into the free entries entry_ids[n] (host array, each in [0, capacity)): latents [n][C][h][w],
+ * *_embeds [n][T][joint_attention_dim], *_pooled [n][pooled_projection_dim], device fp32, read by the enqueued work only.
+ * Runs `batch` prompts per pass through the stream's own staging (text cast, context_embedder, pooled-text MLP), copies them
+ * into their entries, publishes them, then lets idle slots claim: a prompt submitted to an idle stream runs in the next step. */
+int tpdm_stream_submit(tpdm_plan* plan, int n, const int* entry_ids, const float* latents, const float* neg_embeds,
+                       const float* pos_embeds, const float* neg_pooled, const float* pos_pooled, void* stream);
+/* device pointers: counters int[4] followed by `active` (slots holding a prompt) and the skip flag; done_log int[capacity]
+ * (entry ids in completion order, entry k of the log at k % capacity); per entry: out_latents [capacity][C][h][w],
+ * out_steps [capacity], out_sigmas [capacity][max_steps + 1].  A completion counted after a step is readable once that
+ * step has completed. */
+int tpdm_stream_status(tpdm_plan* plan, const int** counters, const int** done_log, const float** out_latents, const int** out_steps,
+                       const float** out_sigmas);
+/* Detach the stream (the caller synchronises first); the plan can then begin a queue or open a new stream. */
+int tpdm_stream_close(tpdm_plan* plan);
+
+/* ----------------------------------------------------------------------------------------------------------------
  * VAE decode of the final latent (SURVEY.md 8(f) rank 1).  Replaces, for the decode step only,
  *   latents = latents / vae.config.scaling_factor + vae.config.shift_factor
  *   image   = vae.decode(latents, return_dict=False)[0];  image_processor.postprocess(image, "pil")

@@ -103,6 +103,11 @@ EXPORTS = {
     "tpdm_queue_step": (C.c_int, [vp, vp]),
     "tpdm_queue_step_graph": (C.c_int, [vp, vp]),
     "tpdm_queue_status": (C.c_int, [vp, C.POINTER(vp), C.POINTER(vp)]),
+    "tpdm_stream_workspace_bytes": (C.c_size_t, [vp, C.c_int]),
+    "tpdm_stream_open": (C.c_int, [vp, C.c_int, C.c_float, vp, C.c_size_t, vp]),
+    "tpdm_stream_submit": (C.c_int, [vp, C.c_int, C.POINTER(C.c_int), vp, vp, vp, vp, vp, vp]),
+    "tpdm_stream_status": (C.c_int, [vp] + [C.POINTER(vp)] * 5),
+    "tpdm_stream_close": (C.c_int, [vp]),
     "tpdm_vae_create": (C.c_int, [C.POINTER(TpdmVaeConfig), C.POINTER(vp)]),
     "tpdm_vae_destroy": (C.c_int, [vp]),
     "tpdm_vae_num_resnets": (C.c_int, [vp]),

@@ -94,6 +94,17 @@ struct tpdm_plan {
     cudaGraphExec_t graph = nullptr;   // one captured queue step (every pointer of a queue step is fixed between steps)
     long long graph_launches = 0;
   } q;
+  // open prompt stream (tpdm_stream_*): the queue above runs over a ring of `capacity` entries, prompts are admitted between steps
+  struct Stream {
+    int open = 0, capacity = 0;
+    int *order = nullptr, *counters = nullptr, *done_log = nullptr;
+    float* noise = nullptr;
+    // admission staging, never read by a queue step: bf16 text [2*slots][T][J] (row 2k + half), its context_embedder output and
+    // the pooled-text MLP of the same rows
+    bf16* enc = nullptr;
+    float *ctx0 = nullptr, *phid = nullptr, *text = nullptr;
+    GemmOp ctx_embed;
+  } st;
   // tpdm_sample_step_graph: one captured graph per step index (the step index only moves pointers inside the plan's own buffers),
   // valid for the guidance / predict / injected-ratio setting they were captured under
   std::vector<cudaGraphExec_t> step_graph;
@@ -565,6 +576,7 @@ int tpdm_sample_begin(tpdm_plan* p, const float* latents, const float* neg_embed
                       void* stream) {
   TPDM_CHECK(p && latents && neg_embeds && pos_embeds && neg_pooled && pos_pooled, TPDM_ERR_ARG, "tpdm_sample_begin: null argument");
   TPDM_CHECK(p->cfg_pairs, TPDM_ERR_STATE, "tpdm_sample_begin: the plan was created without cfg_pairs");
+  TPDM_CHECK(!p->st.open, TPDM_ERR_STATE, "tpdm_sample_begin: the plan has an open prompt stream (tpdm_stream_close first)");
   TPDM_CHECK(p->ctx->has_mmdit && p->ctx->has_tpm, TPDM_ERR_STATE, "tpdm_sample_begin: needs both MMDiT and TimePredictor weights");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const tpdm_ctx* ctx = p->ctx;
@@ -723,6 +735,12 @@ QueueArgs queue_args(const tpdm_plan* p, int init) {
   a.rec_alphas = q.rec_alphas;
   a.rec_betas = q.rec_betas;
   a.rec_logprobs = q.rec_logprobs;
+  if (p->st.open) {
+    a.order = p->st.order;
+    a.counters = p->st.counters;
+    a.done_log = p->st.done_log;
+    a.capacity = p->st.capacity;
+  }
   return a;
 }
 int queue_move(tpdm_plan* p, cudaStream_t s) {
@@ -746,6 +764,7 @@ int tpdm_queue_begin(tpdm_plan* p, int n_prompts, const float* latents_all, cons
                  out_latents && out_steps,
              TPDM_ERR_ARG, "tpdm_queue_begin: null argument");
   TPDM_CHECK(p->cfg_pairs, TPDM_ERR_STATE, "tpdm_queue_begin: the plan was created without cfg_pairs");
+  TPDM_CHECK(!p->st.open, TPDM_ERR_STATE, "tpdm_queue_begin: the plan has an open prompt stream (tpdm_stream_close first)");
   TPDM_CHECK(p->ctx->has_mmdit && p->ctx->has_tpm, TPDM_ERR_STATE, "tpdm_queue_begin: needs both MMDiT and TimePredictor weights");
   TPDM_CHECK(n_prompts >= p->B, TPDM_ERR_ARG, "tpdm_queue_begin: %d prompts for %d slots (use a plan with fewer slots)", n_prompts, p->B);
   TPDM_CHECK(order != nullptr || n_queued == n_prompts || n_queued <= 0, TPDM_ERR_ARG, "tpdm_queue_begin: n_queued needs an order table");
@@ -837,7 +856,7 @@ int tpdm_queue_step(tpdm_plan* p, void* stream) {
   TPDM_TRY(k_queue_schedule(queue_args(p, 0), s));
   TPDM_TRY(k_unpatchify(p->pout, B, 1, p->guidance, ctx->cfg.out_channels, p->Hl, p->Wl, nullptr, p->latents, p->q.sigma_cur,
                         p->q.sigma_next, 1, nullptr, s));
-  TPDM_TRY(k_queue_advance(queue_args(p, 0), s));
+  TPDM_TRY(p->st.open ? k_stream_advance(queue_args(p, 0), 0, s) : k_queue_advance(queue_args(p, 0), s));
   TPDM_TRY(queue_move(p, s));
   return 0;
 }
@@ -846,6 +865,7 @@ int tpdm_queue_set_rollout(tpdm_plan* p, unsigned long long seed, const float* r
                            float* tembs, void* tpm_inputs) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_queue_set_rollout: null plan");
   TPDM_CHECK(p->q.begun, TPDM_ERR_STATE, "tpdm_queue_set_rollout: call tpdm_queue_begin first");
+  TPDM_CHECK(!p->st.open, TPDM_ERR_STATE, "tpdm_queue_set_rollout: a prompt stream runs predict mode only");
   // the probe step of longest-first scheduling ran the Beta mode, so such a queue cannot start sampled trajectories
   TPDM_CHECK(p->q.init_step == 0, TPDM_ERR_STATE, "tpdm_queue_set_rollout: the queue began after %d probe steps (init_step > 0)", p->q.init_step);
   tpdm_plan::Queue& q = p->q;
@@ -896,6 +916,190 @@ int tpdm_queue_status(tpdm_plan* p, const int** active_slots, const int** slot_p
   TPDM_CHECK(p && p->q.begun, TPDM_ERR_STATE, "tpdm_queue_status: call tpdm_queue_begin first");
   if (active_slots) *active_slots = p->q.active;
   if (slot_prompts) *slot_prompts = p->q.slot_prompt;
+  return 0;
+}
+
+// ---- open prompt stream -------------------------------------------------------------------------------------------
+namespace {
+// ring of `capacity` entries + slot state + counters + admission staging, in the order tpdm_stream_open hands them out
+void carve_stream(tpdm_plan* p, int capacity, Carver& c) {
+  tpdm_plan::Queue& q = p->q;
+  tpdm_plan::Stream& st = p->st;
+  const size_t cap = capacity, B = p->B, T = p->T, D = p->ctx->D, J = p->ctx->cfg.joint_attention_dim;
+  const size_t lat = static_cast<size_t>(p->ctx->cfg.in_channels) * p->Hl * p->Wl;
+  st.noise = c.take<float>(cap * lat);
+  q.ctx0_all = c.take<float>(cap * 2 * T * D);
+  q.text_all = c.take<float>(cap * 2 * D);
+  q.out_latents = c.take<float>(cap * lat);
+  q.out_sigmas = c.take<float>(cap * (p->max_steps + 1));
+  q.out_steps = c.take<int>(cap);
+  st.order = c.take<int>(cap);
+  st.done_log = c.take<int>(cap);
+  q.sigma_cur = c.take<float>(2 * B);
+  q.sigma_next = q.sigma_cur ? q.sigma_cur + B : nullptr;
+  q.slot_prompt = c.take<int>(5 * B + kStreamCounters + 2);
+  if (q.slot_prompt) {
+    q.slot_step = q.slot_prompt + B;
+    q.slot_flush = q.slot_step + B;
+    q.slot_load = q.slot_flush + B;
+    q.slot_active = q.slot_load + B;
+    st.counters = q.slot_active + B;
+    q.active = st.counters + kStreamCounters;   // right behind the counters: one copy reads both
+    q.idle_flag = q.active + 1;
+  }
+  st.enc = c.take<bf16>(2 * B * T * J);
+  st.ctx0 = c.take<float>(2 * B * T * D);
+  st.phid = c.take<float>(2 * B * D);
+  st.text = c.take<float>(2 * B * D);
+}
+
+// context_embedder + pooled-text MLP of n <= slots prompts into the staging rows 2k + half (half 0 = negative, 1 = positive)
+int stream_embed(tpdm_plan* p, int n, const float* neg, const float* pos, const float* neg_pooled, const float* pos_pooled, cudaStream_t s) {
+  const tpdm_ctx* ctx = p->ctx;
+  const tpdm_weights& w = ctx->w;
+  tpdm_plan::Stream& st = p->st;
+  const int D = ctx->D, PD = ctx->cfg.pooled_projection_dim;
+  const long long row = static_cast<long long>(p->T) * ctx->cfg.joint_attention_dim;
+  for (int k = 0; k < n; ++k) {
+    TPDM_TRY(k_cast_bf16(neg + k * row, st.enc + (2 * k) * row, row, s));
+    TPDM_TRY(k_cast_bf16(pos + k * row, st.enc + (2 * k + 1) * row, row, s));
+  }
+  GemmOp op = st.ctx_embed;   // the TMA maps cover 2 * slots rows; run the first 2n
+  op.batch = 2 * n;
+  op.num_tiles = op.batch * op.tiles_m_per_batch * op.tiles_n;
+  TPDM_TRY(gemm_launch(&op, 1, s));
+  TPDM_TRY(k_gemv_f32(w.p_w1, w.p_b1, neg_pooled, PD, nullptr, st.phid, 2 * D, n, D, PD, 0, s));
+  TPDM_TRY(k_gemv_f32(w.p_w1, w.p_b1, pos_pooled, PD, nullptr, st.phid + D, 2 * D, n, D, PD, 0, s));
+  TPDM_TRY(k_gemv_f32(w.p_w2, w.p_b2, st.phid, D, nullptr, st.text, D, 2 * n, D, D, 1, s));
+  return 0;
+}
+}  // namespace
+
+size_t tpdm_stream_workspace_bytes(const tpdm_plan* p, int capacity) {
+  if (!p || capacity <= 0) return 0;
+  tpdm_plan probe;
+  probe.ctx = p->ctx;
+  probe.B = p->B;
+  probe.T = p->T;
+  probe.Hl = p->Hl;
+  probe.Wl = p->Wl;
+  probe.max_steps = p->max_steps;
+  Carver c(nullptr);
+  carve_stream(&probe, capacity, c);
+  return c.off + 1024;
+}
+
+int tpdm_stream_open(tpdm_plan* p, int capacity, float guidance_scale, void* workspace, size_t workspace_bytes, void* stream) {
+  TPDM_CHECK(p && workspace, TPDM_ERR_ARG, "tpdm_stream_open: null argument");
+  TPDM_CHECK(p->cfg_pairs, TPDM_ERR_STATE, "tpdm_stream_open: the plan was created without cfg_pairs");
+  TPDM_CHECK(p->ctx->has_mmdit && p->ctx->has_tpm, TPDM_ERR_STATE, "tpdm_stream_open: needs both MMDiT and TimePredictor weights");
+  TPDM_CHECK(!p->st.open, TPDM_ERR_STATE, "tpdm_stream_open: the plan already has an open stream");
+  TPDM_CHECK(!p->q.begun, TPDM_ERR_STATE, "tpdm_stream_open: a prompt queue has begun on this plan (open the stream on a fresh plan)");
+  TPDM_CHECK(capacity > 0, TPDM_ERR_ARG, "tpdm_stream_open: capacity %d must be positive", capacity);
+  const size_t need = tpdm_stream_workspace_bytes(p, capacity);
+  TPDM_CHECK((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0 && workspace_bytes >= need, TPDM_ERR_ARG,
+             "tpdm_stream_open: workspace must be 1 KiB aligned and >= %zu bytes", need);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const tpdm_ctx* ctx = p->ctx;
+  const int B = p->B, T = p->T, D = ctx->D, J = ctx->cfg.joint_attention_dim;
+  tpdm_plan::Queue& q = p->q;
+  tpdm_plan::Stream& st = p->st;
+  if (q.graph) {
+    cudaGraphExecDestroy(q.graph);
+    q.graph = nullptr;
+  }
+  Carver c(workspace);
+  carve_stream(p, capacity, c);
+  TPDM_TRY(gemm_op_init(&st.ctx_embed, st.enc, J, static_cast<long long>(T) * J, T, 2 * B, J, ctx->w.ctx_w, D, EPI_BIAS_F32, st.ctx0,
+                        static_cast<long long>(T) * D, D, ctx->w.ctx_b, nullptr, 0));
+  st.capacity = capacity;
+  q.n_prompts = q.n_queued = capacity;
+  q.noise_all = st.noise;
+  q.ticket = nullptr;
+  q.order = nullptr;
+  q.init_sigma = nullptr;
+  q.init_step = 0;
+  q.predict = 1;
+  q.seed = 0;
+  q.ratios_all = nullptr;
+  q.rec_alphas = q.rec_betas = q.rec_logprobs = q.rec_tembs = nullptr;
+  q.rec_tpm = nullptr;
+  p->guidance = guidance_scale;
+  p->predict = 1;
+  TPDM_CUDA_OK(cudaMemsetAsync(q.sigma_cur, 0, sizeof(float) * 2 * B, s));
+  TPDM_CUDA_OK(cudaMemsetAsync(q.slot_prompt, 0xff, sizeof(int) * B, s));  // -1: every slot is idle
+  TPDM_CUDA_OK(cudaMemsetAsync(q.slot_step, 0, sizeof(int) * (4 * B + kStreamCounters + 2), s));
+  st.open = 1;
+  q.begun = 1;
+  p->begun = 0;
+  TPDM_TRY(k_stream_advance(queue_args(p, 0), 1, s));   // nothing submitted: every slot stays idle, the skip flag is raised
+  return 0;
+}
+
+int tpdm_stream_submit(tpdm_plan* p, int n, const int* entry_ids, const float* latents, const float* neg_embeds, const float* pos_embeds,
+                       const float* neg_pooled, const float* pos_pooled, void* stream) {
+  TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_stream_submit: null plan");
+  TPDM_CHECK(p->st.open, TPDM_ERR_STATE, "tpdm_stream_submit: the plan has no open stream");
+  TPDM_CHECK(n > 0 && entry_ids && latents && neg_embeds && pos_embeds && neg_pooled && pos_pooled, TPDM_ERR_ARG,
+             "tpdm_stream_submit: null argument or n <= 0");
+  tpdm_plan::Stream& st = p->st;
+  TPDM_CHECK(n <= st.capacity, TPDM_ERR_ARG, "tpdm_stream_submit: %d prompts for a ring of %d entries", n, st.capacity);
+  std::vector<char> seen(st.capacity, 0);   // a repeated id would publish one entry twice and overrun unclaimed order slots
+  for (int k = 0; k < n; ++k) {
+    const int id = entry_ids[k];
+    TPDM_CHECK(id >= 0 && id < st.capacity, TPDM_ERR_ARG, "tpdm_stream_submit: entry id %d outside [0,%d)", id, st.capacity);
+    TPDM_CHECK(!seen[id], TPDM_ERR_ARG, "tpdm_stream_submit: entry id %d given twice", id);
+    seen[id] = 1;
+  }
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const tpdm_ctx* ctx = p->ctx;
+  tpdm_plan::Queue& q = p->q;
+  const int D = ctx->D, PD = ctx->cfg.pooled_projection_dim;
+  const size_t nctx = static_cast<size_t>(p->T) * D, row = static_cast<size_t>(p->T) * ctx->cfg.joint_attention_dim;
+  const size_t lat = static_cast<size_t>(ctx->cfg.in_channels) * p->Hl * p->Wl;
+  const int pass = p->B < kStreamPublishMax ? p->B : kStreamPublishMax;
+  for (int k0 = 0; k0 < n; k0 += pass) {
+    const int m = n - k0 < pass ? n - k0 : pass;
+    TPDM_TRY(stream_embed(p, m, neg_embeds + k0 * row, pos_embeds + k0 * row, neg_pooled + static_cast<size_t>(k0) * PD,
+                          pos_pooled + static_cast<size_t>(k0) * PD, s));
+    StreamEntries e{};
+    for (int k = 0; k < m; ++k) {
+      const size_t id = entry_ids[k0 + k];
+      e.id[k] = static_cast<int>(id);
+      TPDM_CUDA_OK(cudaMemcpyAsync(st.noise + id * lat, latents + (k0 + k) * lat, lat * sizeof(float), cudaMemcpyDeviceToDevice, s));
+      TPDM_CUDA_OK(cudaMemcpyAsync(q.ctx0_all + id * 2 * nctx, st.ctx0 + static_cast<size_t>(k) * 2 * nctx, 2 * nctx * sizeof(float),
+                                   cudaMemcpyDeviceToDevice, s));
+      TPDM_CUDA_OK(cudaMemcpyAsync(q.text_all + id * 2 * D, st.text + static_cast<size_t>(k) * 2 * D, 2 * D * sizeof(float),
+                                   cudaMemcpyDeviceToDevice, s));
+    }
+    TPDM_TRY(k_stream_publish(st.order, st.counters, st.capacity, e, m, s));
+  }
+  // idle slots take the new tickets now, so the next step already computes them
+  TPDM_TRY(k_stream_advance(queue_args(p, 0), 1, s));
+  return queue_move(p, s);
+}
+
+int tpdm_stream_status(tpdm_plan* p, const int** counters, const int** done_log, const float** out_latents, const int** out_steps,
+                       const float** out_sigmas) {
+  TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_stream_status: null plan");
+  TPDM_CHECK(p->st.open, TPDM_ERR_STATE, "tpdm_stream_status: the plan has no open stream");
+  if (counters) *counters = p->st.counters;
+  if (done_log) *done_log = p->st.done_log;
+  if (out_latents) *out_latents = p->q.out_latents;
+  if (out_steps) *out_steps = p->q.out_steps;
+  if (out_sigmas) *out_sigmas = p->q.out_sigmas;
+  return 0;
+}
+
+int tpdm_stream_close(tpdm_plan* p) {
+  TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_stream_close: null plan");
+  TPDM_CHECK(p->st.open, TPDM_ERR_STATE, "tpdm_stream_close: the plan has no open stream");
+  if (p->q.graph) {
+    cudaGraphExecDestroy(p->q.graph);
+    p->q.graph = nullptr;
+  }
+  p->st = tpdm_plan::Stream{};
+  p->q = tpdm_plan::Queue{};
   return 0;
 }
 

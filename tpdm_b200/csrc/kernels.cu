@@ -881,6 +881,20 @@ __global__ void __launch_bounds__(256) queue_record_kernel(const int* __restrict
   }
 }
 
+// count the step of an occupied slot: returns true when its trajectory ended (final step count written), else moves it on
+__device__ __forceinline__ bool queue_slot_retires(const QueueArgs& a, int i, int prompt) {
+  const int step = a.slot_step[i] + 1;
+  const float sn = a.sigma_next[i];
+  if (a.out_sigmas) a.out_sigmas[static_cast<long long>(prompt) * (a.max_steps + 1) + step] = sn;
+  if (sn < a.min_sigma || step >= a.max_steps) {   // the prompt-level form of the batch-wide exit test (:608)
+    a.out_steps[prompt] = step;
+    return true;
+  }
+  a.slot_step[i] = step;
+  a.sigma_cur[i] = sn;
+  return false;
+}
+
 // after the Euler step: count the step, retire finished trajectories, hand the freed slots their next ticket
 __global__ void queue_advance_kernel(const QueueArgs a) {
   const int i = threadIdx.x;
@@ -888,18 +902,9 @@ __global__ void queue_advance_kernel(const QueueArgs a) {
   if (i < a.B) {
     int prompt = a.slot_prompt[i], flush = -1, load = 0;
     bool need = a.init != 0;
-    if (!a.init && prompt >= 0) {
-      const int step = a.slot_step[i] + 1;
-      const float sn = a.sigma_next[i];
-      if (a.out_sigmas) a.out_sigmas[static_cast<long long>(prompt) * (a.max_steps + 1) + step] = sn;
-      if (sn < a.min_sigma || step >= a.max_steps) {   // the prompt-level form of the batch-wide exit test (:608)
-        flush = prompt;
-        a.out_steps[prompt] = step;
-        need = true;
-      } else {
-        a.slot_step[i] = step;
-        a.sigma_cur[i] = sn;
-      }
+    if (!a.init && prompt >= 0 && queue_slot_retires(a, i, prompt)) {
+      flush = prompt;
+      need = true;
     }
     if (need) {
       const int t = atomicAdd_system(a.ticket, 1);
@@ -920,6 +925,76 @@ __global__ void queue_advance_kernel(const QueueArgs a) {
     *a.active = n;
     *a.idle_flag = n == 0 ? 1 : 0;
   }
+}
+
+// exclusive count of `flag` over the threads below this one (slot order) and the block total; every thread of the block calls it
+__device__ __forceinline__ int block_rank(int flag, int* total, int* warp_counts) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+  const unsigned m = __ballot_sync(0xffffffffu, flag != 0);
+  if (lane == 0) warp_counts[warp] = __popc(m);
+  __syncthreads();
+  int below = 0, all = 0;
+  for (int w = 0; w < nwarps; ++w) {
+    const int c = warp_counts[w];
+    below += w < warp ? c : 0;
+    all += c;
+  }
+  __syncthreads();  // warp_counts is reused by the next call
+  *total = all;
+  return below + __popc(m & ((1u << lane) - 1u));
+}
+
+// Stream mode of queue_advance_kernel.  The claim head is private to the stream, so tickets are handed out by rank in slot order
+// (deterministic, no atomics); finished entries are appended to the completion log in the same order.
+__global__ void stream_advance_kernel(const QueueArgs a, int admit) {
+  __shared__ int warp_counts[32];
+  const int i = threadIdx.x;
+  const int submitted = a.counters[kStreamSubmitted], head = a.counters[kStreamClaimed], completed = a.counters[kStreamCompleted];
+  const int ran = *a.active > 0 ? 1 : 0;   // slots held a prompt when the step began: it was not skipped
+  int prompt = -1, flush = -1;
+  if (i < a.B) {
+    prompt = a.slot_prompt[i];
+    if (!admit && prompt >= 0 && queue_slot_retires(a, i, prompt)) {
+      flush = prompt;
+      prompt = -1;
+    }
+  }
+  const int need = i < a.B && prompt < 0 ? 1 : 0;
+  int n_need = 0, n_flush = 0;
+  const int r_need = block_rank(need, &n_need, warp_counts);
+  const int r_flush = block_rank(flush >= 0, &n_flush, warp_counts);
+  int holds = 0;
+  if (i < a.B) {
+    int load = 0;
+    if (need) {
+      const int t = head + r_need;
+      prompt = t < submitted ? a.order[t % a.capacity] : -1;
+      a.slot_prompt[i] = prompt;
+      a.slot_step[i] = 0;
+      a.sigma_cur[i] = 1.0f;   // sigma = ones (:508)
+      load = prompt >= 0 ? 1 : 0;
+      if (prompt >= 0 && a.out_sigmas) a.out_sigmas[static_cast<long long>(prompt) * (a.max_steps + 1)] = 1.0f;
+    }
+    if (flush >= 0) a.done_log[(completed + r_flush) % a.capacity] = flush;
+    a.slot_flush[i] = flush;
+    a.slot_load[i] = load;
+    holds = prompt >= 0 ? 1 : 0;
+    a.slot_active[i] = holds;
+  }
+  const int n = __syncthreads_count(holds);
+  if (i == 0) {
+    a.counters[kStreamClaimed] = head + n_need < submitted ? head + n_need : submitted;
+    a.counters[kStreamCompleted] = completed + n_flush;
+    if (!admit) a.counters[kStreamExecuted] += ran;
+    *a.active = n;
+    *a.idle_flag = n == 0 ? 1 : 0;
+  }
+}
+
+__global__ void stream_publish_kernel(int* order, int* counters, int capacity, const StreamEntries e, int n) {
+  const int s = counters[kStreamSubmitted];
+  for (int k = 0; k < n; ++k) order[(s + k) % capacity] = e.id[k];
+  counters[kStreamSubmitted] = s + n;
 }
 
 __global__ void __launch_bounds__(256) queue_move_kernel(const int* __restrict__ slot_prompt, const int* __restrict__ slot_flush,
@@ -1315,6 +1390,23 @@ int k_queue_schedule(const QueueArgs& a, cudaStream_t s) {
 int k_queue_advance(const QueueArgs& a, cudaStream_t s) {
   TPDM_CHECK(a.B <= 1024, TPDM_ERR_SHAPE, "queue: %d slots > 1024", a.B);
   queue_advance_kernel<<<1, ((a.B + 31) / 32) * 32, 0, s>>>(a);
+  count_launch();
+  TPDM_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
+int k_stream_advance(const QueueArgs& a, int admit, cudaStream_t s) {
+  TPDM_CHECK(a.B <= 1024, TPDM_ERR_SHAPE, "queue: %d slots > 1024", a.B);
+  TPDM_CHECK(a.counters && a.done_log && a.order && a.capacity > 0, TPDM_ERR_STATE, "stream_advance: the plan has no open stream");
+  stream_advance_kernel<<<1, ((a.B + 31) / 32) * 32, 0, s>>>(a, admit);
+  count_launch();
+  TPDM_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
+int k_stream_publish(int* order, int* counters, int capacity, const StreamEntries& e, int n, cudaStream_t s) {
+  TPDM_CHECK(n >= 0 && n <= kStreamPublishMax, TPDM_ERR_ARG, "stream_publish: %d entries per launch (at most %d)", n, kStreamPublishMax);
+  stream_publish_kernel<<<1, 1, 0, s>>>(order, counters, capacity, e, n);
   count_launch();
   TPDM_CUDA_OK(cudaGetLastError());
   return 0;

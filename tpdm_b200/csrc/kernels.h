@@ -113,9 +113,24 @@ struct QueueArgs {
   unsigned long long seed;
   const float* ratios_all;
   float *rec_alphas, *rec_betas, *rec_logprobs;
+  // stream mode (tpdm_stream_*): prompt ids are ring entry ids; `order` is the ring [capacity] ticket -> entry, `counters` the
+  // stream's kStream* counters and `done_log` [capacity] the completion log.  `ticket`, `n_prompts`, `init_*` are unused.
+  int* counters;
+  int* done_log;
+  int capacity;
 };
+enum StreamCounter { kStreamSubmitted = 0, kStreamClaimed, kStreamCompleted, kStreamExecuted, kStreamCounters };
 int k_queue_schedule(const QueueArgs& a, cudaStream_t s);
 int k_queue_advance(const QueueArgs& a, cudaStream_t s);
+// stream mode: retire finished slots into the completion log, then every slot without a prompt (finished now or idle before)
+// claims the next submitted ticket in slot order.  admit = 1: no step ran (after an admission): only idle slots claim.
+int k_stream_advance(const QueueArgs& a, int admit, cudaStream_t s);
+// order[(submitted + k) % capacity] = entries[k] for k < n, then submitted += n (one thread, stream-ordered)
+constexpr int kStreamPublishMax = 64;
+struct StreamEntries {
+  int id[kStreamPublishMax];
+};
+int k_stream_publish(int* order, int* counters, int capacity, const StreamEntries& e, int n, cudaStream_t s);
 // per occupied slot b at (prompt, step) = (slot_prompt[b], slot_step[b]): tembs_all[prompt][step] = temb_cfg[b] ([D]) and
 // tpm_all[prompt][step] = tpm_x[b] (tpm_elems bf16); either destination may be null
 int k_queue_record(const int* slot_prompt, const int* slot_step, int B, int max_steps, int D, const float* temb_cfg, float* tembs_all,

@@ -6,6 +6,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import weakref
 from typing import Dict, Optional, Tuple
 
 import torch
@@ -297,6 +298,7 @@ class Engine:
                 pack_fp8_blocks(self.weights, transformer_sd, transformer_cfg, device)
                 L.check(lib.tpdm_set_fp8_weights(self.ctx, self.weights.fp8_blocks))
         self.plans: Dict[Tuple, Plan] = {}
+        self._streams = weakref.WeakSet()    # open PromptStreams: they read the packed weights from their own CUDA stream
         self.min_sigma = min_sigma
 
     def __del__(self):
@@ -311,8 +313,19 @@ class Engine:
         """Copy new TimePredictor values into the already packed device tensors (pointers and TMA descriptors unchanged)."""
         if not self.has_tpm:
             raise RuntimeError("engine was built without a TimePredictor")
+        busy = [st for st in self._streams if st._open and st._harvested != st._submitted]
+        if busy:
+            raise RuntimeError("the TimePredictor weights cannot change while an open prompt stream has requests in flight: their "
+                               "trajectories would switch weights part-way (drain or close the stream first)")
+        cur = torch.cuda.current_stream(self.device)
+        for st in self._streams:            # the copies run after the stream's queued steps and before its next ones
+            if st._open:
+                cur.wait_stream(st._cs)
         with torch.cuda.device(self.device):
             pack_time_predictor(self.weights, tpm_sd, self.device)
+        for st in self._streams:
+            if st._open:
+                st._cs.wait_stream(cur)
 
     def plan(self, batch: int, cfg_pairs: bool, latent: int, n_text: int, max_steps: int = 1) -> Plan:
         key = (batch, bool(cfg_pairs), latent, n_text, max_steps)
@@ -598,3 +611,227 @@ class Engine:
         torch.cuda.current_stream(dev).wait_stream(qs)
         self._queue_keepalive = (ws, lat, pe, ne, pp, npp, ticket, order, init_sigma, rt)
         return dict(latents=out_lat, steps=out_steps, sigmas=out_sig, device_steps=steps_run + (1 if init_step else 0), **rec)
+
+    def open_stream(self, slots: int, capacity: int, max_inference_steps: int, guidance_scale: float, use_graph: bool = True, *,
+                    latent: int, n_text: int = 333, prepare_latents=None) -> "PromptStream":
+        """An open device-side prompt queue (``tpdm_stream_*``): ``slots`` prompts in flight, up to ``capacity`` admitted and not
+        yet collected, prompts submitted while it runs.  The stream owns a private plan (outside ``self.plans``) and CUDA stream,
+        so ``sample``, ``sample_queue`` and ``mmdit_forward`` calls on this engine stay independent of it.  ``latent`` is the
+        latent side, ``n_text`` the text length every prompt must have; ``prepare_latents(n, generator, dtype)`` draws latents for
+        a ``submit`` without them."""
+        return PromptStream(self, slots, capacity, max_inference_steps, guidance_scale, use_graph, latent, n_text, prepare_latents)
+
+
+class PromptStream:
+    """Continuous batching for serving: ``submit`` admits prompts into the running queue, ``step`` runs denoising steps (every slot
+    whose trajectory ends takes the next submitted prompt on the device), ``results`` returns the requests that finished.  Each
+    request gets what batch-1 ``forward(predict=True)`` gives it.  Everything runs on the stream's own CUDA stream; the host
+    looks at the device counters one step late, so it never stalls the device while prompts are in flight.  The stream reads the
+    engine's packed weights: a TimePredictor refresh (``Engine.refresh_time_predictor``, which ``get_engine`` makes after an
+    optimizer step) raises RuntimeError while requests are in flight, and is ordered against the stream's steps otherwise."""
+
+    _READBACK_RING = 64
+
+    def __init__(self, engine: Engine, slots: int, capacity: int, max_steps: int, guidance_scale: float, use_graph: bool, latent: int,
+                 n_text: int, prepare_latents=None):
+        if slots < 1 or capacity < 1:
+            raise ValueError(f"slots ({slots}) and capacity ({capacity}) must be positive")
+        if not (engine.has_mmdit and engine.has_tpm):
+            raise RuntimeError("a prompt stream needs both MMDiT and TimePredictor weights")
+        lib = L.load()
+        dev = engine.device
+        self.engine, self.slots, self.capacity, self.max_steps, self.latent, self.n_text = engine, slots, capacity, max_steps, latent, n_text
+        self._prepare_latents = prepare_latents
+        self._step_fn = lib.tpdm_queue_step_graph if use_graph else lib.tpdm_queue_step
+        with torch.cuda.device(dev):
+            self._plan = Plan(engine, slots, True, latent, n_text, max_steps)    # private: never handed out by Engine.plan
+            self._cs = torch.cuda.Stream(device=dev)
+            nbytes = lib.tpdm_stream_workspace_bytes(self._plan.handle, capacity)
+            self._ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
+            base = (self._ws.data_ptr() + 1023) // 1024 * 1024
+            self._cs.wait_stream(torch.cuda.current_stream(dev))
+            with torch.cuda.stream(self._cs):
+                L.check(lib.tpdm_stream_open(self._plan.handle, capacity, float(guidance_scale), base, nbytes, L.stream_ptr()))
+            self._open = True
+            engine._streams.add(self)
+            ptrs = [L.vp() for _ in range(5)]
+            L.check(lib.tpdm_stream_status(self._plan.handle, *[C.byref(p) for p in ptrs]))
+        Cc = engine.cfg["in_channels"]
+        view = lambda p, dtype, shape: self._view(p.value, dtype, shape)
+        self._counters = view(ptrs[0], torch.int32, (6,))            # submitted, claimed, completed, executed, active, skip flag
+        self._log = view(ptrs[1], torch.int32, (capacity,))
+        self._out_lat = view(ptrs[2], torch.float32, (capacity, Cc, latent, latent))
+        self._out_steps = view(ptrs[3], torch.int32, (capacity,))
+        self._out_sig = view(ptrs[4], torch.float32, (capacity, max_steps + 1))
+        self._host = torch.zeros(self._READBACK_RING, 6, dtype=torch.int32).pin_memory()
+        self._pending = []                       # (event, ring row) of readbacks not yet looked at, oldest first
+        self._reads = 0
+        self._last = [0] * 6                     # the newest readback looked at
+        self._free = list(range(capacity - 1, -1, -1))
+        self._entry_req = {}                     # entry -> request id
+        self._next_id = self._submitted = self._harvested = 0
+        self._freed = []                         # events after the copies out of entries freed since the last submit
+
+    def _view(self, ptr: int, dtype: torch.dtype, shape) -> torch.Tensor:
+        off = ptr - self._ws.data_ptr()
+        n = 1
+        for s in shape:
+            n *= s
+        return self._ws[off: off + n * torch.empty((), dtype=dtype).element_size()].view(dtype).view(shape)
+
+    def _check_open(self):
+        if not self._open:
+            raise RuntimeError("the prompt stream is closed")
+
+    # ---- admission ---------------------------------------------------------------------------------------------
+    def submit(self, prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds, negative_pooled_prompt_embeds, latents=None,
+               generator=None) -> list:
+        """Admit n prompts; returns their request ids (increasing).  Latents default to ``prepare_latents`` (as ``forward`` draws
+        them).  A ring without n free entries raises RuntimeError and admits nothing."""
+        self._check_open()
+        eng, dev, f32 = self.engine, self.engine.device, torch.float32
+        n = prompt_embeds.shape[0]
+        J, PD, Cc = eng.cfg["joint_attention_dim"], eng.cfg["pooled_projection_dim"], eng.cfg["in_channels"]
+        if latents is None:
+            if self._prepare_latents is None:
+                raise ValueError("latents are required (this stream has no latent sampler)")
+            latents = self._prepare_latents(n, generator, prompt_embeds.dtype)
+        want = dict(prompt_embeds=(n, self.n_text, J), negative_prompt_embeds=(n, self.n_text, J), pooled_prompt_embeds=(n, PD),
+                    negative_pooled_prompt_embeds=(n, PD), latents=(n, Cc, self.latent, self.latent))
+        got = dict(prompt_embeds=prompt_embeds, negative_prompt_embeds=negative_prompt_embeds, pooled_prompt_embeds=pooled_prompt_embeds,
+                   negative_pooled_prompt_embeds=negative_pooled_prompt_embeds, latents=latents)
+        for k, shape in want.items():
+            if tuple(got[k].shape) != shape:
+                raise ValueError(f"{k} must have shape {shape} (text length {self.n_text}), got {tuple(got[k].shape)}")
+        if n < 1:
+            raise ValueError("submit needs at least one prompt")
+        if n > len(self._free):
+            raise RuntimeError(f"the prompt stream is full: {n} prompts for {len(self._free)} free entries of {self.capacity}")
+        cvt = lambda t: t.to(device=dev, dtype=f32).contiguous()
+        ts = [cvt(latents), cvt(negative_prompt_embeds), cvt(prompt_embeds), cvt(negative_pooled_prompt_embeds), cvt(pooled_prompt_embeds)]
+        entries = self._free[len(self._free) - n:][::-1]       # taken off the free list only once the library accepted them
+        ids = (C.c_int * n)(*entries)
+        self._cs.wait_stream(torch.cuda.current_stream(dev))   # the inputs
+        for ev in self._freed:
+            self._cs.wait_event(ev)
+        with torch.cuda.device(dev), torch.cuda.stream(self._cs):
+            L.check(L.load().tpdm_stream_submit(self._plan.handle, n, ids, *[L.ptr(t) for t in ts], L.stream_ptr()))
+        del self._free[len(self._free) - n:]
+        self._freed.clear()
+        for t in ts:
+            t.record_stream(self._cs)            # alive until the admission kernels have read them
+        rids = list(range(self._next_id, self._next_id + n))
+        self._entry_req.update(zip(entries, rids))
+        self._next_id += n
+        self._submitted += n
+        return rids
+
+    # ---- steps -------------------------------------------------------------------------------------------------
+    def _consume(self, block: bool):
+        """Look at the readbacks in order: all completed ones, and with ``block`` the older ones than the newest (one step late)."""
+        while self._pending:
+            ev, row = self._pending[0]
+            if not ev.query():
+                if not (block and len(self._pending) > 1):
+                    break
+                ev.synchronize()
+            self._last = self._host[row].tolist()
+            self._pending.pop(0)
+
+    def _idle(self) -> bool:
+        # no slot held a prompt after the newest step looked at, and nothing was submitted since
+        return self._last[4] == 0 and self._last[0] == self._submitted
+
+    def step(self, n: int = 1) -> None:
+        """Enqueue up to n denoising steps.  Stops (launching nothing) once no slot is active and nothing is pending."""
+        self._check_open()
+        dev = self.engine.device
+        with torch.cuda.device(dev), torch.cuda.stream(self._cs):
+            stream = L.stream_ptr()
+            for _ in range(n):
+                self._consume(block=False)
+                if self._idle():
+                    break
+                L.check(self._step_fn(self._plan.handle, stream))
+                row = self._reads % self._READBACK_RING
+                self._reads += 1
+                self._host[row].copy_(self._counters, non_blocking=True)
+                ev = torch.cuda.Event()
+                ev.record()
+                self._pending.append((ev, row))
+                self._consume(block=True)      # the flags of the previous step: the device never waits for the host
+
+    @property
+    def device_steps(self) -> int:
+        """Denoising steps the device executed (steps skipped on an idle stream are not counted)."""
+        self._check_open()
+        self._cs.synchronize()
+        self._consume(block=False)
+        return int(self._last[3])
+
+    # ---- completions -------------------------------------------------------------------------------------------
+    def results(self) -> dict:
+        """``{request id: dict(latents (C, h, w), steps, sigmas (steps,))}`` of the requests finished since the last call, as far as
+        the host has seen (one step late); their entries are free again."""
+        self._check_open()
+        self._consume(block=False)
+        done = self._last[2]
+        if done == self._harvested:
+            return {}
+        dev = self.engine.device
+        cur = torch.cuda.current_stream(dev)
+        with torch.cuda.device(dev):
+            # those log entries and outputs were written by steps that have completed; the steps queued after them do not touch them
+            k = torch.arange(self._harvested, done, device=dev) % self.capacity
+            ents = self._log[k].long()
+            steps = self._out_steps[ents].tolist()
+            lat = self._out_lat[ents].clone()
+            sig = self._out_sig[ents].clone()
+        out = {}
+        for j, (e, s) in enumerate(zip(ents.tolist(), steps)):
+            out[self._entry_req.pop(e)] = dict(latents=lat[j], steps=s, sigmas=sig[j, 1: s + 1])
+            self._free.append(e)
+        self._harvested = done
+        ev = torch.cuda.Event()
+        ev.record(cur)                         # the next admission, which may reuse these entries, runs after these copies
+        self._freed.append(ev)
+        return out
+
+    def drain(self) -> dict:
+        """Step until every submitted request has finished; returns the results not collected yet."""
+        self._check_open()
+        out = {}
+        bound = (self._submitted - self._harvested + self.slots - 1) // self.slots * self.max_steps + 2 * self.max_steps + 4
+        for _ in range(bound):
+            out.update(self.results())
+            if self._harvested == self._submitted:
+                return out
+            self.step()
+            if self._idle():
+                self._cs.synchronize()
+                self._consume(block=False)
+        out.update(self.results())
+        if self._harvested != self._submitted:
+            raise RuntimeError("the prompt stream did not drain within the step bound")
+        return out
+
+    def close(self) -> None:
+        if not self._open:
+            return
+        self._cs.synchronize()
+        L.check(L.load().tpdm_stream_close(self._plan.handle))
+        self._open = False
+        self.engine._streams.discard(self)
+        self._pending.clear()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass

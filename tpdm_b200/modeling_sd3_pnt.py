@@ -419,6 +419,20 @@ class SD3PredictNextTimeStepModel(nn.Module):
             betas=None, sigmas=res["sigmas"], logprobs=None, prob_masks=None, latents=res["latents"], steps=res["steps"],
             device_steps=res["device_steps"])
 
+    def open_prompt_stream(self, slots: int, capacity: int, max_inference_steps: int = 28, guidance_scale: float = 7.0,
+                           use_graph: bool = True, n_text: int = 333):
+        """An open prompt queue for serving (engine.PromptStream): ``slots`` prompts in flight, up to ``capacity`` admitted and
+        not yet collected.  ``submit`` admits prompts while it runs (latents drawn as ``forward`` draws them when not given),
+        ``step`` runs denoising steps, ``results`` returns the finished requests; each gets what ``forward(predict=True)`` with
+        batch size 1 gives it.  ``n_text`` is the text length of every prompt (333 for SD3's CLIP + T5 embeddings)."""
+        if guidance_scale is None:
+            raise ValueError("guidance_scale=None is unsupported (as in the reference, whose sigma.repeat(2) is unconditional, :526)")
+        side = self.default_sample_size * self.vae_scale_factor
+        C = self.transformer.config.in_channels
+        draw = lambda n, generator, dtype: self.prepare_latents(n, C, side, side, dtype, self.device, generator, None)
+        return self.get_engine().open_stream(int(slots), int(capacity), int(max_inference_steps), float(guidance_scale), use_graph,
+                                             latent=side // self.vae_scale_factor, n_text=int(n_text), prepare_latents=draw)
+
     # ---------------------------------------------------------------------------------------------------------------
     def _replay_trainer(self, grid: int, samples: int):
         """TimePredictorTrainer (native forward with saved activations + backward) behind the differentiable replay."""
