@@ -447,6 +447,40 @@ int tpdm_ln_modulate_fp8(const float* x, const float* shift, const float* scale,
  * accumulation; epi 0 -> bf16, 1 -> f32, 2 gelu -> bf16.  N > 128, K % 16 == 0. */
 int tpdm_gemm_fp8(const void* A8, const float* a_scale, const void* W8, const float* w_scale, const float* bias, void* out, int batch,
                   int rows, int N, int K, int epi, void* stream);
+/* Launch guards of the calling thread, the two the device-side prompt queue uses: when *skip_flag != 0 (device int) every
+ * guarded launch returns at once; batch entry b of a launch is skipped when slot_active[b % slots] == 0 (device int[slots]).
+ * They apply to every later launch of this library on the thread -- plan calls included -- until they are cleared with
+ * (NULL, NULL, 1).  tpdm_queue_step clears both when it returns; tpdm_sample_step clears only the skip flag.  Guarded: the GEMMs
+ * (both kernels, bf16 and E4M3), attention and ln_modulate (bf16 and E4M3).  slots < 1 is TPDM_ERR_ARG. */
+int tpdm_set_launch_guards(const int* skip_flag, const int* slot_active, int slots);
+/* One op of tpdm_gemm_ops: out = epilogue(A . W^T) as in tpdm_gemm_bf16, with free strides.  Element (b, r, k) of A is at
+ * A + b * a_batch_stride + r * a_row_stride + k; output element (b, r, n) at out + b * out_batch_stride + r * ldo + n; the gate of
+ * epi 3 at gate + b * gate_stride + n (strides in elements).  a_scale / w_scale both set: A and W are E4M3 codes with row
+ * scales [batch][rows] and channel scales [N] (epi 0-2, N > 128; see tpdm_gemm_fp8); one of them alone is TPDM_ERR_ARG.
+ * ksplit > 1: K is cut into ksplit ranges of ceil(nkb / ksplit) 64-wide k-blocks (nkb = ceil(K / 64)); range s writes its
+ * partial product to out + (s * batch + b) * out_batch_stride (bias-free epi 1 with N <= 128 only). */
+typedef struct tpdm_gemm_op_desc {
+  const void* A;
+  int64_t a_row_stride;
+  int64_t a_batch_stride;
+  const void* W;
+  void* out;
+  int64_t out_batch_stride;
+  const float* bias;     /* [N] or NULL */
+  const float* gate;     /* epi 3 only */
+  const float* a_scale;  /* E4M3 operands only */
+  const float* w_scale;
+  int32_t rows;
+  int32_t batch;
+  int32_t K;
+  int32_t N;
+  int32_t epi;           /* 0 bias->bf16, 1 bias->f32, 2 bias+gelu->bf16, 3 out(f32) += gate * (acc + bias) */
+  int32_t ldo;
+  int32_t gate_stride;
+  int32_t ksplit;        /* 1 = no split */
+} tpdm_gemm_op_desc;
+/* One persistent GEMM launch over n_ops (1 or 2) ops, the grouped form the MMDiT blocks use for the image and text streams. */
+int tpdm_gemm_ops(const tpdm_gemm_op_desc* ops, int n_ops, void* stream);
 
 #ifdef __cplusplus
 }

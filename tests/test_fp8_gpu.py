@@ -6,6 +6,8 @@ the plain fp32 oracle the error is printed and held to 4e-2."""
 import pytest
 import torch
 
+from kernel_check import assert_launch, gemm_magnitude, guarded
+
 pytestmark = pytest.mark.gpu
 
 VEL_TOL, PLAIN_VEL_TOL, SIGMA_TOL, LATENT_TOL = 2e-2, 4e-2, 1e-3, 3e-2
@@ -98,7 +100,8 @@ GEMM_SHAPES = [   # (batch, rows, N, K, epi): SD3-M QKV image rows and text tail
 
 @pytest.mark.parametrize("batch,rows,N,K,epi", GEMM_SHAPES)
 def test_gemm_fp8_vs_dequantized_fp32(L, batch, rows, N, K, epi):
-    _no_tf32()
+    """every element against the float64 product of the dequantized operands (tests/kernel_check.py); nothing written outside
+    [batch][rows][N]"""
     lib = L.load()
     torch.manual_seed(2)
     A = torch.randn(batch, rows, K, device="cuda")
@@ -106,18 +109,16 @@ def test_gemm_fp8_vs_dequantized_fp32(L, batch, rows, N, K, epi):
     bias = torch.randn(N, device="cuda") * 0.1
     a8, a_s = _quantize(L, A)
     w8, w_s = _quantize(L, W)
-    deq = lambda c, s: c.view(torch.float8_e4m3fn).float() * s.unsqueeze(-1)
-    acc = deq(a8, a_s) @ deq(w8, w_s).t() + bias
-    if epi == 1:
-        out, tol = torch.zeros(batch, rows, N, device="cuda"), 1e-4
-    else:
-        out, tol = torch.zeros(batch, rows, N, device="cuda", dtype=torch.bfloat16), 2e-3
-    ref = torch.nn.functional.gelu(acc, approximate="tanh") if epi == 2 else acc
+    deq = lambda c, s: c.view(torch.float8_e4m3fn).double() * s.double().unsqueeze(-1)
+    a64, w64 = deq(a8, a_s), deq(w8, w_s)
+    pre = a64 @ w64.t() + bias.double()
+    mag = gemm_magnitude(a64, w64, bias)
+    buf, out = guarded((batch, rows, N), torch.float32 if epi == 1 else torch.bfloat16)
+    ref = torch.nn.functional.gelu(pre, approximate="tanh") if epi == 2 else pre
+    before = buf.clone()
     L.check(lib.tpdm_gemm_fp8(L.ptr(a8), L.ptr(a_s), L.ptr(w8), L.ptr(w_s), L.ptr(bias), L.ptr(out), batch, rows, N, K, epi, None))
     torch.cuda.synchronize()
-    e = rel(out, ref)
-    print(f"[gemm fp8 {batch}x{rows}x{N}x{K} epi {epi}] rel-L2 {e:.2e}")
-    assert e <= tol
+    assert_launch(buf, before, [(out, ref, mag, pre if epi == 2 else None)], what=f"gemm fp8 {batch}x{rows}x{N}x{K} epi {epi}")
 
 
 def test_gemm_fp8_rejects_bad_arguments(L):

@@ -73,6 +73,12 @@ class TpdmSampleState(C.Structure):
                                   "all_done", "tembs", "tpm_input", "history_latents")]
 
 
+class TpdmGemmOpDesc(C.Structure):
+    _fields_ = ([("A", vp), ("a_row_stride", C.c_int64), ("a_batch_stride", C.c_int64), ("W", vp), ("out", vp),
+                 ("out_batch_stride", C.c_int64)] + [(n, vp) for n in ("bias", "gate", "a_scale", "w_scale")] +
+                [(n, C.c_int32) for n in ("rows", "batch", "K", "N", "epi", "ldo", "gate_stride", "ksplit")])
+
+
 EXPORTS = {
     "tpdm_last_error": (C.c_char_p, []),
     "tpdm_abi_version": (C.c_int, []),
@@ -135,6 +141,8 @@ EXPORTS = {
     "tpdm_quantize_fp8_rows": (C.c_int, [vp, C.c_int, C.c_int, vp, vp, vp]),
     "tpdm_ln_modulate_fp8": (C.c_int, [vp, vp, vp, C.c_int, vp, vp, C.c_int, C.c_int, C.c_int, vp]),
     "tpdm_gemm_fp8": (C.c_int, [vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
+    "tpdm_set_launch_guards": (C.c_int, [vp, vp, C.c_int]),
+    "tpdm_gemm_ops": (C.c_int, [C.POINTER(TpdmGemmOpDesc), C.c_int, vp]),
 }
 
 _lib = None

@@ -1168,4 +1168,34 @@ int tpdm_gemm_fp8(const void* A8, const float* a_scale, const void* W8, const fl
   return gemm_launch(&op, 1, static_cast<cudaStream_t>(stream));
 }
 
+int tpdm_set_launch_guards(const int* skip, const int* slot_active, int slots) {
+  TPDM_CHECK(slots >= 1, TPDM_ERR_ARG, "tpdm_set_launch_guards: slots %d < 1", slots);
+  set_skip_flag(skip);
+  set_batch_mask(slot_active, slots);
+  return 0;
+}
+
+int tpdm_gemm_ops(const tpdm_gemm_op_desc* ops, int n_ops, void* stream) {
+  TPDM_CHECK(ops, TPDM_ERR_ARG, "tpdm_gemm_ops: null argument");
+  TPDM_CHECK(n_ops >= 1 && n_ops <= 2, TPDM_ERR_ARG, "tpdm_gemm_ops: %d ops (1 or 2 per launch)", n_ops);
+  for (int i = 0; i < n_ops; ++i) {
+    const tpdm_gemm_op_desc& d = ops[i];
+    TPDM_CHECK(d.A && d.W && d.out, TPDM_ERR_ARG, "tpdm_gemm_ops: op %d: null argument", i);
+    TPDM_CHECK(d.epi >= 0 && d.epi <= 3, TPDM_ERR_ARG, "tpdm_gemm_ops: op %d: epilogue %d unknown", i, d.epi);
+    TPDM_CHECK((d.a_scale == nullptr) == (d.w_scale == nullptr), TPDM_ERR_ARG, "tpdm_gemm_ops: op %d: E4M3 operands need both scales", i);
+  }
+  GemmOp g[2];
+  for (int i = 0; i < n_ops; ++i) {
+    const tpdm_gemm_op_desc& d = ops[i];
+    if (d.a_scale)
+      TPDM_TRY(gemm_op_init_fp8(&g[i], d.A, d.a_row_stride, d.a_batch_stride, d.a_scale, d.rows, d.batch, d.K, d.W, d.w_scale, d.N, d.epi,
+                                d.out, d.out_batch_stride, d.ldo, d.bias));
+    else
+      TPDM_TRY(gemm_op_init(&g[i], d.A, d.a_row_stride, d.a_batch_stride, d.rows, d.batch, d.K, d.W, d.N, d.epi, d.out, d.out_batch_stride,
+                            d.ldo, d.bias, d.gate, d.gate_stride));
+    TPDM_TRY(gemm_op_set_ksplit(&g[i], d.ksplit));
+  }
+  return gemm_launch(g, n_ops, static_cast<cudaStream_t>(stream));
+}
+
 }  // extern "C"
