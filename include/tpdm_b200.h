@@ -318,9 +318,17 @@ int tpdm_queue_status(tpdm_plan* plan, const int** active_slots, const int** slo
  * Steps are tpdm_queue_step / tpdm_queue_step_graph on the plan (one captured graph: the ring, counters and staging never move).
  * A slot without a prompt -- its trajectory just ended, or it was idle -- takes the next submitted ticket in slot order (no
  * atomics, deterministic); a step of a stream with no active slot is skipped on the device.  Each request follows exactly the
- * trajectory tpdm_sample_* gives it with batch 1 and predict = 1.  TPDM_ERR_STATE: open on a plan whose queue has begun or whose
- * stream is open; tpdm_queue_begin / tpdm_sample_begin / tpdm_queue_set_rollout while the stream is open; the other stream
- * calls without an open stream.
+ * trajectory tpdm_sample_* gives it with batch 1 and predict = 1.
+ * A plan's buffers belong to one driver at a time: the lockstep sampler after tpdm_sample_begin, the closed queue after
+ * tpdm_queue_begin, the open stream from tpdm_stream_open to tpdm_stream_close.  Each begin hands the plan to its driver, and a
+ * call that needs another owner returns TPDM_ERR_STATE and enqueues nothing:
+ *   tpdm_sample_begin, tpdm_queue_begin           refused while a stream is open
+ *   tpdm_sample_step, tpdm_sample_step_graph      need the sampler: refused after a later tpdm_queue_begin / tpdm_stream_open
+ *   tpdm_queue_set_rollout                        needs the closed queue
+ *   tpdm_queue_step, _step_graph, tpdm_queue_status   need the closed queue or the stream: refused after a later
+ *                                                 tpdm_sample_begin (its steps would run on the slots the sampler overwrote)
+ *   tpdm_stream_open                              refused while a queue owns the plan or a stream is open
+ *   tpdm_stream_submit, _status, _close           need the open stream; after close the plan is owned by nobody
  * ---------------------------------------------------------------------------------------------------------------- */
 size_t tpdm_stream_workspace_bytes(const tpdm_plan* plan, int capacity);
 /* workspace: 1 KiB aligned, >= tpdm_stream_workspace_bytes; borrowed until tpdm_stream_close.  Encodes the TMA maps of the

@@ -3,6 +3,7 @@ or a call fails, an exception is raised."""
 from __future__ import annotations
 
 import ctypes as C
+import math
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -190,3 +191,19 @@ def stream_ptr() -> int:
     import torch
 
     return torch.cuda.current_stream().cuda_stream
+
+
+def aligned_workspace(nbytes: int, device):
+    """A device byte tensor holding ``nbytes`` bytes from a 1 KiB-aligned address on, as the library's workspaces need:
+    (tensor, that address)."""
+    import torch
+
+    ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=device)
+    return ws, (ws.data_ptr() + 1023) // 1024 * 1024
+
+
+def view_at(ws, ptr: int, dtype, shape):
+    """Typed view of the buffer the library placed at device address ``ptr`` inside the workspace tensor ``ws``."""
+    off = ptr - ws.data_ptr()
+    n = math.prod(shape) * dtype.itemsize
+    return ws[off: off + n].view(dtype).view(shape)

@@ -51,6 +51,28 @@ struct Carver {
   }
 };
 
+// which driver owns the plan's buffers: the lockstep sampler, the closed prompt queue or the open prompt stream
+enum class Mode { kIdle, kSample, kQueue, kStream };
+
+// one captured step and the launches it replays
+struct StepGraph {
+  cudaGraphExec_t exec = nullptr;
+  long long launches = 0;
+  StepGraph() = default;
+  StepGraph(const StepGraph&) = delete;
+  StepGraph& operator=(StepGraph&& o) noexcept {  // the moved-from graph destroys what this one held
+    std::swap(exec, o.exec);
+    std::swap(launches, o.launches);
+    return *this;
+  }
+  void drop() {
+    if (exec) cudaGraphExecDestroy(exec);
+    exec = nullptr;
+    launches = 0;
+  }
+  ~StepGraph() { drop(); }
+};
+
 }  // namespace
 
 struct tpdm_plan {
@@ -71,13 +93,14 @@ struct tpdm_plan {
   float *latents, *velocity, *sigma_hist, *alphas, *betas, *logprobs, *tembs, *history, *ratios;
   int *masks, *all_done;
   float guidance = 7.0f;
-  int predict = 1, begun = 0, have_ratios = 0;
+  int predict = 1, have_ratios = 0;
+  Mode mode = Mode::kIdle;
   unsigned long long seed = 0;
   std::vector<BlockOps> blk;
   GemmOp ctx_embed, proj_out, conv1;
   // device-side prompt queue (tpdm_queue_*): the plan's batch entries are in-flight slots
   struct Queue {
-    int n_prompts = 0, begun = 0;
+    int n_prompts = 0;
     const float* noise_all = nullptr;
     float *ctx0_all = nullptr, *text_all = nullptr, *sigma_cur = nullptr, *sigma_next = nullptr, *out_latents = nullptr, *out_sigmas = nullptr;
     int *slot_prompt = nullptr, *slot_step = nullptr, *slot_flush = nullptr, *slot_load = nullptr, *slot_active = nullptr, *ticket = nullptr,
@@ -91,12 +114,11 @@ struct tpdm_plan {
     const float* ratios_all = nullptr;
     float *rec_alphas = nullptr, *rec_betas = nullptr, *rec_logprobs = nullptr, *rec_tembs = nullptr;
     bf16* rec_tpm = nullptr;
-    cudaGraphExec_t graph = nullptr;   // one captured queue step (every pointer of a queue step is fixed between steps)
-    long long graph_launches = 0;
+    StepGraph graph;   // one captured queue step (every pointer of a queue step is fixed between steps)
   } q;
   // open prompt stream (tpdm_stream_*): the queue above runs over a ring of `capacity` entries, prompts are admitted between steps
   struct Stream {
-    int open = 0, capacity = 0;
+    int capacity = 0;
     int *order = nullptr, *counters = nullptr, *done_log = nullptr;
     float* noise = nullptr;
     // admission staging, never read by a queue step: bf16 text [2*slots][T][J] (row 2k + half), its context_embedder output and
@@ -107,23 +129,63 @@ struct tpdm_plan {
   } st;
   // tpdm_sample_step_graph: one captured graph per step index (the step index only moves pointers inside the plan's own buffers),
   // valid for the guidance / predict / injected-ratio setting they were captured under
-  std::vector<cudaGraphExec_t> step_graph;
-  std::vector<long long> step_graph_launches;
+  std::vector<StepGraph> step_graph;
   float graph_guidance = 0.f;
   int graph_predict = -1, graph_have_ratios = -1;
-  void drop_step_graphs() {
-    for (cudaGraphExec_t g : step_graph)
-      if (g) cudaGraphExecDestroy(g);
-    step_graph.clear();
-    step_graph_launches.clear();
-  }
-  ~tpdm_plan() {
-    if (q.graph) cudaGraphExecDestroy(q.graph);
-    drop_step_graphs();
-  }
 };
 
 namespace {
+
+constexpr unsigned in(Mode m) { return 1u << static_cast<int>(m); }
+
+// TPDM_ERR_STATE unless the plan is in one of the `allowed` modes (a mask of in(Mode)); the message says what comes first
+int check_mode(const tpdm_plan* p, unsigned allowed, const char* who) {
+  if (allowed & in(p->mode)) return 0;
+  const char* why = p->mode == Mode::kStream        ? "the plan has an open prompt stream (tpdm_stream_close first)"
+                    : allowed == in(Mode::kSample)  ? "call tpdm_sample_begin first"
+                    : allowed & in(Mode::kQueue)    ? "call tpdm_queue_begin first"
+                    : allowed == in(Mode::kStream)  ? "the plan has no open stream"
+                                                    : "a prompt queue runs on this plan";
+  return fail(TPDM_ERR_STATE, "%s: %s", who, why);
+}
+
+// Replays g, capturing it from enqueue(stream) on first use.  The launch counters count a replay like the plain launches.
+template <typename F>
+int replay_or_capture(StepGraph& g, cudaStream_t s, const char* who, F enqueue) {
+  if (g.exec == nullptr) {
+    const long long before = launches_so_far();
+    cudaGraph_t graph = nullptr;
+    TPDM_CUDA_OK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+    const int st = enqueue(s);
+    const cudaError_t e = cudaStreamEndCapture(s, &graph);
+    if (st != 0) {
+      if (graph) cudaGraphDestroy(graph);
+      return st;
+    }
+    TPDM_CHECK(e == cudaSuccess && graph != nullptr, TPDM_ERR_CUDA, "%s: stream capture failed: %s", who, cudaGetErrorString(e));
+    const cudaError_t ei = cudaGraphInstantiate(&g.exec, graph, 0);
+    cudaGraphDestroy(graph);
+    TPDM_CHECK(ei == cudaSuccess, TPDM_ERR_CUDA, "%s: cudaGraphInstantiate failed: %s", who, cudaGetErrorString(ei));
+    g.launches = launches_so_far() - before;
+    count_launches(-g.launches);  // the capture itself launched nothing
+  }
+  TPDM_CUDA_OK(cudaGraphLaunch(g.exec, s));
+  count_launches(g.launches);
+  return 0;
+}
+
+void set_shape(tpdm_plan* p, int batch, int cfg_pairs, int latent_h, int latent_w, int n_text, int max_steps) {
+  p->B = batch;
+  p->cfg_pairs = cfg_pairs ? 1 : 0;
+  p->Bt = cfg_pairs ? 2 * batch : batch;
+  p->Hl = latent_h;
+  p->Wl = latent_w;
+  p->g = latent_w / 2;
+  p->N = p->g * p->g;
+  p->T = n_text;
+  p->S = p->N + p->T;
+  p->max_steps = max_steps;
+}
 
 void carve(tpdm_plan* p, Carver& c) {
   const tpdm_ctx* ctx = p->ctx;
@@ -489,15 +551,7 @@ size_t tpdm_plan_workspace_bytes(const tpdm_ctx* ctx, int batch, int cfg_pairs, 
   if (check_shapes(ctx, batch, latent_h, latent_w, n_text, max_steps) != 0) return 0;
   tpdm_plan p;
   p.ctx = const_cast<tpdm_ctx*>(ctx);
-  p.B = batch;
-  p.Bt = cfg_pairs ? 2 * batch : batch;
-  p.Hl = latent_h;
-  p.Wl = latent_w;
-  p.g = latent_w / 2;
-  p.N = p.g * p.g;
-  p.T = n_text;
-  p.S = p.N + p.T;
-  p.max_steps = max_steps;
+  set_shape(&p, batch, cfg_pairs, latent_h, latent_w, n_text, max_steps);
   Carver c(nullptr);
   carve(&p, c);
   return c.off + 1024;
@@ -514,16 +568,7 @@ int tpdm_plan_create(tpdm_ctx* ctx, int batch, int cfg_pairs, int latent_h, int 
   tpdm_plan* p = new (std::nothrow) tpdm_plan();
   TPDM_CHECK(p, TPDM_ERR_NOMEM, "out of host memory");
   p->ctx = ctx;
-  p->B = batch;
-  p->cfg_pairs = cfg_pairs ? 1 : 0;
-  p->Bt = cfg_pairs ? 2 * batch : batch;
-  p->Hl = latent_h;
-  p->Wl = latent_w;
-  p->g = latent_w / 2;
-  p->N = p->g * p->g;
-  p->T = n_text;
-  p->S = p->N + p->T;
-  p->max_steps = max_steps;
+  set_shape(p, batch, cfg_pairs, latent_h, latent_w, n_text, max_steps);
   Carver c(workspace);
   carve(p, c);
   int st = build_ops(p);
@@ -576,7 +621,7 @@ int tpdm_sample_begin(tpdm_plan* p, const float* latents, const float* neg_embed
                       void* stream) {
   TPDM_CHECK(p && latents && neg_embeds && pos_embeds && neg_pooled && pos_pooled, TPDM_ERR_ARG, "tpdm_sample_begin: null argument");
   TPDM_CHECK(p->cfg_pairs, TPDM_ERR_STATE, "tpdm_sample_begin: the plan was created without cfg_pairs");
-  TPDM_CHECK(!p->st.open, TPDM_ERR_STATE, "tpdm_sample_begin: the plan has an open prompt stream (tpdm_stream_close first)");
+  TPDM_TRY(check_mode(p, in(Mode::kIdle) | in(Mode::kSample) | in(Mode::kQueue), "tpdm_sample_begin"));
   TPDM_CHECK(p->ctx->has_mmdit && p->ctx->has_tpm, TPDM_ERR_STATE, "tpdm_sample_begin: needs both MMDiT and TimePredictor weights");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const tpdm_ctx* ctx = p->ctx;
@@ -591,13 +636,13 @@ int tpdm_sample_begin(tpdm_plan* p, const float* latents, const float* neg_embed
   // sigma = ones (modeling_sd3_pnt.py:508); stream-ordered like everything else (no host staging, no synchronisation)
   TPDM_TRY(k_sample_init(p->sigma_hist, p->masks, p->all_done, p->B, p->max_steps, s));
   TPDM_TRY(set_prompts(p, neg_embeds, pos_embeds, neg_pooled, pos_pooled, s));
-  p->begun = 1;
+  p->mode = Mode::kSample;
   return 0;
 }
 
 int tpdm_sample_step(tpdm_plan* p, int step, void* stream) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_sample_step: null plan");
-  TPDM_CHECK(p->begun, TPDM_ERR_STATE, "tpdm_sample_step: call tpdm_sample_begin first");
+  TPDM_TRY(check_mode(p, in(Mode::kSample), "tpdm_sample_step"));
   TPDM_CHECK(step >= 0 && step < p->max_steps, TPDM_ERR_ARG, "tpdm_sample_step: step %d outside [0,%d)", step, p->max_steps);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const tpdm_ctx* ctx = p->ctx;
@@ -637,42 +682,20 @@ int tpdm_sample_step(tpdm_plan* p, int step, void* stream) {
 
 int tpdm_sample_step_graph(tpdm_plan* p, int step, void* stream) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_sample_step_graph: null plan");
-  TPDM_CHECK(p->begun, TPDM_ERR_STATE, "tpdm_sample_step_graph: call tpdm_sample_begin first");
+  TPDM_TRY(check_mode(p, in(Mode::kSample), "tpdm_sample_step_graph"));
   TPDM_CHECK(step >= 0 && step < p->max_steps, TPDM_ERR_ARG, "tpdm_sample_step_graph: step %d outside [0,%d)", step, p->max_steps);
   // The Philox seed of a sampled trajectory is a kernel argument that changes with every call, and per-launch profiling records
   // events on the stream: both take the plain path.  (predict / injected ratios never read the seed.)
   if ((!p->predict && !p->have_ratios) || profiling_active()) return tpdm_sample_step(p, step, stream);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (p->graph_guidance != p->guidance || p->graph_predict != p->predict || p->graph_have_ratios != p->have_ratios) {
-    p->drop_step_graphs();
+    p->step_graph.clear();
     p->graph_guidance = p->guidance;
     p->graph_predict = p->predict;
     p->graph_have_ratios = p->have_ratios;
   }
-  if (p->step_graph.empty()) {
-    p->step_graph.assign(p->max_steps, nullptr);
-    p->step_graph_launches.assign(p->max_steps, 0);
-  }
-  if (p->step_graph[step] == nullptr) {
-    const long long before = launches_so_far();
-    cudaGraph_t g = nullptr;
-    TPDM_CUDA_OK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-    const int st = tpdm_sample_step(p, step, s);
-    const cudaError_t e = cudaStreamEndCapture(s, &g);
-    if (st != 0) {
-      if (g) cudaGraphDestroy(g);
-      return st;
-    }
-    TPDM_CHECK(e == cudaSuccess && g != nullptr, TPDM_ERR_CUDA, "tpdm_sample_step_graph: stream capture failed: %s", cudaGetErrorString(e));
-    const cudaError_t ei = cudaGraphInstantiate(&p->step_graph[step], g, 0);
-    cudaGraphDestroy(g);
-    TPDM_CHECK(ei == cudaSuccess, TPDM_ERR_CUDA, "tpdm_sample_step_graph: cudaGraphInstantiate failed: %s", cudaGetErrorString(ei));
-    p->step_graph_launches[step] = launches_so_far() - before;
-    count_launches(-p->step_graph_launches[step]);  // the capture itself launched nothing
-  }
-  TPDM_CUDA_OK(cudaGraphLaunch(p->step_graph[step], s));
-  count_launches(p->step_graph_launches[step]);
-  return 0;
+  if (p->step_graph.empty()) p->step_graph = std::vector<StepGraph>(p->max_steps);
+  return replay_or_capture(p->step_graph[step], static_cast<cudaStream_t>(stream), "tpdm_sample_step_graph",
+                           [&](cudaStream_t s) { return tpdm_sample_step(p, step, s); });
 }
 
 int tpdm_sample_state_get(tpdm_plan* p, tpdm_sample_state* out) {
@@ -693,14 +716,23 @@ int tpdm_sample_state_get(tpdm_plan* p, tpdm_sample_state* out) {
 
 // ---- device-side prompt queue ------------------------------------------------------------------------------------
 namespace {
-size_t queue_bytes(const tpdm_plan* p, int n_prompts) {
-  const size_t ctx = static_cast<size_t>(p->T) * p->ctx->D, D = p->ctx->D, B = p->B;
-  Carver c(nullptr);
-  c.take<float>(static_cast<size_t>(n_prompts) * 2 * ctx);
-  c.take<float>(static_cast<size_t>(n_prompts) * 2 * D);
-  c.take<float>(2 * B);
-  c.take<int>(5 * B + 8);
-  return c.off + 1024;
+// text branch of every prompt + slot state + counters, in the order tpdm_queue_begin hands them out
+void carve_queue(tpdm_plan* p, int n_prompts, Carver& c) {
+  tpdm_plan::Queue& q = p->q;
+  const size_t n = n_prompts, B = p->B, D = p->ctx->D;
+  q.ctx0_all = c.take<float>(n * 2 * p->T * D);
+  q.text_all = c.take<float>(n * 2 * D);
+  q.sigma_cur = c.take<float>(2 * B);
+  q.sigma_next = q.sigma_cur ? q.sigma_cur + B : nullptr;
+  q.slot_prompt = c.take<int>(5 * B + 8);
+  if (q.slot_prompt) {
+    q.slot_step = q.slot_prompt + B;
+    q.slot_flush = q.slot_step + B;
+    q.slot_load = q.slot_flush + B;
+    q.slot_active = q.slot_load + B;
+    q.active = q.slot_active + B;
+    q.idle_flag = q.active + 1;
+  }
 }
 QueueArgs queue_args(const tpdm_plan* p, int init) {
   const tpdm_plan::Queue& q = p->q;
@@ -735,7 +767,7 @@ QueueArgs queue_args(const tpdm_plan* p, int init) {
   a.rec_alphas = q.rec_alphas;
   a.rec_betas = q.rec_betas;
   a.rec_logprobs = q.rec_logprobs;
-  if (p->st.open) {
+  if (p->mode == Mode::kStream) {
     a.order = p->st.order;
     a.counters = p->st.counters;
     a.done_log = p->st.done_log;
@@ -753,7 +785,12 @@ int queue_move(tpdm_plan* p, cudaStream_t s) {
 
 size_t tpdm_queue_workspace_bytes(const tpdm_plan* p, int n_prompts) {
   if (!p || n_prompts <= 0) return 0;
-  return queue_bytes(p, n_prompts);
+  tpdm_plan probe;
+  probe.ctx = p->ctx;
+  set_shape(&probe, p->B, p->cfg_pairs, p->Hl, p->Wl, p->T, p->max_steps);
+  Carver c(nullptr);
+  carve_queue(&probe, n_prompts, c);
+  return c.off + 1024;
 }
 
 int tpdm_queue_begin(tpdm_plan* p, int n_prompts, const float* latents_all, const float* neg_embeds_all, const float* pos_embeds_all,
@@ -764,36 +801,24 @@ int tpdm_queue_begin(tpdm_plan* p, int n_prompts, const float* latents_all, cons
                  out_latents && out_steps,
              TPDM_ERR_ARG, "tpdm_queue_begin: null argument");
   TPDM_CHECK(p->cfg_pairs, TPDM_ERR_STATE, "tpdm_queue_begin: the plan was created without cfg_pairs");
-  TPDM_CHECK(!p->st.open, TPDM_ERR_STATE, "tpdm_queue_begin: the plan has an open prompt stream (tpdm_stream_close first)");
+  TPDM_TRY(check_mode(p, in(Mode::kIdle) | in(Mode::kSample) | in(Mode::kQueue), "tpdm_queue_begin"));
   TPDM_CHECK(p->ctx->has_mmdit && p->ctx->has_tpm, TPDM_ERR_STATE, "tpdm_queue_begin: needs both MMDiT and TimePredictor weights");
   TPDM_CHECK(n_prompts >= p->B, TPDM_ERR_ARG, "tpdm_queue_begin: %d prompts for %d slots (use a plan with fewer slots)", n_prompts, p->B);
   TPDM_CHECK(order != nullptr || n_queued == n_prompts || n_queued <= 0, TPDM_ERR_ARG, "tpdm_queue_begin: n_queued needs an order table");
   TPDM_CHECK(n_queued <= n_prompts, TPDM_ERR_ARG, "tpdm_queue_begin: n_queued %d exceeds the %d prompts", n_queued, n_prompts);
   TPDM_CHECK(init_step >= 0 && init_step < p->max_steps && (init_step == 0) == (init_sigma == nullptr), TPDM_ERR_ARG,
              "tpdm_queue_begin: init_sigma and init_step (%d) go together, init_step < max_steps", init_step);
-  TPDM_CHECK((reinterpret_cast<uintptr_t>(queue_workspace) & 1023) == 0 && queue_workspace_bytes >= queue_bytes(p, n_prompts), TPDM_ERR_ARG,
-             "tpdm_queue_begin: queue workspace must be 1 KiB aligned and >= %zu bytes", queue_bytes(p, n_prompts));
+  const size_t need = tpdm_queue_workspace_bytes(p, n_prompts);
+  TPDM_CHECK((reinterpret_cast<uintptr_t>(queue_workspace) & 1023) == 0 && queue_workspace_bytes >= need, TPDM_ERR_ARG,
+             "tpdm_queue_begin: queue workspace must be 1 KiB aligned and >= %zu bytes", need);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const tpdm_ctx* ctx = p->ctx;
   const int B = p->B, D = ctx->D, T = p->T, J = ctx->cfg.joint_attention_dim, PD = ctx->cfg.pooled_projection_dim;
   const size_t nctx = static_cast<size_t>(T) * D;
   tpdm_plan::Queue& q = p->q;
-  if (q.graph) {
-    cudaGraphExecDestroy(q.graph);
-    q.graph = nullptr;
-  }
+  q = tpdm_plan::Queue{};
   Carver c(queue_workspace);
-  q.ctx0_all = c.take<float>(static_cast<size_t>(n_prompts) * 2 * nctx);
-  q.text_all = c.take<float>(static_cast<size_t>(n_prompts) * 2 * D);
-  q.sigma_cur = c.take<float>(2 * B);
-  q.sigma_next = q.sigma_cur + B;
-  q.slot_prompt = c.take<int>(5 * B + 8);
-  q.slot_step = q.slot_prompt + B;
-  q.slot_flush = q.slot_step + B;
-  q.slot_load = q.slot_flush + B;
-  q.slot_active = q.slot_load + B;
-  q.active = q.slot_active + B;
-  q.idle_flag = q.active + 1;
+  carve_queue(p, n_prompts, c);
   q.n_prompts = n_prompts;
   q.n_queued = n_queued > 0 ? n_queued : n_prompts;
   q.order = order;
@@ -804,11 +829,6 @@ int tpdm_queue_begin(tpdm_plan* p, int n_prompts, const float* latents_all, cons
   q.out_latents = out_latents;
   q.out_steps = out_steps;
   q.out_sigmas = out_sigmas;
-  q.predict = 1;
-  q.seed = 0;
-  q.ratios_all = nullptr;
-  q.rec_alphas = q.rec_betas = q.rec_logprobs = q.rec_tembs = nullptr;
-  q.rec_tpm = nullptr;
   p->guidance = guidance_scale;
   p->predict = 1;
   // sigma-independent text branch of every prompt, B prompts at a time through the plan's own buffers
@@ -828,14 +848,13 @@ int tpdm_queue_begin(tpdm_plan* p, int n_prompts, const float* latents_all, cons
   TPDM_CUDA_OK(cudaMemsetAsync(q.slot_step, 0, sizeof(int) * (4 * B + 8), s));
   TPDM_TRY(k_queue_advance(queue_args(p, 1), s));
   TPDM_TRY(queue_move(p, s));
-  q.begun = 1;
-  p->begun = 0;  // the per-batch sampler state is not valid while the queue owns the plan
+  p->mode = Mode::kQueue;
   return 0;
 }
 
 int tpdm_queue_step(tpdm_plan* p, void* stream) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_queue_step: null plan");
-  TPDM_CHECK(p->q.begun, TPDM_ERR_STATE, "tpdm_queue_step: call tpdm_queue_begin first");
+  TPDM_TRY(check_mode(p, in(Mode::kQueue) | in(Mode::kStream), "tpdm_queue_step"));
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const tpdm_ctx* ctx = p->ctx;
   const int B = p->B;
@@ -856,7 +875,7 @@ int tpdm_queue_step(tpdm_plan* p, void* stream) {
   TPDM_TRY(k_queue_schedule(queue_args(p, 0), s));
   TPDM_TRY(k_unpatchify(p->pout, B, 1, p->guidance, ctx->cfg.out_channels, p->Hl, p->Wl, nullptr, p->latents, p->q.sigma_cur,
                         p->q.sigma_next, 1, nullptr, s));
-  TPDM_TRY(p->st.open ? k_stream_advance(queue_args(p, 0), 0, s) : k_queue_advance(queue_args(p, 0), s));
+  TPDM_TRY(p->mode == Mode::kStream ? k_stream_advance(queue_args(p, 0), 0, s) : k_queue_advance(queue_args(p, 0), s));
   TPDM_TRY(queue_move(p, s));
   return 0;
 }
@@ -864,15 +883,11 @@ int tpdm_queue_step(tpdm_plan* p, void* stream) {
 int tpdm_queue_set_rollout(tpdm_plan* p, unsigned long long seed, const float* ratios_all, float* alphas, float* betas, float* logprobs,
                            float* tembs, void* tpm_inputs) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_queue_set_rollout: null plan");
-  TPDM_CHECK(p->q.begun, TPDM_ERR_STATE, "tpdm_queue_set_rollout: call tpdm_queue_begin first");
-  TPDM_CHECK(!p->st.open, TPDM_ERR_STATE, "tpdm_queue_set_rollout: a prompt stream runs predict mode only");
+  TPDM_TRY(check_mode(p, in(Mode::kQueue), "tpdm_queue_set_rollout"));  // a prompt stream runs predict mode only
   // the probe step of longest-first scheduling ran the Beta mode, so such a queue cannot start sampled trajectories
   TPDM_CHECK(p->q.init_step == 0, TPDM_ERR_STATE, "tpdm_queue_set_rollout: the queue began after %d probe steps (init_step > 0)", p->q.init_step);
   tpdm_plan::Queue& q = p->q;
-  if (q.graph) {  // the captured step holds the predict-mode arguments
-    cudaGraphExecDestroy(q.graph);
-    q.graph = nullptr;
-  }
+  q.graph.drop();  // the captured step holds the predict-mode arguments
   q.predict = 0;
   q.seed = seed;
   q.ratios_all = ratios_all;
@@ -886,34 +901,16 @@ int tpdm_queue_set_rollout(tpdm_plan* p, unsigned long long seed, const float* r
 
 int tpdm_queue_step_graph(tpdm_plan* p, void* stream) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_queue_step_graph: null plan");
-  TPDM_CHECK(p->q.begun, TPDM_ERR_STATE, "tpdm_queue_step_graph: call tpdm_queue_begin first");
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (p->q.graph == nullptr) {
-    // a queue step has no host-side argument that changes between steps (a rollout's seed is fixed for the whole drain):
-    // capture it once, replay it every step
-    const long long before = launches_so_far();
-    cudaGraph_t g = nullptr;
-    TPDM_CUDA_OK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-    const int st = tpdm_queue_step(p, s);
-    const cudaError_t e = cudaStreamEndCapture(s, &g);
-    if (st != 0) {
-      if (g) cudaGraphDestroy(g);
-      return st;
-    }
-    TPDM_CHECK(e == cudaSuccess && g != nullptr, TPDM_ERR_CUDA, "tpdm_queue_step_graph: stream capture failed: %s", cudaGetErrorString(e));
-    const cudaError_t ei = cudaGraphInstantiate(&p->q.graph, g, 0);
-    cudaGraphDestroy(g);
-    TPDM_CHECK(ei == cudaSuccess, TPDM_ERR_CUDA, "tpdm_queue_step_graph: cudaGraphInstantiate failed: %s", cudaGetErrorString(ei));
-    p->q.graph_launches = launches_so_far() - before;
-    count_launches(-p->q.graph_launches);  // the capture itself launched nothing
-  }
-  TPDM_CUDA_OK(cudaGraphLaunch(p->q.graph, s));
-  count_launches(p->q.graph_launches);
-  return 0;
+  TPDM_TRY(check_mode(p, in(Mode::kQueue) | in(Mode::kStream), "tpdm_queue_step_graph"));
+  // a queue step has no host-side argument that changes between steps (a rollout's seed is fixed for the whole drain):
+  // capture it once, replay it every step
+  return replay_or_capture(p->q.graph, static_cast<cudaStream_t>(stream), "tpdm_queue_step_graph",
+                           [&](cudaStream_t s) { return tpdm_queue_step(p, s); });
 }
 
 int tpdm_queue_status(tpdm_plan* p, const int** active_slots, const int** slot_prompts) {
-  TPDM_CHECK(p && p->q.begun, TPDM_ERR_STATE, "tpdm_queue_status: call tpdm_queue_begin first");
+  TPDM_CHECK(p, TPDM_ERR_STATE, "tpdm_queue_status: call tpdm_queue_begin first");
+  TPDM_TRY(check_mode(p, in(Mode::kQueue) | in(Mode::kStream), "tpdm_queue_status"));
   if (active_slots) *active_slots = p->q.active;
   if (slot_prompts) *slot_prompts = p->q.slot_prompt;
   return 0;
@@ -979,11 +976,7 @@ size_t tpdm_stream_workspace_bytes(const tpdm_plan* p, int capacity) {
   if (!p || capacity <= 0) return 0;
   tpdm_plan probe;
   probe.ctx = p->ctx;
-  probe.B = p->B;
-  probe.T = p->T;
-  probe.Hl = p->Hl;
-  probe.Wl = p->Wl;
-  probe.max_steps = p->max_steps;
+  set_shape(&probe, p->B, p->cfg_pairs, p->Hl, p->Wl, p->T, p->max_steps);
   Carver c(nullptr);
   carve_stream(&probe, capacity, c);
   return c.off + 1024;
@@ -993,8 +986,7 @@ int tpdm_stream_open(tpdm_plan* p, int capacity, float guidance_scale, void* wor
   TPDM_CHECK(p && workspace, TPDM_ERR_ARG, "tpdm_stream_open: null argument");
   TPDM_CHECK(p->cfg_pairs, TPDM_ERR_STATE, "tpdm_stream_open: the plan was created without cfg_pairs");
   TPDM_CHECK(p->ctx->has_mmdit && p->ctx->has_tpm, TPDM_ERR_STATE, "tpdm_stream_open: needs both MMDiT and TimePredictor weights");
-  TPDM_CHECK(!p->st.open, TPDM_ERR_STATE, "tpdm_stream_open: the plan already has an open stream");
-  TPDM_CHECK(!p->q.begun, TPDM_ERR_STATE, "tpdm_stream_open: a prompt queue has begun on this plan (open the stream on a fresh plan)");
+  TPDM_TRY(check_mode(p, in(Mode::kIdle) | in(Mode::kSample), "tpdm_stream_open"));
   TPDM_CHECK(capacity > 0, TPDM_ERR_ARG, "tpdm_stream_open: capacity %d must be positive", capacity);
   const size_t need = tpdm_stream_workspace_bytes(p, capacity);
   TPDM_CHECK((reinterpret_cast<uintptr_t>(workspace) & 1023) == 0 && workspace_bytes >= need, TPDM_ERR_ARG,
@@ -1004,10 +996,7 @@ int tpdm_stream_open(tpdm_plan* p, int capacity, float guidance_scale, void* wor
   const int B = p->B, T = p->T, D = ctx->D, J = ctx->cfg.joint_attention_dim;
   tpdm_plan::Queue& q = p->q;
   tpdm_plan::Stream& st = p->st;
-  if (q.graph) {
-    cudaGraphExecDestroy(q.graph);
-    q.graph = nullptr;
-  }
+  q = tpdm_plan::Queue{};
   Carver c(workspace);
   carve_stream(p, capacity, c);
   TPDM_TRY(gemm_op_init(&st.ctx_embed, st.enc, J, static_cast<long long>(T) * J, T, 2 * B, J, ctx->w.ctx_w, D, EPI_BIAS_F32, st.ctx0,
@@ -1015,23 +1004,12 @@ int tpdm_stream_open(tpdm_plan* p, int capacity, float guidance_scale, void* wor
   st.capacity = capacity;
   q.n_prompts = q.n_queued = capacity;
   q.noise_all = st.noise;
-  q.ticket = nullptr;
-  q.order = nullptr;
-  q.init_sigma = nullptr;
-  q.init_step = 0;
-  q.predict = 1;
-  q.seed = 0;
-  q.ratios_all = nullptr;
-  q.rec_alphas = q.rec_betas = q.rec_logprobs = q.rec_tembs = nullptr;
-  q.rec_tpm = nullptr;
   p->guidance = guidance_scale;
   p->predict = 1;
   TPDM_CUDA_OK(cudaMemsetAsync(q.sigma_cur, 0, sizeof(float) * 2 * B, s));
   TPDM_CUDA_OK(cudaMemsetAsync(q.slot_prompt, 0xff, sizeof(int) * B, s));  // -1: every slot is idle
   TPDM_CUDA_OK(cudaMemsetAsync(q.slot_step, 0, sizeof(int) * (4 * B + kStreamCounters + 2), s));
-  st.open = 1;
-  q.begun = 1;
-  p->begun = 0;
+  p->mode = Mode::kStream;
   TPDM_TRY(k_stream_advance(queue_args(p, 0), 1, s));   // nothing submitted: every slot stays idle, the skip flag is raised
   return 0;
 }
@@ -1039,7 +1017,7 @@ int tpdm_stream_open(tpdm_plan* p, int capacity, float guidance_scale, void* wor
 int tpdm_stream_submit(tpdm_plan* p, int n, const int* entry_ids, const float* latents, const float* neg_embeds, const float* pos_embeds,
                        const float* neg_pooled, const float* pos_pooled, void* stream) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_stream_submit: null plan");
-  TPDM_CHECK(p->st.open, TPDM_ERR_STATE, "tpdm_stream_submit: the plan has no open stream");
+  TPDM_TRY(check_mode(p, in(Mode::kStream), "tpdm_stream_submit"));
   TPDM_CHECK(n > 0 && entry_ids && latents && neg_embeds && pos_embeds && neg_pooled && pos_pooled, TPDM_ERR_ARG,
              "tpdm_stream_submit: null argument or n <= 0");
   tpdm_plan::Stream& st = p->st;
@@ -1082,7 +1060,7 @@ int tpdm_stream_submit(tpdm_plan* p, int n, const int* entry_ids, const float* l
 int tpdm_stream_status(tpdm_plan* p, const int** counters, const int** done_log, const float** out_latents, const int** out_steps,
                        const float** out_sigmas) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_stream_status: null plan");
-  TPDM_CHECK(p->st.open, TPDM_ERR_STATE, "tpdm_stream_status: the plan has no open stream");
+  TPDM_TRY(check_mode(p, in(Mode::kStream), "tpdm_stream_status"));
   if (counters) *counters = p->st.counters;
   if (done_log) *done_log = p->st.done_log;
   if (out_latents) *out_latents = p->q.out_latents;
@@ -1093,13 +1071,10 @@ int tpdm_stream_status(tpdm_plan* p, const int** counters, const int** done_log,
 
 int tpdm_stream_close(tpdm_plan* p) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_stream_close: null plan");
-  TPDM_CHECK(p->st.open, TPDM_ERR_STATE, "tpdm_stream_close: the plan has no open stream");
-  if (p->q.graph) {
-    cudaGraphExecDestroy(p->q.graph);
-    p->q.graph = nullptr;
-  }
+  TPDM_TRY(check_mode(p, in(Mode::kStream), "tpdm_stream_close"));
   p->st = tpdm_plan::Stream{};
   p->q = tpdm_plan::Queue{};
+  p->mode = Mode::kIdle;
   return 0;
 }
 

@@ -4,6 +4,7 @@ operation of the path runs inside the C-ABI library (no eager fallback exists).
 """
 from __future__ import annotations
 
+import collections
 import ctypes as C
 import os
 import weakref
@@ -203,6 +204,50 @@ def pack_time_predictor(pw: PackedWeights, sd: Dict[str, torch.Tensor], device) 
     pw._set(s, "tpm_fc2_b", _f32(g("fc2.bias")))
 
 
+class _FlagReadback:
+    """Device int32 flags looked at one step late, so that the device never waits for the host: ``push`` copies them into the
+    next row of a pinned ring behind the step just enqueued (one copy, one event record), and a row is looked at once its
+    copy has completed.  ``last`` is the newest row looked at (zeros before the first)."""
+
+    def __init__(self, width: int, ring: int = 64):
+        self._host = torch.zeros(ring, width, dtype=torch.int32).pin_memory()
+        self._events = [torch.cuda.Event() for _ in range(ring)]
+        self._pending = collections.deque()      # rows pushed and not looked at, oldest first
+        self._pushes = 0
+        self.last = [0] * width
+
+    def push(self, src: torch.Tensor) -> None:
+        row = self._pushes % len(self._events)
+        self._pushes += 1
+        self._host[row].copy_(src, non_blocking=True)
+        self._events[row].record()
+        self._pending.append(row)
+
+    def _take(self) -> list:
+        row = self._pending.popleft()
+        self._events[row].synchronize()
+        self.last = self._host[row].tolist()
+        return self.last
+
+    def settle(self) -> Optional[list]:
+        """Waits for every push but the newest; returns the newest row that settled (None: none did)."""
+        seen = None
+        while len(self._pending) > 1:
+            seen = self._take()
+        return seen
+
+    def poll(self) -> Optional[list]:
+        """Looks at the completed rows without blocking; returns the newest (None: none completed since the last look)."""
+        seen = None
+        while self._pending and self._events[self._pending[0]].query():
+            seen = self._take()
+        return seen
+
+    def wait_all(self) -> None:
+        while self._pending:
+            self._take()
+
+
 class Plan:
     """A shape-bound workspace with typed torch views over the library's state buffers."""
 
@@ -212,9 +257,7 @@ class Plan:
         nbytes = lib.tpdm_plan_workspace_bytes(engine.ctx, batch, int(cfg_pairs), latent, latent, n_text, max_steps)
         if nbytes == 0:
             L.check(L.TPDM_ERR_SHAPE if lib.tpdm_last_error() else L.TPDM_ERR_ARG)
-        self.workspace = torch.empty(nbytes + 1024, dtype=torch.uint8, device=engine.device)
-        base = (self.workspace.data_ptr() + 1023) // 1024 * 1024
-        self._base_off = base - self.workspace.data_ptr()
+        self.workspace, base = L.aligned_workspace(nbytes, engine.device)
         handle = L.vp()
         L.check(lib.tpdm_plan_create(engine.ctx, batch, int(cfg_pairs), latent, latent, n_text, max_steps, base, nbytes, C.byref(handle)))
         self.handle = handle
@@ -225,27 +268,20 @@ class Plan:
             cfg, D, g = engine.cfg, engine.D, latent // 2
             Cc = cfg["in_channels"]
             f32, i32 = torch.float32, torch.int32
+            view = lambda ptr, dtype, shape: L.view_at(self.workspace, ptr, dtype, shape)
             self.state = dict(
-                latents=self._view(st.latents, f32, (batch, Cc, latent, latent)),
-                velocity=self._view(st.velocity, f32, (batch, Cc, latent, latent)),
-                sigma_hist=self._view(st.sigma_hist, f32, (batch, max_steps + 1)),
-                alphas=self._view(st.alphas, f32, (batch, max_steps)),
-                betas=self._view(st.betas, f32, (batch, max_steps)),
-                logprobs=self._view(st.logprobs, f32, (batch, max_steps)),
-                prob_masks=self._view(st.prob_masks, i32, (batch, max_steps)),
-                all_done=self._view(st.all_done, i32, (max_steps,)),
-                tembs=self._view(st.tembs, f32, (max_steps, batch, D)),
-                tpm_input=self._view(st.tpm_input, torch.bfloat16, (batch, g, g, 2 * D)),
-                history_latents=self._view(st.history_latents, f32, (max_steps, batch, Cc, latent, latent)),
+                latents=view(st.latents, f32, (batch, Cc, latent, latent)),
+                velocity=view(st.velocity, f32, (batch, Cc, latent, latent)),
+                sigma_hist=view(st.sigma_hist, f32, (batch, max_steps + 1)),
+                alphas=view(st.alphas, f32, (batch, max_steps)),
+                betas=view(st.betas, f32, (batch, max_steps)),
+                logprobs=view(st.logprobs, f32, (batch, max_steps)),
+                prob_masks=view(st.prob_masks, i32, (batch, max_steps)),
+                all_done=view(st.all_done, i32, (max_steps,)),
+                tembs=view(st.tembs, f32, (max_steps, batch, D)),
+                tpm_input=view(st.tpm_input, torch.bfloat16, (batch, g, g, 2 * D)),
+                history_latents=view(st.history_latents, f32, (max_steps, batch, Cc, latent, latent)),
             )
-
-    def _view(self, ptr: int, dtype: torch.dtype, shape) -> torch.Tensor:
-        off = ptr - self.workspace.data_ptr()
-        n = 1
-        for s in shape:
-            n *= s
-        nb = n * torch.empty((), dtype=dtype).element_size()
-        return self.workspace[off: off + nb].view(dtype).view(shape)
 
     def __del__(self):
         try:
@@ -299,6 +335,7 @@ class Engine:
                 L.check(lib.tpdm_set_fp8_weights(self.ctx, self.weights.fp8_blocks))
         self.plans: Dict[Tuple, Plan] = {}
         self._streams = weakref.WeakSet()    # open PromptStreams: they read the packed weights from their own CUDA stream
+        self._sample_flags, self._queue_flags = _FlagReadback(1), _FlagReadback(1)    # all_done[step] / active slots
         self.min_sigma = min_sigma
 
     def __del__(self):
@@ -410,12 +447,7 @@ class Engine:
             rec = torch.empty(B, max_inference_steps, g, g, 2 * self.D, device=dev, dtype=torch.bfloat16)
         if record_velocity:
             vel = torch.empty(B, max_inference_steps, Cc, h, w, device=dev, dtype=f32)
-        done_host = getattr(self, "_done_host", None)
-        if done_host is None or done_host.numel() < max_inference_steps:
-            done_host = self._done_host = torch.zeros(max(64, max_inference_steps), dtype=torch.int32).pin_memory()
-        events = getattr(self, "_step_events", None)
-        if events is None:
-            events = self._step_events = [torch.cuda.Event(), torch.cuda.Event()]
+        flags = self._sample_flags
         executed = max_inference_steps
         step_fn = lib.tpdm_sample_step_graph if use_graph else lib.tpdm_sample_step
         side = None
@@ -434,15 +466,13 @@ class Engine:
                     rec[:, step].copy_(st["tpm_input"])
                 if vel is not None:
                     vel[:, step].copy_(st["velocity"])
-                done_host[step: step + 1].copy_(st["all_done"][step: step + 1], non_blocking=True)
-                events[step & 1].record()
-                if step >= 1:       # the flag of the previous step: the device never waits for the host
-                    events[(step - 1) & 1].synchronize()
-                    if int(done_host[step - 1]) != 0:
-                        executed = step  # steps [0, step) are real; step `step` was skipped on the device
-                        break
+                flags.push(st["all_done"][step: step + 1])
+                done = flags.settle()      # the flag of the previous step: the device never waits for the host
+                if step >= 1 and done[0] != 0:
+                    executed = step  # steps [0, step) are real; step `step` was skipped on the device
+                    break
             else:
-                events[(max_inference_steps - 1) & 1].synchronize()
+                flags.wait_all()
         if side is not None:
             torch.cuda.current_stream(dev).wait_stream(side)
             for t in (lat, pe, ne, pp, npp, rt, rec, vel):
@@ -564,9 +594,8 @@ class Engine:
                 return dict(latents=out_lat, steps=out_steps, sigmas=out_sig, device_steps=1)
         plan = self.plan(slots, True, h, prompt_embeds.shape[1], max_inference_steps)
         nbytes = lib.tpdm_queue_workspace_bytes(plan.handle, P)
-        ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
-        base = (ws.data_ptr() + 1023) // 1024 * 1024
-        active_host = torch.ones(64, dtype=torch.int32).pin_memory()
+        ws, base = L.aligned_workspace(nbytes, dev)
+        flags = self._queue_flags
         # the step is replayed from a CUDA graph (captured on the first step), which needs a non-default stream
         qs = getattr(self, "_queue_stream", None)
         if qs is None:
@@ -584,30 +613,24 @@ class Engine:
                                                    L.ptr(rec["logprobs_raw"]), L.ptr(rec.get("tembs")), L.ptr(rec.get("tpm_inputs_nhwc"))))
             act_p, slot_p = L.vp(), L.vp()
             L.check(lib.tpdm_queue_status(plan.handle, C.byref(act_p), C.byref(slot_p)))
-            off = act_p.value - ws.data_ptr()          # the counters live in the queue workspace
-            active = ws[off: off + 4].view(torch.int32)
-            ring = active_host.numel()
-            events = [None] * ring
+            active = L.view_at(ws, act_p.value, torch.int32, (1,))     # the counters live in the queue workspace
             limit = (P + slots - 1) // slots * max_inference_steps + 2 * max_inference_steps   # upper bound on device steps
             steps_run = 0
             drained = False
             for it in range(limit):
                 L.check(step_fn(plan.handle, stream))
                 steps_run += 1
-                active_host[it % ring: it % ring + 1].copy_(active, non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record()
-                events[it % ring] = ev
-                if it >= 1:                      # look at the flag one step late: the device never waits for the host
-                    events[(it - 1) % ring].synchronize()
-                    if int(active_host[(it - 1) % ring]) == 0:
-                        drained = True
-                        break
+                flags.push(active)
+                prev = flags.settle()      # the count after the previous step: the device never waits for the host
+                if it >= 1 and prev[0] == 0:
+                    drained = True
+                    break
             if not drained:
                 torch.cuda.current_stream().synchronize()
                 if int(active.item()) != 0:
                     raise RuntimeError("sample_queue: the queue did not drain within the step bound")
             torch.cuda.current_stream().synchronize()
+            flags.wait_all()
         torch.cuda.current_stream(dev).wait_stream(qs)
         self._queue_keepalive = (ws, lat, pe, ne, pp, npp, ticket, order, init_sigma, rt)
         return dict(latents=out_lat, steps=out_steps, sigmas=out_sig, device_steps=steps_run + (1 if init_step else 0), **rec)
@@ -630,8 +653,6 @@ class PromptStream:
     engine's packed weights: a TimePredictor refresh (``Engine.refresh_time_predictor``, which ``get_engine`` makes after an
     optimizer step) raises RuntimeError while requests are in flight, and is ordered against the stream's steps otherwise."""
 
-    _READBACK_RING = 64
-
     def __init__(self, engine: Engine, slots: int, capacity: int, max_steps: int, guidance_scale: float, use_graph: bool, latent: int,
                  n_text: int, prepare_latents=None):
         if slots < 1 or capacity < 1:
@@ -647,8 +668,7 @@ class PromptStream:
             self._plan = Plan(engine, slots, True, latent, n_text, max_steps)    # private: never handed out by Engine.plan
             self._cs = torch.cuda.Stream(device=dev)
             nbytes = lib.tpdm_stream_workspace_bytes(self._plan.handle, capacity)
-            self._ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
-            base = (self._ws.data_ptr() + 1023) // 1024 * 1024
+            self._ws, base = L.aligned_workspace(nbytes, dev)
             self._cs.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(self._cs):
                 L.check(lib.tpdm_stream_open(self._plan.handle, capacity, float(guidance_scale), base, nbytes, L.stream_ptr()))
@@ -657,27 +677,17 @@ class PromptStream:
             ptrs = [L.vp() for _ in range(5)]
             L.check(lib.tpdm_stream_status(self._plan.handle, *[C.byref(p) for p in ptrs]))
         Cc = engine.cfg["in_channels"]
-        view = lambda p, dtype, shape: self._view(p.value, dtype, shape)
+        view = lambda p, dtype, shape: L.view_at(self._ws, p.value, dtype, shape)
         self._counters = view(ptrs[0], torch.int32, (6,))            # submitted, claimed, completed, executed, active, skip flag
         self._log = view(ptrs[1], torch.int32, (capacity,))
         self._out_lat = view(ptrs[2], torch.float32, (capacity, Cc, latent, latent))
         self._out_steps = view(ptrs[3], torch.int32, (capacity,))
         self._out_sig = view(ptrs[4], torch.float32, (capacity, max_steps + 1))
-        self._host = torch.zeros(self._READBACK_RING, 6, dtype=torch.int32).pin_memory()
-        self._pending = []                       # (event, ring row) of readbacks not yet looked at, oldest first
-        self._reads = 0
-        self._last = [0] * 6                     # the newest readback looked at
+        self._flags = _FlagReadback(6)
         self._free = list(range(capacity - 1, -1, -1))
         self._entry_req = {}                     # entry -> request id
         self._next_id = self._submitted = self._harvested = 0
         self._freed = []                         # events after the copies out of entries freed since the last submit
-
-    def _view(self, ptr: int, dtype: torch.dtype, shape) -> torch.Tensor:
-        off = ptr - self._ws.data_ptr()
-        n = 1
-        for s in shape:
-            n *= s
-        return self._ws[off: off + n * torch.empty((), dtype=dtype).element_size()].view(dtype).view(shape)
 
     def _check_open(self):
         if not self._open:
@@ -727,20 +737,10 @@ class PromptStream:
         return rids
 
     # ---- steps -------------------------------------------------------------------------------------------------
-    def _consume(self, block: bool):
-        """Look at the readbacks in order: all completed ones, and with ``block`` the older ones than the newest (one step late)."""
-        while self._pending:
-            ev, row = self._pending[0]
-            if not ev.query():
-                if not (block and len(self._pending) > 1):
-                    break
-                ev.synchronize()
-            self._last = self._host[row].tolist()
-            self._pending.pop(0)
-
     def _idle(self) -> bool:
         # no slot held a prompt after the newest step looked at, and nothing was submitted since
-        return self._last[4] == 0 and self._last[0] == self._submitted
+        last = self._flags.last
+        return last[4] == 0 and last[0] == self._submitted
 
     def step(self, n: int = 1) -> None:
         """Enqueue up to n denoising steps.  Stops (launching nothing) once no slot is active and nothing is pending."""
@@ -749,33 +749,27 @@ class PromptStream:
         with torch.cuda.device(dev), torch.cuda.stream(self._cs):
             stream = L.stream_ptr()
             for _ in range(n):
-                self._consume(block=False)
+                self._flags.poll()
                 if self._idle():
                     break
                 L.check(self._step_fn(self._plan.handle, stream))
-                row = self._reads % self._READBACK_RING
-                self._reads += 1
-                self._host[row].copy_(self._counters, non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record()
-                self._pending.append((ev, row))
-                self._consume(block=True)      # the flags of the previous step: the device never waits for the host
+                self._flags.push(self._counters)
+                self._flags.settle()           # the flags of the previous step: the device never waits for the host
 
     @property
     def device_steps(self) -> int:
         """Denoising steps the device executed (steps skipped on an idle stream are not counted)."""
         self._check_open()
-        self._cs.synchronize()
-        self._consume(block=False)
-        return int(self._last[3])
+        self._flags.wait_all()
+        return int(self._flags.last[3])
 
     # ---- completions -------------------------------------------------------------------------------------------
     def results(self) -> dict:
         """``{request id: dict(latents (C, h, w), steps, sigmas (steps,))}`` of the requests finished since the last call, as far as
         the host has seen (one step late); their entries are free again."""
         self._check_open()
-        self._consume(block=False)
-        done = self._last[2]
+        self._flags.poll()
+        done = self._flags.last[2]
         if done == self._harvested:
             return {}
         dev = self.engine.device
@@ -808,8 +802,7 @@ class PromptStream:
                 return out
             self.step()
             if self._idle():
-                self._cs.synchronize()
-                self._consume(block=False)
+                self._flags.wait_all()
         out.update(self.results())
         if self._harvested != self._submitted:
             raise RuntimeError("the prompt stream did not drain within the step bound")
@@ -822,7 +815,6 @@ class PromptStream:
         L.check(L.load().tpdm_stream_close(self._plan.handle))
         self._open = False
         self.engine._streams.discard(self)
-        self._pending.clear()
 
     def __enter__(self):
         return self

@@ -66,8 +66,7 @@ class TimePredictorTrainer:
         self.load_from_module()
         with torch.cuda.device(dev):
             nbytes = lib.tpdm_tpm_trainer_workspace_bytes(self.D, self.C1, grid, max_samples)
-            self.workspace = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
-            base = (self.workspace.data_ptr() + 1023) // 1024 * 1024
+            self.workspace, base = L.aligned_workspace(nbytes, dev)
             h = L.vp()
             L.check(lib.tpdm_tpm_trainer_create(self.D, self.C1, grid, max_samples, float(time_predictor.epsilon), base, nbytes, C.byref(h)))
             self.handle = h

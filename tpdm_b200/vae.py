@@ -203,8 +203,8 @@ class AutoencoderKL(nn.Module):
         nbytes = lib.tpdm_vae_workspace_bytes(self._ctx, h, w)
         if self._workspace is None or self._workspace.numel() < nbytes + 1024:
             self._workspace = None
-            self._workspace = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
-        base = (self._workspace.data_ptr() + 1023) // 1024 * 1024
+            self._workspace, self._workspace_base = L.aligned_workspace(nbytes, dev)
+        base = self._workspace_base
         H, W = h * self.upscale, w * self.upscale
         image = torch.empty(B, self.config.out_channels, H, W, device=dev) if want_image else None
         rgb = torch.empty(B, H, W, self.config.out_channels, device=dev, dtype=torch.uint8) if want_rgb else None
