@@ -315,10 +315,15 @@ int tpdm_queue_status(tpdm_plan* plan, const int** active_slots, const int** slo
  * handed to tpdm_stream_submit, and free again once its id was read from the completion log and its outputs were copied.
  * Counters (device int[4]): submitted, claimed, completed, executed steps.  Every stream call and every step is enqueued on
  * ONE stream, so ordering is by stream order; nothing synchronises the host.
- * Steps are tpdm_queue_step / tpdm_queue_step_graph on the plan (one captured graph: the ring, counters and staging never move).
+ * Steps are tpdm_queue_step / tpdm_queue_step_graph on the plan (one captured graph: the ring, counters, staging and request
+ * options never move, so requests with different options never force a recapture).
  * A slot without a prompt -- its trajectory just ended, or it was idle -- takes the next submitted ticket in slot order (no
- * atomics, deterministic); a step of a stream with no active slot is skipped on the device.  Each request follows exactly the
- * trajectory tpdm_sample_* gives it with batch 1 and predict = 1.
+ * atomics, deterministic); a step of a stream with no active slot is skipped on the device.
+ * Each entry also carries its request's options (tpdm_request_options: guidance scale, step cap, predict, seed); a slot that
+ * claims the entry runs its CFG combines with that guidance.  A request follows exactly the trajectory tpdm_sample_* gives it
+ * with batch 1, guidance_scale, max_steps = its cap and its predict; with predict = 0 the Beta draws are those of
+ * tpdm_sample_begin's `seed` = its seed (keyed by (seed, sample 0, step)).  Every executed step records the request's alpha,
+ * beta and raw log-prob (tpdm_stream_records).
  * A plan's buffers belong to one driver at a time: the lockstep sampler after tpdm_sample_begin, the closed queue after
  * tpdm_queue_begin, the open stream from tpdm_stream_open to tpdm_stream_close.  Each begin hands the plan to its driver, and a
  * call that needs another owner returns TPDM_ERR_STATE and enqueues nothing:
@@ -328,7 +333,7 @@ int tpdm_queue_status(tpdm_plan* plan, const int** active_slots, const int** slo
  *   tpdm_queue_step, _step_graph, tpdm_queue_status   need the closed queue or the stream: refused after a later
  *                                                 tpdm_sample_begin (its steps would run on the slots the sampler overwrote)
  *   tpdm_stream_open                              refused while a queue owns the plan or a stream is open
- *   tpdm_stream_submit, _status, _close           need the open stream; after close the plan is owned by nobody
+ *   tpdm_stream_submit[_options], _status, _records, _close   need the open stream; after close the plan is owned by nobody
  * ---------------------------------------------------------------------------------------------------------------- */
 size_t tpdm_stream_workspace_bytes(const tpdm_plan* plan, int capacity);
 /* workspace: 1 KiB aligned, >= tpdm_stream_workspace_bytes; borrowed until tpdm_stream_close.  Encodes the TMA maps of the
@@ -337,15 +342,32 @@ int tpdm_stream_open(tpdm_plan* plan, int capacity, float guidance_scale, void* 
 /* Admit n prompts into the free entries entry_ids[n] (host array, each in [0, capacity)): latents [n][C][h][w],
  * *_embeds [n][T][joint_attention_dim], *_pooled [n][pooled_projection_dim], device fp32, read by the enqueued work only.
  * Runs `batch` prompts per pass through the stream's own staging (text cast, context_embedder, pooled-text MLP), copies them
- * into their entries, publishes them, then lets idle slots claim: a prompt submitted to an idle stream runs in the next step. */
+ * into their entries, publishes them, then lets idle slots claim: a prompt submitted to an idle stream runs in the next step.
+ * Every prompt gets the stream's defaults: the guidance given to tpdm_stream_open, the plan's max_steps, predict = 1. */
 int tpdm_stream_submit(tpdm_plan* plan, int n, const int* entry_ids, const float* latents, const float* neg_embeds,
                        const float* pos_embeds, const float* neg_pooled, const float* pos_pooled, void* stream);
+/* Options of one request.  Invalid options (non-finite guidance, max_steps outside [1, plan max_steps], predict other than 0 / 1,
+ * reserved != 0) make tpdm_stream_submit_options return TPDM_ERR_ARG before anything is enqueued. */
+typedef struct tpdm_request_options {
+  float guidance_scale;   /* finite */
+  int32_t max_steps;      /* 1 .. plan max_steps */
+  int32_t predict;        /* 1 = Beta mode, 0 = Beta draw from `seed` */
+  int32_t reserved;       /* 0 */
+  uint64_t seed;
+} tpdm_request_options;   /* 24 bytes */
+/* tpdm_stream_submit with options[n] (host array; NULL = the stream's defaults for every prompt) */
+int tpdm_stream_submit_options(tpdm_plan* plan, int n, const int* entry_ids, const float* latents, const float* neg_embeds,
+                               const float* pos_embeds, const float* neg_pooled, const float* pos_pooled,
+                               const tpdm_request_options* options, void* stream);
 /* device pointers: counters int[4] followed by `active` (slots holding a prompt) and the skip flag; done_log int[capacity]
  * (entry ids in completion order, entry k of the log at k % capacity); per entry: out_latents [capacity][C][h][w],
  * out_steps [capacity], out_sigmas [capacity][max_steps + 1].  A completion counted after a step is readable once that
  * step has completed. */
 int tpdm_stream_status(tpdm_plan* plan, const int** counters, const int** done_log, const float** out_latents, const int** out_steps,
                        const float** out_sigmas);
+/* device pointers [capacity][max_steps]: per-entry alpha, beta, raw log-prob of each executed step (step k of an entry's
+ * request at [entry][k], k < its out_steps; later elements are not written).  Readable like the other outputs of an entry. */
+int tpdm_stream_records(tpdm_plan* plan, const float** alphas, const float** betas, const float** logprobs);
 /* Detach the stream (the caller synchronises first); the plan can then begin a queue or open a new stream. */
 int tpdm_stream_close(tpdm_plan* plan);
 

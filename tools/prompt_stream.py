@@ -9,13 +9,17 @@ prompts, (b) a stream (capacity 32) with all 32 submitted at open and drained.  
 steps are the steps the GPU executed; the closed queue enqueues one more, which the device skips, so (a) counts
 ``device_steps - 1``.
 
+``--mixed-options`` adds (m), alternating with (a) and (b): the stream of (b) with per-request options -- prompt i gets guidance
+(3.5, 5, 7, 9)[i % 4]; prompts with i % 4 == 1 are sampled (predict=False, seed 1000 + i) and those with i % 4 == 2 are capped at
+12 steps.  The work per device step is that of (b); only the number of steps differs.
+
 (c) Arrival trace: prompt i arrives at i x ``--interval-factor`` x (a)'s median time per image.  The stream server submits each
 prompt when it arrives and steps while anything is in flight; the FIFO server runs batch-1 ``forward(predict=True)`` per request
 in arrival order.  Latency is host time from arrival (= submit) to the result being on the host.
 
 Prints one JSON object and writes it to ``--out`` when given.
 
-    python tools/prompt_stream.py [--rounds 4] [--out FILE]
+    python tools/prompt_stream.py [--rounds 4] [--mixed-options] [--out FILE]
 """
 import argparse
 import json
@@ -59,6 +63,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--rounds", type=int, default=4)
     ap.add_argument("--interval-factor", type=float, default=1.2)
+    ap.add_argument("--mixed-options", action="store_true")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     dev = torch.device("cuda", 0)
@@ -93,11 +98,22 @@ def main():
             executed = s.device_steps
         return dict(executed=executed, steps=[res[r]["steps"] for r in rids], latents=torch.stack([res[r]["latents"] for r in rids]))
 
-    rows = {"a_closed_queue": [], "b_stream": []}
+    mixed_opts = dict(guidance_scale=[(3.5, 5.0, 7.0, 9.0)[i % 4] for i in range(PROMPTS)], predict=[i % 4 != 1 for i in range(PROMPTS)],
+                      seed=[1000 + i for i in range(PROMPTS)], max_inference_steps=[12 if i % 4 == 2 else MAX_STEPS for i in range(PROMPTS)])
+
+    def stream_mixed():
+        with model.open_prompt_stream(slots=SLOTS, capacity=PROMPTS, max_inference_steps=MAX_STEPS) as s:
+            rids = s.submit(*emb, latents=inp["latents"], **mixed_opts)
+            res = s.drain()
+            executed = s.device_steps
+        return dict(executed=executed, steps=[res[r]["steps"] for r in rids])
+
+    runs = [("a_closed_queue", closed), ("b_stream", stream)] + ([("m_stream_mixed_options", stream_mixed)] if args.mixed_options else [])
+    rows = {name: [] for name, _ in runs}
     agree = []
     for r in range(1 + args.rounds):
         outs = {}
-        for name, fn in (("a_closed_queue", closed), ("b_stream", stream)):
+        for name, fn in runs:
             ms, out = timed(fn)
             outs[name] = out
             if r >= 1:
@@ -110,6 +126,9 @@ def main():
                   ms_per_step_median=med([x["ms_per_step"] for x in v]), images_per_s_median=med([x["images_per_s"] for x in v]))
           for k, v in rows.items()}
     ab["b_over_a_ms_per_step"] = ab["b_stream"]["ms_per_step_median"] / ab["a_closed_queue"]["ms_per_step_median"]
+    if args.mixed_options:
+        ab["m_over_b_ms_per_step"] = ab["m_stream_mixed_options"]["ms_per_step_median"] / ab["b_stream"]["ms_per_step_median"]
+        ab["m_steps_per_prompt"] = outs["m_stream_mixed_options"]["steps"]
     ab["agreement"] = agree
     steps = outs["a_closed_queue"]["steps"]
     ab["steps_per_prompt"] = steps

@@ -80,6 +80,11 @@ class TpdmGemmOpDesc(C.Structure):
                 [(n, C.c_int32) for n in ("rows", "batch", "K", "N", "epi", "ldo", "gate_stride", "ksplit")])
 
 
+class TpdmRequestOptions(C.Structure):
+    _fields_ = [("guidance_scale", C.c_float), ("max_steps", C.c_int32), ("predict", C.c_int32), ("reserved", C.c_int32),
+                ("seed", C.c_uint64)]
+
+
 EXPORTS = {
     "tpdm_last_error": (C.c_char_p, []),
     "tpdm_abi_version": (C.c_int, []),
@@ -113,6 +118,8 @@ EXPORTS = {
     "tpdm_stream_workspace_bytes": (C.c_size_t, [vp, C.c_int]),
     "tpdm_stream_open": (C.c_int, [vp, C.c_int, C.c_float, vp, C.c_size_t, vp]),
     "tpdm_stream_submit": (C.c_int, [vp, C.c_int, C.POINTER(C.c_int), vp, vp, vp, vp, vp, vp]),
+    "tpdm_stream_submit_options": (C.c_int, [vp, C.c_int, C.POINTER(C.c_int), vp, vp, vp, vp, vp, C.POINTER(TpdmRequestOptions), vp]),
+    "tpdm_stream_records": (C.c_int, [vp] + [C.POINTER(vp)] * 3),
     "tpdm_stream_status": (C.c_int, [vp] + [C.POINTER(vp)] * 5),
     "tpdm_stream_close": (C.c_int, [vp]),
     "tpdm_vae_create": (C.c_int, [C.POINTER(TpdmVaeConfig), C.POINTER(vp)]),

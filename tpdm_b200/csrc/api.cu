@@ -5,6 +5,7 @@
 #include <string.h>
 
 #include <new>
+#include <cmath>
 #include <cstdlib>
 #include <vector>
 
@@ -92,7 +93,7 @@ struct tpdm_plan {
   // sampling state
   float *latents, *velocity, *sigma_hist, *alphas, *betas, *logprobs, *tembs, *history, *ratios;
   int *masks, *all_done;
-  float guidance = 7.0f;
+  float* row_guidance;  // [B] guidance scale of each batch row, read by every CFG combine
   int predict = 1, have_ratios = 0;
   Mode mode = Mode::kIdle;
   unsigned long long seed = 0;
@@ -119,8 +120,14 @@ struct tpdm_plan {
   // open prompt stream (tpdm_stream_*): the queue above runs over a ring of `capacity` entries, prompts are admitted between steps
   struct Stream {
     int capacity = 0;
+    float guidance = 7.0f;   // the options of a request submitted without its own
     int *order = nullptr, *counters = nullptr, *done_log = nullptr;
     float* noise = nullptr;
+    // request options [capacity] and per-step records [capacity][max_steps] of each entry
+    float* guidance_all = nullptr;
+    int *max_steps_all = nullptr, *predict_all = nullptr;
+    unsigned long long* seed_all = nullptr;
+    float *rec_alphas = nullptr, *rec_betas = nullptr, *rec_logprobs = nullptr;
     // admission staging, never read by a queue step: bf16 text [2*slots][T][J] (row 2k + half), its context_embedder output and
     // the pooled-text MLP of the same rows
     bf16* enc = nullptr;
@@ -128,9 +135,8 @@ struct tpdm_plan {
     GemmOp ctx_embed;
   } st;
   // tpdm_sample_step_graph: one captured graph per step index (the step index only moves pointers inside the plan's own buffers),
-  // valid for the guidance / predict / injected-ratio setting they were captured under
+  // valid for the predict / injected-ratio setting they were captured under (the guidance is read from row_guidance)
   std::vector<StepGraph> step_graph;
-  float graph_guidance = 0.f;
   int graph_predict = -1, graph_have_ratios = -1;
 };
 
@@ -240,6 +246,7 @@ void carve(tpdm_plan* p, Carver& c) {
   p->all_done = c.take<int>(steps);
   p->tembs = c.take<float>(steps * B * D);
   p->history = c.take<float>(steps * B * lat);
+  p->row_guidance = c.take<float>(B);
 }
 
 int check_shapes(const tpdm_ctx* ctx, int batch, int latent_h, int latent_w, int n_text, int max_steps) {
@@ -425,7 +432,7 @@ int run_mmdit(tpdm_plan* p, const float* latents, int Bl, int dup, const float* 
   }
   const float* mno = p->mod + (R - 2 * D);  // norm_out rows: (scale, shift)
   const int pairs = tpm_taps ? p->cfg_pairs : 0;
-  TPDM_TRY(k_norm_out(p->x_img, p->xn_img, mno + D, mno, R, pairs ? p->B : Bt, pairs, N, D, p->g, p->guidance,
+  TPDM_TRY(k_norm_out(p->x_img, p->xn_img, mno + D, mno, R, pairs ? p->B : Bt, pairs, N, D, p->g, p->row_guidance,
                       tpm_taps ? p->tpm_x : nullptr, h2_out, s));
   TPDM_TRY(gemm_launch(&p->proj_out, 1, s));
   return 0;
@@ -595,7 +602,7 @@ int tpdm_mmdit_forward(tpdm_plan* p, const float* latents, const float* timestep
   TPDM_TRY(set_prompts(p, enc, nullptr, pooled, nullptr, s));
   TPDM_TRY(run_mmdit(p, latents, p->Bt, 1, timestep, 1, 1.0f, 1, out_h1, out_h2, false, s));
   if (out_sample)
-    TPDM_TRY(k_unpatchify(p->pout, p->Bt, 0, 0.f, ctx->cfg.out_channels, p->Hl, p->Wl, out_sample, nullptr, nullptr, nullptr, 0, nullptr, s));
+    TPDM_TRY(k_unpatchify(p->pout, p->Bt, 0, p->row_guidance, ctx->cfg.out_channels, p->Hl, p->Wl, out_sample, nullptr, nullptr, nullptr, 0, nullptr, s));
   if (out_temb)
     TPDM_CUDA_OK(cudaMemcpyAsync(out_temb, p->temb, static_cast<size_t>(p->Bt) * ctx->D * sizeof(float), cudaMemcpyDeviceToDevice, s));
   return 0;
@@ -626,10 +633,10 @@ int tpdm_sample_begin(tpdm_plan* p, const float* latents, const float* neg_embed
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const tpdm_ctx* ctx = p->ctx;
   const size_t lat = static_cast<size_t>(p->B) * ctx->cfg.in_channels * p->Hl * p->Wl;
-  p->guidance = guidance_scale;
   p->predict = predict ? 1 : 0;
   p->have_ratios = ratios ? 1 : 0;
   p->seed = seed;
+  TPDM_TRY(k_fill_f32(p->row_guidance, p->B, guidance_scale, s));
   TPDM_CUDA_OK(cudaMemcpyAsync(p->latents, latents, lat * sizeof(float), cudaMemcpyDeviceToDevice, s));
   if (ratios)
     TPDM_CUDA_OK(cudaMemcpyAsync(p->ratios, ratios, static_cast<size_t>(p->B) * p->max_steps * sizeof(float), cudaMemcpyDeviceToDevice, s));
@@ -654,7 +661,7 @@ int tpdm_sample_step(tpdm_plan* p, int step, void* stream) {
   int st_mm = run_mmdit(p, p->latents, B, 2, p->sigma_hist + step, T1, 1000.0f, 2, nullptr, nullptr, true, s);
   set_skip_flag(nullptr);
   TPDM_TRY(st_mm);
-  TPDM_TRY(k_cfg_combine(p->temb, p->temb_cfg, p->tembs + static_cast<size_t>(step) * B * D, B, D, p->guidance, s));
+  TPDM_TRY(k_cfg_combine(p->temb, p->temb_cfg, p->tembs + static_cast<size_t>(step) * B * D, B, D, p->row_guidance, s));
   TPDM_TRY(run_tpm(p, B, p->temb_cfg, p->alpha_beta, s));
   ScheduleArgs a;
   a.alpha_beta = p->alpha_beta;
@@ -675,7 +682,7 @@ int tpdm_sample_step(tpdm_plan* p, int step, void* stream) {
   a.min_sigma = ctx->cfg.min_sigma;
   a.epsilon = ctx->cfg.epsilon;
   TPDM_TRY(k_schedule(a, s));
-  TPDM_TRY(k_unpatchify(p->pout, B, 1, p->guidance, ctx->cfg.out_channels, p->Hl, p->Wl, p->velocity, p->latents, p->sigma_hist + step,
+  TPDM_TRY(k_unpatchify(p->pout, B, 1, p->row_guidance, ctx->cfg.out_channels, p->Hl, p->Wl, p->velocity, p->latents, p->sigma_hist + step,
                         p->sigma_hist + step + 1, T1, p->history + static_cast<size_t>(step) * lat, s));
   return 0;
 }
@@ -687,9 +694,8 @@ int tpdm_sample_step_graph(tpdm_plan* p, int step, void* stream) {
   // The Philox seed of a sampled trajectory is a kernel argument that changes with every call, and per-launch profiling records
   // events on the stream: both take the plain path.  (predict / injected ratios never read the seed.)
   if ((!p->predict && !p->have_ratios) || profiling_active()) return tpdm_sample_step(p, step, stream);
-  if (p->graph_guidance != p->guidance || p->graph_predict != p->predict || p->graph_have_ratios != p->have_ratios) {
+  if (p->graph_predict != p->predict || p->graph_have_ratios != p->have_ratios) {
     p->step_graph.clear();
-    p->graph_guidance = p->guidance;
     p->graph_predict = p->predict;
     p->graph_have_ratios = p->have_ratios;
   }
@@ -767,11 +773,20 @@ QueueArgs queue_args(const tpdm_plan* p, int init) {
   a.rec_alphas = q.rec_alphas;
   a.rec_betas = q.rec_betas;
   a.rec_logprobs = q.rec_logprobs;
+  a.row_guidance = p->row_guidance;
   if (p->mode == Mode::kStream) {
-    a.order = p->st.order;
-    a.counters = p->st.counters;
-    a.done_log = p->st.done_log;
-    a.capacity = p->st.capacity;
+    const tpdm_plan::Stream& st = p->st;
+    a.order = st.order;
+    a.counters = st.counters;
+    a.done_log = st.done_log;
+    a.capacity = st.capacity;
+    a.entry_guidance = st.guidance_all;
+    a.entry_max_steps = st.max_steps_all;
+    a.entry_predict = st.predict_all;
+    a.entry_seed = st.seed_all;
+    a.rec_alphas = st.rec_alphas;
+    a.rec_betas = st.rec_betas;
+    a.rec_logprobs = st.rec_logprobs;
   }
   return a;
 }
@@ -829,8 +844,8 @@ int tpdm_queue_begin(tpdm_plan* p, int n_prompts, const float* latents_all, cons
   q.out_latents = out_latents;
   q.out_steps = out_steps;
   q.out_sigmas = out_sigmas;
-  p->guidance = guidance_scale;
   p->predict = 1;
+  TPDM_TRY(k_fill_f32(p->row_guidance, B, guidance_scale, s));
   // sigma-independent text branch of every prompt, B prompts at a time through the plan's own buffers
   // (context_embedder + pooled-text MLP: transformer_sd3.py:337 and half of :336), parked per prompt as (uncond, cond)
   for (int c0 = 0; c0 < n_prompts; c0 += B) {
@@ -864,7 +879,7 @@ int tpdm_queue_step(tpdm_plan* p, void* stream) {
   if (B > 1) set_batch_mask(p->q.slot_active, B);
   int st_mm = run_mmdit(p, p->latents, B, 2, p->q.sigma_cur, 1, 1000.0f, 2, nullptr, nullptr, true, s);
   set_skip_flag(nullptr);
-  if (st_mm == 0) st_mm = k_cfg_combine(p->temb, p->temb_cfg, nullptr, B, ctx->D, p->guidance, s);
+  if (st_mm == 0) st_mm = k_cfg_combine(p->temb, p->temb_cfg, nullptr, B, ctx->D, p->row_guidance, s);
   if (st_mm == 0) st_mm = run_tpm(p, B, p->temb_cfg, p->alpha_beta, s);
   set_batch_mask(nullptr, 1);
   TPDM_TRY(st_mm);
@@ -873,7 +888,7 @@ int tpdm_queue_step(tpdm_plan* p, void* stream) {
     TPDM_TRY(k_queue_record(q.slot_prompt, q.slot_step, B, p->max_steps, ctx->D, p->temb_cfg, q.rec_tembs, p->tpm_x, q.rec_tpm,
                             static_cast<long long>(p->g) * p->g * 2 * ctx->D, s));
   TPDM_TRY(k_queue_schedule(queue_args(p, 0), s));
-  TPDM_TRY(k_unpatchify(p->pout, B, 1, p->guidance, ctx->cfg.out_channels, p->Hl, p->Wl, nullptr, p->latents, p->q.sigma_cur,
+  TPDM_TRY(k_unpatchify(p->pout, B, 1, p->row_guidance, ctx->cfg.out_channels, p->Hl, p->Wl, nullptr, p->latents, p->q.sigma_cur,
                         p->q.sigma_next, 1, nullptr, s));
   TPDM_TRY(p->mode == Mode::kStream ? k_stream_advance(queue_args(p, 0), 0, s) : k_queue_advance(queue_args(p, 0), s));
   TPDM_TRY(queue_move(p, s));
@@ -883,7 +898,7 @@ int tpdm_queue_step(tpdm_plan* p, void* stream) {
 int tpdm_queue_set_rollout(tpdm_plan* p, unsigned long long seed, const float* ratios_all, float* alphas, float* betas, float* logprobs,
                            float* tembs, void* tpm_inputs) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_queue_set_rollout: null plan");
-  TPDM_TRY(check_mode(p, in(Mode::kQueue), "tpdm_queue_set_rollout"));  // a prompt stream runs predict mode only
+  TPDM_TRY(check_mode(p, in(Mode::kQueue), "tpdm_queue_set_rollout"));  // a prompt stream takes the mode per request
   // the probe step of longest-first scheduling ran the Beta mode, so such a queue cannot start sampled trajectories
   TPDM_CHECK(p->q.init_step == 0, TPDM_ERR_STATE, "tpdm_queue_set_rollout: the queue began after %d probe steps (init_step > 0)", p->q.init_step);
   tpdm_plan::Queue& q = p->q;
@@ -932,6 +947,13 @@ void carve_stream(tpdm_plan* p, int capacity, Carver& c) {
   q.out_steps = c.take<int>(cap);
   st.order = c.take<int>(cap);
   st.done_log = c.take<int>(cap);
+  st.guidance_all = c.take<float>(cap);
+  st.max_steps_all = c.take<int>(cap);
+  st.predict_all = c.take<int>(cap);
+  st.seed_all = c.take<unsigned long long>(cap);
+  st.rec_alphas = c.take<float>(cap * p->max_steps);
+  st.rec_betas = c.take<float>(cap * p->max_steps);
+  st.rec_logprobs = c.take<float>(cap * p->max_steps);
   q.sigma_cur = c.take<float>(2 * B);
   q.sigma_next = q.sigma_cur ? q.sigma_cur + B : nullptr;
   q.slot_prompt = c.take<int>(5 * B + kStreamCounters + 2);
@@ -1002,10 +1024,11 @@ int tpdm_stream_open(tpdm_plan* p, int capacity, float guidance_scale, void* wor
   TPDM_TRY(gemm_op_init(&st.ctx_embed, st.enc, J, static_cast<long long>(T) * J, T, 2 * B, J, ctx->w.ctx_w, D, EPI_BIAS_F32, st.ctx0,
                         static_cast<long long>(T) * D, D, ctx->w.ctx_b, nullptr, 0));
   st.capacity = capacity;
+  st.guidance = guidance_scale;
   q.n_prompts = q.n_queued = capacity;
   q.noise_all = st.noise;
-  p->guidance = guidance_scale;
   p->predict = 1;
+  TPDM_TRY(k_fill_f32(p->row_guidance, B, guidance_scale, s));   // idle rows; a slot takes its request's value when it claims one
   TPDM_CUDA_OK(cudaMemsetAsync(q.sigma_cur, 0, sizeof(float) * 2 * B, s));
   TPDM_CUDA_OK(cudaMemsetAsync(q.slot_prompt, 0xff, sizeof(int) * B, s));  // -1: every slot is idle
   TPDM_CUDA_OK(cudaMemsetAsync(q.slot_step, 0, sizeof(int) * (4 * B + kStreamCounters + 2), s));
@@ -1014,8 +1037,9 @@ int tpdm_stream_open(tpdm_plan* p, int capacity, float guidance_scale, void* wor
   return 0;
 }
 
-int tpdm_stream_submit(tpdm_plan* p, int n, const int* entry_ids, const float* latents, const float* neg_embeds, const float* pos_embeds,
-                       const float* neg_pooled, const float* pos_pooled, void* stream) {
+int tpdm_stream_submit_options(tpdm_plan* p, int n, const int* entry_ids, const float* latents, const float* neg_embeds,
+                               const float* pos_embeds, const float* neg_pooled, const float* pos_pooled, const tpdm_request_options* options,
+                               void* stream) {
   TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_stream_submit: null plan");
   TPDM_TRY(check_mode(p, in(Mode::kStream), "tpdm_stream_submit"));
   TPDM_CHECK(n > 0 && entry_ids && latents && neg_embeds && pos_embeds && neg_pooled && pos_pooled, TPDM_ERR_ARG,
@@ -1029,6 +1053,14 @@ int tpdm_stream_submit(tpdm_plan* p, int n, const int* entry_ids, const float* l
     TPDM_CHECK(!seen[id], TPDM_ERR_ARG, "tpdm_stream_submit: entry id %d given twice", id);
     seen[id] = 1;
   }
+  for (int k = 0; options && k < n; ++k) {
+    const tpdm_request_options& o = options[k];
+    TPDM_CHECK(std::isfinite(o.guidance_scale), TPDM_ERR_ARG, "tpdm_stream_submit: prompt %d: guidance_scale is not finite", k);
+    TPDM_CHECK(o.max_steps >= 1 && o.max_steps <= p->max_steps, TPDM_ERR_ARG, "tpdm_stream_submit: prompt %d: max_steps %d outside [1,%d]", k,
+               o.max_steps, p->max_steps);
+    TPDM_CHECK(o.predict == 0 || o.predict == 1, TPDM_ERR_ARG, "tpdm_stream_submit: prompt %d: predict %d is neither 0 nor 1", k, o.predict);
+    TPDM_CHECK(o.reserved == 0, TPDM_ERR_ARG, "tpdm_stream_submit: prompt %d: reserved is %d, must be 0", k, o.reserved);
+  }
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const tpdm_ctx* ctx = p->ctx;
   tpdm_plan::Queue& q = p->q;
@@ -1036,6 +1068,7 @@ int tpdm_stream_submit(tpdm_plan* p, int n, const int* entry_ids, const float* l
   const size_t nctx = static_cast<size_t>(p->T) * D, row = static_cast<size_t>(p->T) * ctx->cfg.joint_attention_dim;
   const size_t lat = static_cast<size_t>(ctx->cfg.in_channels) * p->Hl * p->Wl;
   const int pass = p->B < kStreamPublishMax ? p->B : kStreamPublishMax;
+  const tpdm_request_options defaults{st.guidance, p->max_steps, 1, 0, 0};
   for (int k0 = 0; k0 < n; k0 += pass) {
     const int m = n - k0 < pass ? n - k0 : pass;
     TPDM_TRY(stream_embed(p, m, neg_embeds + k0 * row, pos_embeds + k0 * row, neg_pooled + static_cast<size_t>(k0) * PD,
@@ -1043,18 +1076,37 @@ int tpdm_stream_submit(tpdm_plan* p, int n, const int* entry_ids, const float* l
     StreamEntries e{};
     for (int k = 0; k < m; ++k) {
       const size_t id = entry_ids[k0 + k];
+      const tpdm_request_options& o = options ? options[k0 + k] : defaults;
       e.id[k] = static_cast<int>(id);
+      e.guidance[k] = o.guidance_scale;
+      e.max_steps[k] = o.max_steps;
+      e.predict[k] = o.predict;
+      e.seed[k] = o.seed;
       TPDM_CUDA_OK(cudaMemcpyAsync(st.noise + id * lat, latents + (k0 + k) * lat, lat * sizeof(float), cudaMemcpyDeviceToDevice, s));
       TPDM_CUDA_OK(cudaMemcpyAsync(q.ctx0_all + id * 2 * nctx, st.ctx0 + static_cast<size_t>(k) * 2 * nctx, 2 * nctx * sizeof(float),
                                    cudaMemcpyDeviceToDevice, s));
       TPDM_CUDA_OK(cudaMemcpyAsync(q.text_all + id * 2 * D, st.text + static_cast<size_t>(k) * 2 * D, 2 * D * sizeof(float),
                                    cudaMemcpyDeviceToDevice, s));
     }
-    TPDM_TRY(k_stream_publish(st.order, st.counters, st.capacity, e, m, s));
+    TPDM_TRY(k_stream_publish(queue_args(p, 0), st.order, e, m, s));
   }
   // idle slots take the new tickets now, so the next step already computes them
   TPDM_TRY(k_stream_advance(queue_args(p, 0), 1, s));
   return queue_move(p, s);
+}
+
+int tpdm_stream_submit(tpdm_plan* p, int n, const int* entry_ids, const float* latents, const float* neg_embeds, const float* pos_embeds,
+                       const float* neg_pooled, const float* pos_pooled, void* stream) {
+  return tpdm_stream_submit_options(p, n, entry_ids, latents, neg_embeds, pos_embeds, neg_pooled, pos_pooled, nullptr, stream);
+}
+
+int tpdm_stream_records(tpdm_plan* p, const float** alphas, const float** betas, const float** logprobs) {
+  TPDM_CHECK(p, TPDM_ERR_ARG, "tpdm_stream_records: null plan");
+  TPDM_TRY(check_mode(p, in(Mode::kStream), "tpdm_stream_records"));
+  if (alphas) *alphas = p->st.rec_alphas;
+  if (betas) *betas = p->st.rec_betas;
+  if (logprobs) *logprobs = p->st.rec_logprobs;
+  return 0;
 }
 
 int tpdm_stream_status(tpdm_plan* p, const int** counters, const int** done_log, const float** out_latents, const int** out_steps,

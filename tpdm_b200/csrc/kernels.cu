@@ -412,8 +412,9 @@ __global__ void __launch_bounds__(256) ln_modulate_kernel(const __grid_constant_
 // the token->pixel scramble of reshape_hidden_states_to_2d (:551).
 __global__ void __launch_bounds__(256) norm_out_kernel(const float* __restrict__ x, bf16* __restrict__ xn,
                                                        const float* __restrict__ shift, const float* __restrict__ scale,
-                                                       int mod_stride, int B, int cfg_pairs, int N, int D, int g, float guidance,
-                                                       bf16* __restrict__ tpm_x, float* __restrict__ h2_out) {
+                                                       int mod_stride, int B, int cfg_pairs, int N, int D, int g,
+                                                       const float* __restrict__ guidance, bf16* __restrict__ tpm_x,
+                                                       float* __restrict__ h2_out) {
   const int lane = threadIdx.x & 31;
   const long long r = static_cast<long long>(blockIdx.x) * 8 + (threadIdx.x >> 5);
   if (r >= static_cast<long long>(B) * N) return;
@@ -445,8 +446,9 @@ __global__ void __launch_bounds__(256) norm_out_kernel(const float* __restrict__
     }
     if (tpm_x) {
       float c4[4];
+      const float gs = cfg_pairs ? guidance[bl] : 0.f;
 #pragma unroll
-      for (int e = 0; e < 4; ++e) c4[e] = cfg_pairs ? y[0][e] + guidance * (y[1][e] - y[0][e]) : y[0][e];
+      for (int e = 0; e < 4; ++e) c4[e] = cfg_pairs ? y[0][e] + gs * (y[1][e] - y[0][e]) : y[0][e];
       uint2 w;
       w.x = pack_bf16x2(c4[0], c4[1]);
       w.y = pack_bf16x2(c4[2], c4[3]);
@@ -480,7 +482,8 @@ __global__ void __launch_bounds__(256) qk_rmsnorm_kernel(bf16* __restrict__ qkv,
 }
 
 // unpatchify (transformer_sd3.py:377-399) + CFG combine (modeling_sd3_pnt.py:537-538) + custom_step (model_utilis.py:61-69)
-__global__ void __launch_bounds__(256) unpatchify_kernel(const float* __restrict__ pout, int B, int cfg_pairs, float guidance, int C,
+__global__ void __launch_bounds__(256) unpatchify_kernel(const float* __restrict__ pout, int B, int cfg_pairs,
+                                                         const float* __restrict__ guidance, int C,
                                                          int Hl, int Wl, float* __restrict__ velocity, float* __restrict__ latents,
                                                          const float* __restrict__ sigma, const float* __restrict__ sigma_next,
                                                          int sigma_stride, float* __restrict__ history) {
@@ -497,7 +500,7 @@ __global__ void __launch_bounds__(256) unpatchify_kernel(const float* __restrict
   float v = pout[(static_cast<long long>(b) * N + n) * (4 * C) + idx];
   if (cfg_pairs) {
     const float vc = pout[(static_cast<long long>(b + B) * N + n) * (4 * C) + idx];
-    v = v + guidance * (vc - v);
+    v = v + guidance[b] * (vc - v);
   }
   if (velocity) velocity[i] = v;
   if (latents) {
@@ -517,13 +520,18 @@ __global__ void euler_kernel(const float* __restrict__ v, const float* __restric
 }
 
 __global__ void cfg_combine_kernel(const float* __restrict__ in, float* __restrict__ out, float* __restrict__ out2, int B, int n,
-                                   float guidance) {
+                                   const float* __restrict__ guidance) {
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= static_cast<long long>(B) * n) return;
   const float u = in[i], c = in[i + static_cast<long long>(B) * n];
-  const float r = u + guidance * (c - u);
+  const float r = u + guidance[i / n] * (c - u);
   out[i] = r;
   if (out2) out2[i] = r;
+}
+
+__global__ void fill_f32_kernel(float* __restrict__ out, int n, float value) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = value;
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -838,7 +846,8 @@ __global__ void __launch_bounds__(256) sum_partials_kernel(const float* __restri
 // ---- device-side prompt queue ---------------------------------------------------------------------------------
 // schedule update per slot (modeling_sd3_pnt.py:557-590), sigma kept per slot.  predict: ratio = Beta mode.  Rollouts
 // (predict == 0): the prompt's injected ratio or a Philox draw keyed by (prompt, the slot's own trajectory step), recorded per
-// prompt and step.
+// prompt and step.  Stream mode (entry_predict set): each entry's own mode, and its draws keyed by (its seed, 0, its step), as
+// a batch-1 tpdm_sample_* keys them.
 __global__ void queue_schedule_kernel(const QueueArgs a) {
   const int i = threadIdx.x;
   if (i >= a.B) return;
@@ -850,11 +859,14 @@ __global__ void queue_schedule_kernel(const QueueArgs a) {
   }
   const int step = a.slot_step[i];
   const long long o = static_cast<long long>(prompt) * a.max_steps + step;
-  const RatioSource src = a.predict ? kRatioMode : (a.ratios_all ? kRatioGiven : kRatioDraw);
+  const bool entry = a.entry_predict != nullptr;
+  const int predict = entry ? a.entry_predict[prompt] : a.predict;
+  const RatioSource src = predict ? kRatioMode : (!entry && a.ratios_all ? kRatioGiven : kRatioDraw);
   const ScheduleStep r = schedule_step(a.alpha_beta[2 * i], a.alpha_beta[2 * i + 1], sigma, src, src == kRatioGiven ? a.ratios_all[o] : 0.f,
-                                       a.seed, prompt, step, a.prediction_type, a.relative, a.epsilon);
+                                       entry ? a.entry_seed[prompt] : a.seed, entry ? 0 : prompt, step, a.prediction_type, a.relative,
+                                       a.epsilon);
   float sigma_next = r.sigma_next;
-  if (a.predict && sigma < a.min_sigma) sigma_next = 0.f;
+  if (predict && sigma < a.min_sigma) sigma_next = 0.f;
   a.sigma_next[i] = sigma_next;
   if (a.rec_alphas) a.rec_alphas[o] = r.alpha;
   if (a.rec_betas) a.rec_betas[o] = r.beta;
@@ -886,7 +898,8 @@ __device__ __forceinline__ bool queue_slot_retires(const QueueArgs& a, int i, in
   const int step = a.slot_step[i] + 1;
   const float sn = a.sigma_next[i];
   if (a.out_sigmas) a.out_sigmas[static_cast<long long>(prompt) * (a.max_steps + 1) + step] = sn;
-  if (sn < a.min_sigma || step >= a.max_steps) {   // the prompt-level form of the batch-wide exit test (:608)
+  const int cap = a.entry_max_steps ? a.entry_max_steps[prompt] : a.max_steps;
+  if (sn < a.min_sigma || step >= cap) {   // the prompt-level form of the batch-wide exit test (:608)
     a.out_steps[prompt] = step;
     return true;
   }
@@ -972,6 +985,7 @@ __global__ void stream_advance_kernel(const QueueArgs a, int admit) {
       a.slot_prompt[i] = prompt;
       a.slot_step[i] = 0;
       a.sigma_cur[i] = 1.0f;   // sigma = ones (:508)
+      if (prompt >= 0) a.row_guidance[i] = a.entry_guidance[prompt];
       load = prompt >= 0 ? 1 : 0;
       if (prompt >= 0 && a.out_sigmas) a.out_sigmas[static_cast<long long>(prompt) * (a.max_steps + 1)] = 1.0f;
     }
@@ -991,10 +1005,17 @@ __global__ void stream_advance_kernel(const QueueArgs a, int admit) {
   }
 }
 
-__global__ void stream_publish_kernel(int* order, int* counters, int capacity, const StreamEntries e, int n) {
-  const int s = counters[kStreamSubmitted];
-  for (int k = 0; k < n; ++k) order[(s + k) % capacity] = e.id[k];
-  counters[kStreamSubmitted] = s + n;
+__global__ void stream_publish_kernel(const QueueArgs a, int* order, const StreamEntries e, int n) {
+  const int s = a.counters[kStreamSubmitted];
+  for (int k = 0; k < n; ++k) {
+    const int id = e.id[k];
+    a.entry_guidance[id] = e.guidance[k];
+    a.entry_max_steps[id] = e.max_steps[k];
+    a.entry_predict[id] = e.predict[k];
+    a.entry_seed[id] = e.seed[k];
+    order[(s + k) % a.capacity] = id;
+  }
+  a.counters[kStreamSubmitted] = s + n;
 }
 
 __global__ void __launch_bounds__(256) queue_move_kernel(const int* __restrict__ slot_prompt, const int* __restrict__ slot_flush,
@@ -1284,7 +1305,7 @@ int k_ln_modulate(const LnSeg* segs, int nseg, int D, cudaStream_t s) {
 }
 
 int k_norm_out(const float* x, bf16* xn, const float* shift, const float* scale, int mod_stride, int B, int cfg_pairs, int N, int D,
-               int g, float guidance, bf16* tpm_x, float* h2_out, cudaStream_t s) {
+               int g, const float* guidance, bf16* tpm_x, float* h2_out, cudaStream_t s) {
   norm_out_kernel<<<blocks_for(static_cast<long long>(B) * N, 8), 256, 0, s>>>(x, xn, shift, scale, mod_stride, B, cfg_pairs, N, D, g,
                                                                                guidance, tpm_x, h2_out);
   count_launch();
@@ -1300,7 +1321,7 @@ int k_qk_rmsnorm(bf16* qkv, int Bt, int S, int row0, int rows, int H, int dp, in
   return 0;
 }
 
-int k_unpatchify(const float* pout, int B, int cfg_pairs, float guidance, int C, int Hl, int Wl, float* velocity, float* latents,
+int k_unpatchify(const float* pout, int B, int cfg_pairs, const float* guidance, int C, int Hl, int Wl, float* velocity, float* latents,
                  const float* sigma, const float* sigma_next, int sigma_stride, float* history, cudaStream_t s) {
   const long long total = static_cast<long long>(B) * C * Hl * Wl;
   unpatchify_kernel<<<blocks_for(total, 256), 256, 0, s>>>(pout, B, cfg_pairs, guidance, C, Hl, Wl, velocity, latents, sigma, sigma_next,
@@ -1318,8 +1339,15 @@ int k_euler(const float* v, const float* sigma_next, const float* sigma, const f
   return 0;
 }
 
-int k_cfg_combine(const float* in, float* out, float* out2, int B, int n, float guidance, cudaStream_t s) {
+int k_cfg_combine(const float* in, float* out, float* out2, int B, int n, const float* guidance, cudaStream_t s) {
   cfg_combine_kernel<<<blocks_for(static_cast<long long>(B) * n, 256), 256, 0, s>>>(in, out, out2, B, n, guidance);
+  count_launch();
+  TPDM_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+
+int k_fill_f32(float* out, int n, float value, cudaStream_t s) {
+  fill_f32_kernel<<<blocks_for(n, 256), 256, 0, s>>>(out, n, value);
   count_launch();
   TPDM_CUDA_OK(cudaGetLastError());
   return 0;
@@ -1397,16 +1425,19 @@ int k_queue_advance(const QueueArgs& a, cudaStream_t s) {
 
 int k_stream_advance(const QueueArgs& a, int admit, cudaStream_t s) {
   TPDM_CHECK(a.B <= 1024, TPDM_ERR_SHAPE, "queue: %d slots > 1024", a.B);
-  TPDM_CHECK(a.counters && a.done_log && a.order && a.capacity > 0, TPDM_ERR_STATE, "stream_advance: the plan has no open stream");
+  TPDM_CHECK(a.counters && a.done_log && a.order && a.capacity > 0 && a.entry_guidance && a.row_guidance, TPDM_ERR_STATE,
+             "stream_advance: the plan has no open stream");
   stream_advance_kernel<<<1, ((a.B + 31) / 32) * 32, 0, s>>>(a, admit);
   count_launch();
   TPDM_CUDA_OK(cudaGetLastError());
   return 0;
 }
 
-int k_stream_publish(int* order, int* counters, int capacity, const StreamEntries& e, int n, cudaStream_t s) {
+int k_stream_publish(const QueueArgs& a, int* order, const StreamEntries& e, int n, cudaStream_t s) {
   TPDM_CHECK(n >= 0 && n <= kStreamPublishMax, TPDM_ERR_ARG, "stream_publish: %d entries per launch (at most %d)", n, kStreamPublishMax);
-  stream_publish_kernel<<<1, 1, 0, s>>>(order, counters, capacity, e, n);
+  TPDM_CHECK(a.counters && order && a.entry_guidance && a.entry_max_steps && a.entry_predict && a.entry_seed, TPDM_ERR_STATE,
+             "stream_publish: the plan has no open stream");
+  stream_publish_kernel<<<1, 1, 0, s>>>(a, order, e, n);
   count_launch();
   TPDM_CUDA_OK(cudaGetLastError());
   return 0;

@@ -40,25 +40,27 @@ int k_ln_modulate(const LnSeg* segs, int nseg, int D, cudaStream_t s);
 int k_quantize_fp8_rows(const float* x, int rows, int K, uint8_t* codes, float* scales, cudaStream_t s);
 
 // norm_out for the sampling loop: LN-modulate both CFG halves (bf16 -> xn for proj_out) and write
-// h2 = u + guidance*(c - u), scrambled to pixel order, into tpm_x[bl][pix][D:2D];  optional fp32 h2 [2B][N][D]
+// h2 = u + guidance[bl]*(c - u), scrambled to pixel order, into tpm_x[bl][pix][D:2D];  optional fp32 h2 [2B][N][D]
 int k_norm_out(const float* x, bf16* xn, const float* shift, const float* scale, int mod_stride, int B, int cfg_pairs, int N,
-               int D, int g, float guidance, bf16* tpm_x, float* h2_out, cudaStream_t s);
+               int D, int g, const float* guidance, bf16* tpm_x, float* h2_out, cudaStream_t s);
 
 // in-place RMSNorm(eps 1e-6) of the q and k head vectors of tokens [row0, row0+rows) in qkv [Bt][S][3*H*dp]
 int k_qk_rmsnorm(bf16* qkv, int Bt, int S, int row0, int rows, int H, int dp, int d, const float* wq, const float* wk,
                  cudaStream_t s);
 
-// pout [Bt][N][4*C] -> velocity [B][C][Hl][Wl] (CFG-combined when cfg_pairs), optional Euler update of latents:
+// pout [Bt][N][4*C] -> velocity [B][C][Hl][Wl] (CFG-combined with guidance[b] when cfg_pairs), optional Euler update of latents:
 //   latents += (sigma_next - sigma) * v ; history (optional) gets the updated latents
-int k_unpatchify(const float* pout, int B, int cfg_pairs, float guidance, int C, int Hl, int Wl, float* velocity,
+int k_unpatchify(const float* pout, int B, int cfg_pairs, const float* guidance, int C, int Hl, int Wl, float* velocity,
                  float* latents, const float* sigma, const float* sigma_next, int sigma_stride, float* history,
                  cudaStream_t s);
 
 int k_euler(const float* v, const float* sigma_next, const float* sigma, const float* sample, float* prev, int B, long long n,
             cudaStream_t s);
 
-// out[b] = u[b] + guidance * (c[b] - u[b]) for [B][n] halves of in [2B][n]; also copied to out2 when non-null
-int k_cfg_combine(const float* in, float* out, float* out2, int B, int n, float guidance, cudaStream_t s);
+// out[b] = u[b] + guidance[b] * (c[b] - u[b]) for [B][n] halves of in [2B][n]; also copied to out2 when non-null
+int k_cfg_combine(const float* in, float* out, float* out2, int B, int n, const float* guidance, cudaStream_t s);
+// out[0, n) = value (stream-ordered, graph-safe)
+int k_fill_f32(float* out, int n, float value, cudaStream_t s);
 
 // ---- TimePredictor pieces ----
 int k_nchw_to_nhwc_bf16(const float* x, bf16* out, int B, int C, int g, cudaStream_t s);
@@ -118,6 +120,14 @@ struct QueueArgs {
   int* counters;
   int* done_log;
   int capacity;
+  // per-entry request options [capacity] (stream mode; null otherwise): guidance, step cap, predict and Philox seed.  When set,
+  // they replace the queue-wide max_steps / predict / seed, and a slot that claims an entry copies its guidance to
+  // row_guidance [B], the per-row guidance the CFG kernels read.
+  float* entry_guidance;
+  int* entry_max_steps;
+  int* entry_predict;
+  unsigned long long* entry_seed;
+  float* row_guidance;
 };
 enum StreamCounter { kStreamSubmitted = 0, kStreamClaimed, kStreamCompleted, kStreamExecuted, kStreamCounters };
 int k_queue_schedule(const QueueArgs& a, cudaStream_t s);
@@ -125,12 +135,18 @@ int k_queue_advance(const QueueArgs& a, cudaStream_t s);
 // stream mode: retire finished slots into the completion log, then every slot without a prompt (finished now or idle before)
 // claims the next submitted ticket in slot order.  admit = 1: no step ran (after an admission): only idle slots claim.
 int k_stream_advance(const QueueArgs& a, int admit, cudaStream_t s);
-// order[(submitted + k) % capacity] = entries[k] for k < n, then submitted += n (one thread, stream-ordered)
+// entry_*[id[k]] = the options of entry k and order[(submitted + k) % capacity] = id[k] for k < n (order: the ring a.order
+// points to), then submitted += n (one
+// thread, stream-ordered; the options travel in the kernel's parameters, 24 bytes per entry)
 constexpr int kStreamPublishMax = 64;
 struct StreamEntries {
   int id[kStreamPublishMax];
+  float guidance[kStreamPublishMax];
+  int max_steps[kStreamPublishMax];
+  int predict[kStreamPublishMax];
+  unsigned long long seed[kStreamPublishMax];
 };
-int k_stream_publish(int* order, int* counters, int capacity, const StreamEntries& e, int n, cudaStream_t s);
+int k_stream_publish(const QueueArgs& a, int* order, const StreamEntries& e, int n, cudaStream_t s);
 // per occupied slot b at (prompt, step) = (slot_prompt[b], slot_step[b]): tembs_all[prompt][step] = temb_cfg[b] ([D]) and
 // tpm_all[prompt][step] = tpm_x[b] (tpm_elems bf16); either destination may be null
 int k_queue_record(const int* slot_prompt, const int* slot_step, int B, int max_steps, int D, const float* temb_cfg, float* tembs_all,

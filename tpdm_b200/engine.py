@@ -6,6 +6,7 @@ from __future__ import annotations
 
 import collections
 import ctypes as C
+import math
 import os
 import weakref
 from typing import Dict, Optional, Tuple
@@ -641,14 +642,16 @@ class Engine:
         yet collected, prompts submitted while it runs.  The stream owns a private plan (outside ``self.plans``) and CUDA stream,
         so ``sample``, ``sample_queue`` and ``mmdit_forward`` calls on this engine stay independent of it.  ``latent`` is the
         latent side, ``n_text`` the text length every prompt must have; ``prepare_latents(n, generator, dtype)`` draws latents for
-        a ``submit`` without them."""
+        a ``submit`` without them.  ``guidance_scale`` and ``max_inference_steps`` are the defaults of a request submitted
+        without its own, and ``max_inference_steps`` bounds every request's step cap."""
         return PromptStream(self, slots, capacity, max_inference_steps, guidance_scale, use_graph, latent, n_text, prepare_latents)
 
 
 class PromptStream:
     """Continuous batching for serving: ``submit`` admits prompts into the running queue, ``step`` runs denoising steps (every slot
     whose trajectory ends takes the next submitted prompt on the device), ``results`` returns the requests that finished.  Each
-    request gets what batch-1 ``forward(predict=True)`` gives it.  Everything runs on the stream's own CUDA stream; the host
+    request has its own guidance scale, step cap and schedule mode (the Beta mode, or Beta draws from its own seed) and gets what
+    batch-1 ``forward`` with those options gives it; requests with different options share the slots and the one captured step.  Everything runs on the stream's own CUDA stream; the host
     looks at the device counters one step late, so it never stalls the device while prompts are in flight.  The stream reads the
     engine's packed weights: a TimePredictor refresh (``Engine.refresh_time_predictor``, which ``get_engine`` makes after an
     optimizer step) raises RuntimeError while requests are in flight, and is ordered against the stream's steps otherwise."""
@@ -662,6 +665,7 @@ class PromptStream:
         lib = L.load()
         dev = engine.device
         self.engine, self.slots, self.capacity, self.max_steps, self.latent, self.n_text = engine, slots, capacity, max_steps, latent, n_text
+        self.guidance_scale = float(guidance_scale)
         self._prepare_latents = prepare_latents
         self._step_fn = lib.tpdm_queue_step_graph if use_graph else lib.tpdm_queue_step
         with torch.cuda.device(dev):
@@ -674,8 +678,9 @@ class PromptStream:
                 L.check(lib.tpdm_stream_open(self._plan.handle, capacity, float(guidance_scale), base, nbytes, L.stream_ptr()))
             self._open = True
             engine._streams.add(self)
-            ptrs = [L.vp() for _ in range(5)]
-            L.check(lib.tpdm_stream_status(self._plan.handle, *[C.byref(p) for p in ptrs]))
+            ptrs = [L.vp() for _ in range(8)]
+            L.check(lib.tpdm_stream_status(self._plan.handle, *[C.byref(p) for p in ptrs[:5]]))
+            L.check(lib.tpdm_stream_records(self._plan.handle, *[C.byref(p) for p in ptrs[5:]]))
         Cc = engine.cfg["in_channels"]
         view = lambda p, dtype, shape: L.view_at(self._ws, p.value, dtype, shape)
         self._counters = view(ptrs[0], torch.int32, (6,))            # submitted, claimed, completed, executed, active, skip flag
@@ -683,6 +688,7 @@ class PromptStream:
         self._out_lat = view(ptrs[2], torch.float32, (capacity, Cc, latent, latent))
         self._out_steps = view(ptrs[3], torch.int32, (capacity,))
         self._out_sig = view(ptrs[4], torch.float32, (capacity, max_steps + 1))
+        self._records = [view(p, torch.float32, (capacity, max_steps)) for p in ptrs[5:]]     # alphas, betas, logprobs
         self._flags = _FlagReadback(6)
         self._free = list(range(capacity - 1, -1, -1))
         self._entry_req = {}                     # entry -> request id
@@ -694,10 +700,50 @@ class PromptStream:
             raise RuntimeError("the prompt stream is closed")
 
     # ---- admission ---------------------------------------------------------------------------------------------
+    def _options(self, n: int, guidance_scale, max_inference_steps, predict, seed, generator):
+        """The n requests' tpdm_request_options; ValueError for a bad value.  Unset seeds of sampled requests are drawn from
+        ``generator`` (after the latents), as ``forward`` draws its one seed."""
+        def per_prompt(name, v, default):
+            if v is None:
+                return [default] * n
+            if isinstance(v, torch.Tensor):
+                v = v.tolist() if v.dim() else v.item()
+            if isinstance(v, (list, tuple)):
+                if len(v) != n:
+                    raise ValueError(f"{name} has {len(v)} values for {n} prompts")
+                return [default if x is None else x for x in v]
+            return [v] * n
+
+        gs = [float(g) for g in per_prompt("guidance_scale", guidance_scale, self.guidance_scale)]
+        caps = [int(m) for m in per_prompt("max_inference_steps", max_inference_steps, self.max_steps)]
+        pred = [bool(x) for x in per_prompt("predict", predict, True)]
+        for g in gs:
+            if not math.isfinite(g):
+                raise ValueError(f"guidance_scale {g} is not finite")
+        for m in caps:
+            if not 1 <= m <= self.max_steps:
+                raise ValueError(f"max_inference_steps {m} outside [1, {self.max_steps}] (the stream's max_inference_steps)")
+        if seed is None and not all(pred):
+            gen = generator[0] if isinstance(generator, (list, tuple)) else generator
+            seed = torch.randint(0, 2**62, (n,), generator=gen, device=gen.device if gen is not None else "cpu").tolist()
+        seeds = [int(x) for x in per_prompt("seed", seed, 0)]
+        for x in seeds:
+            if not 0 <= x < 2**64:
+                raise ValueError(f"seed {x} outside [0, 2**64)")
+        opts = (L.TpdmRequestOptions * n)()
+        for k in range(n):
+            opts[k].guidance_scale, opts[k].max_steps, opts[k].predict, opts[k].seed = gs[k], caps[k], int(pred[k]), seeds[k]
+        return opts
+
     def submit(self, prompt_embeds, negative_prompt_embeds, pooled_prompt_embeds, negative_pooled_prompt_embeds, latents=None,
-               generator=None) -> list:
+               generator=None, *, guidance_scale=None, max_inference_steps=None, predict=True, seed=None) -> list:
         """Admit n prompts; returns their request ids (increasing).  Latents default to ``prepare_latents`` (as ``forward`` draws
-        them).  A ring without n free entries raises RuntimeError and admits nothing."""
+        them).  Request options, each one value for all n prompts or a sequence of n (None: the stream's default):
+        ``guidance_scale`` (default: the stream's), ``max_inference_steps`` (the step cap, 1 to the stream's
+        ``max_inference_steps``, which is the default), ``predict`` (True: the Beta mode; False: Beta draws keyed by ``seed``, as
+        ``forward(predict=False)`` draws them with that Philox seed) and ``seed`` (in [0, 2**64); by default drawn from
+        ``generator`` after the latents as ``torch.randint(0, 2**62, (n,))``).  A bad option raises ValueError and a ring without
+        n free entries RuntimeError; either admits nothing."""
         self._check_open()
         eng, dev, f32 = self.engine, self.engine.device, torch.float32
         n = prompt_embeds.shape[0]
@@ -717,6 +763,7 @@ class PromptStream:
             raise ValueError("submit needs at least one prompt")
         if n > len(self._free):
             raise RuntimeError(f"the prompt stream is full: {n} prompts for {len(self._free)} free entries of {self.capacity}")
+        opts = self._options(n, guidance_scale, max_inference_steps, predict, seed, generator)
         cvt = lambda t: t.to(device=dev, dtype=f32).contiguous()
         ts = [cvt(latents), cvt(negative_prompt_embeds), cvt(prompt_embeds), cvt(negative_pooled_prompt_embeds), cvt(pooled_prompt_embeds)]
         entries = self._free[len(self._free) - n:][::-1]       # taken off the free list only once the library accepted them
@@ -725,7 +772,7 @@ class PromptStream:
         for ev in self._freed:
             self._cs.wait_event(ev)
         with torch.cuda.device(dev), torch.cuda.stream(self._cs):
-            L.check(L.load().tpdm_stream_submit(self._plan.handle, n, ids, *[L.ptr(t) for t in ts], L.stream_ptr()))
+            L.check(L.load().tpdm_stream_submit_options(self._plan.handle, n, ids, *[L.ptr(t) for t in ts], opts, L.stream_ptr()))
         del self._free[len(self._free) - n:]
         self._freed.clear()
         for t in ts:
@@ -765,8 +812,9 @@ class PromptStream:
 
     # ---- completions -------------------------------------------------------------------------------------------
     def results(self) -> dict:
-        """``{request id: dict(latents (C, h, w), steps, sigmas (steps,))}`` of the requests finished since the last call, as far as
-        the host has seen (one step late); their entries are free again."""
+        """``{request id: dict(latents (C, h, w), steps, sigmas, alphas, betas, logprobs (each (steps,)))}`` of the requests
+        finished since the last call, as far as the host has seen (one step late); their entries are free again.  ``logprobs``
+        are the raw Beta log-probabilities of the ratio each step took (``forward``'s ``logprobs`` before masking)."""
         self._check_open()
         self._flags.poll()
         done = self._flags.last[2]
@@ -781,9 +829,11 @@ class PromptStream:
             steps = self._out_steps[ents].tolist()
             lat = self._out_lat[ents].clone()
             sig = self._out_sig[ents].clone()
+            rec = [r[ents].clone() for r in self._records]
         out = {}
         for j, (e, s) in enumerate(zip(ents.tolist(), steps)):
-            out[self._entry_req.pop(e)] = dict(latents=lat[j], steps=s, sigmas=sig[j, 1: s + 1])
+            out[self._entry_req.pop(e)] = dict(latents=lat[j], steps=s, sigmas=sig[j, 1: s + 1], alphas=rec[0][j, :s], betas=rec[1][j, :s],
+                                               logprobs=rec[2][j, :s])
             self._free.append(e)
         self._harvested = done
         ev = torch.cuda.Event()

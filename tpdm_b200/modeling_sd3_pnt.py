@@ -423,8 +423,11 @@ class SD3PredictNextTimeStepModel(nn.Module):
                            use_graph: bool = True, n_text: int = 333):
         """An open prompt queue for serving (engine.PromptStream): ``slots`` prompts in flight, up to ``capacity`` admitted and
         not yet collected.  ``submit`` admits prompts while it runs (latents drawn as ``forward`` draws them when not given),
-        ``step`` runs denoising steps, ``results`` returns the finished requests; each gets what ``forward(predict=True)`` with
-        batch size 1 gives it.  ``n_text`` is the text length of every prompt (333 for SD3's CLIP + T5 embeddings)."""
+        ``step`` runs denoising steps, ``results`` returns the finished requests.  Each request may bring its own
+        ``guidance_scale``, ``max_inference_steps``, ``predict`` and ``seed`` (``PromptStream.submit``) and gets what ``forward``
+        with batch size 1 and those options gives it.  ``guidance_scale`` and ``max_inference_steps`` here are the defaults of a
+        request without its own (with ``predict=True``); ``max_inference_steps`` is also the largest step cap a request may ask
+        for.  ``n_text`` is the text length of every prompt (333 for SD3's CLIP + T5 embeddings)."""
         if guidance_scale is None:
             raise ValueError("guidance_scale=None is unsupported (as in the reference, whose sigma.repeat(2) is unconditional, :526)")
         side = self.default_sample_size * self.vae_scale_factor
