@@ -466,6 +466,12 @@ int tpdm_conv3x3_wgrad(const void* dyt, const void* x_shifted_nchw, float* dw, i
 /* LayerNorm(eps 1e-6, no affine) * (1 + scale[b]) + shift[b] : x fp32 [batch][rows][D] -> bf16 */
 int tpdm_ln_modulate(const float* x, const float* shift, const float* scale, int mod_stride, void* out_bf16, int batch,
                      int rows, int D, void* stream);
+/* tpdm_ln_modulate over two segments in ONE launch, the form every MMDiT block runs for its image and text rows: segment i
+ * is x_i fp32 [batch][rows_i][D] -> out_i bf16, modulated by shift_i / scale_i (batch entry b at + b * mod_stride).  For tests of
+ * that launch; the blocks reach the same launch internally. */
+int tpdm_ln_modulate_pair(const float* x0, const float* shift0, const float* scale0, void* out0_bf16, int rows0, const float* x1,
+                          const float* shift1, const float* scale1, void* out1_bf16, int rows1, int mod_stride, int batch, int D,
+                          void* stream);
 /* E4M3 row quantization, the rounding every FP8 operand of the library uses: per row, amax = max |x|, codes =
  * cvt.rn.satfinite.e4m3(x * (448 / amax)), scale = amax / 448 (IEEE fp32 divisions), so x ~= code * scale; a zero row gets
  * scale 1 and zero codes.  x fp32 [rows][K] (K % 4 == 0) -> codes E4M3 [rows][K], scales fp32 [rows]. */

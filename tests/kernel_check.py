@@ -21,6 +21,9 @@ import torch
 # Largest observed ratio on a B200 (1000 W power limit): 1.56e-6, the conv3x3 test at g = 64, C = 3072 (K = 27648); the
 # largest GEMM ratio was 8.3e-7 (K = 6144, epi 3).  2 * 1.56e-6 = 3.1e-6 <= 2^-18 = 3.8e-6.
 TAU = 2.0 ** -18
+# LayerNorm-modulate (ln_modulate_reference), the same rule over tests/test_ln_modulate_gpu.py and test_ln_modulate: largest
+# observed ratio on a B200 (1000 W power limit) 8.3e-8, the two-segment launch at D = 2432; 2 * 8.3e-8 = 1.7e-7 <= 2^-22 = 2.4e-7.
+TAU_LN = 2.0 ** -22
 
 BF16_ROUNDING = 2.0 ** -8
 GELU_TANH_APPROX = 0.5 * 2.0 ** -10
@@ -57,6 +60,17 @@ def gemm_magnitude(A: torch.Tensor, W: torch.Tensor, bias: torch.Tensor | None =
     """M = |A| . |W|^T + |bias| in float64 (A [..., K], W [N, K])."""
     m = A.double().abs() @ W.double().abs().t()
     return m + bias.double().abs() if bias is not None else m
+
+
+def ln_modulate_reference(x: torch.Tensor, shift: torch.Tensor, scale: torch.Tensor, eps: float = 1e-6):
+    """(ref, M) in float64 for LayerNorm(x) * (1 + scale) + shift, x [B][rows][D], shift / scale [B][D]:
+    M = (|x| + |mean|) rstd |1 + scale| + |shift|, where |mean| covers the fp32 cancellation in x - mean of a row whose mean is
+    far larger than its spread."""
+    x = x.double()
+    mean = x.mean(-1, keepdim=True)
+    rstd = ((x - mean).square().mean(-1, keepdim=True) + eps).rsqrt()
+    s1, sh = 1.0 + scale.double()[:, None], shift.double()[:, None]
+    return (x - mean) * rstd * s1 + sh, (x.abs() + mean.abs()) * rstd * s1.abs() + sh.abs()
 
 
 def ratio(out: torch.Tensor, ref: torch.Tensor, mag: torch.Tensor, gelu_x: torch.Tensor | None = None) -> torch.Tensor:

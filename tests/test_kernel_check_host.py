@@ -152,3 +152,14 @@ def test_set_launch_guards_argument_errors(lib):
         with pytest.raises(ValueError, match="slots"):
             L.check(lib.tpdm_set_launch_guards(None, None, slots))
     L.check(lib.tpdm_set_launch_guards(None, None, 1))
+
+
+def test_ln_modulate_pair_argument_errors(lib):
+    from tpdm_b200 import _lib as L
+
+    p = [0x1000, 0x2000, 0x3000, 0x4000]   # never dereferenced: both calls fail their argument check first
+    with pytest.raises(ValueError, match="null"):
+        L.check(lib.tpdm_ln_modulate_pair(*p, 4, None, *p[1:], 4, 6 * 64, 1, 64, None))
+    with pytest.raises(ValueError, match="rows"):
+        L.check(lib.tpdm_ln_modulate_pair(*p, 4, *p, 0, 6 * 64, 1, 64, None))
+    assert b"tpdm_ln_modulate_pair" in lib.tpdm_last_error()

@@ -6,7 +6,8 @@ import math
 import pytest
 import torch
 
-from kernel_check import assert_launch, gemm_magnitude, guarded
+from attention_check import assert_attention, attention_out, check_attention
+from kernel_check import TAU_LN, assert_launch, gemm_magnitude, guarded, ln_modulate_reference
 
 pytestmark = pytest.mark.gpu
 
@@ -76,15 +77,7 @@ def test_joint_attention(L, Bt, S, H, d, q_rows):
     qkv = torch.zeros(Bt, S, 3, H, dp, device="cuda")
     qkv[..., :d] = torch.randn(Bt, S, 3, H, d, device="cuda") * 1.5
     qkv = qkv.bfloat16().contiguous()
-    out = torch.zeros(Bt, S, H, dp, device="cuda", dtype=torch.bfloat16)
-    q, k, v = (qkv[:, :, i, :, :d].float().transpose(1, 2) for i in range(3))
-    ref = torch.nn.functional.scaled_dot_product_attention(q, k, v).transpose(1, 2)
-    L.check(lib.tpdm_joint_attention(L.ptr(qkv), L.ptr(out), Bt, S, H, dp, d, q_rows, None))
-    torch.cuda.synchronize()
-    rows = q_rows or S
-    assert rel(out[:, :rows, :, :d], ref[:, :rows]) < 6e-3
-    if dp > d:
-        assert float(out[..., d:].float().abs().max()) == 0.0
+    check_attention(L, qkv, d, q_rows, what=f"attention Bt={Bt} S={S} H={H} d={d} q_rows={q_rows}")   # pad columns exactly 0
     # ordinary activations never leave the fast kernel (the exact kernel behind it is an empty launch)
     assert lib.tpdm_attention_redo_count() in (0, -1)
 
@@ -95,7 +88,6 @@ def test_attention_large_logits_trigger_rescale(L, jump):
     in every 32-key chunk position of a 128-key tile (chunks 0/1 are rescaled before their P is handed to the MMA warp, chunks
     2/3 after the first half of P V has been issued), in the first and in later tiles, and as a ramp that moves it many times."""
     torch.manual_seed(2)
-    lib = L.load()
     Bt, S, H, d = 1, 512, 2, 64
     qkv = torch.randn(Bt, S, 3, H, d, device="cuda")
     qkv[:, :, 0] *= 6.0
@@ -104,13 +96,7 @@ def test_attention_large_logits_trigger_rescale(L, jump):
     else:
         qkv[:, jump:, 1] *= 6.0     # later keys carry much larger logits
     qkv = qkv.bfloat16().contiguous()
-    out = torch.zeros(Bt, S, H, d, device="cuda", dtype=torch.bfloat16)
-    q, k, v = (qkv[:, :, i].float().transpose(1, 2) for i in range(3))
-    ref = torch.nn.functional.scaled_dot_product_attention(q, k, v).transpose(1, 2)
-    L.check(lib.tpdm_joint_attention(L.ptr(qkv), L.ptr(out), Bt, S, H, 64, d, 0, None))
-    torch.cuda.synchronize()
-    assert torch.isfinite(out.float()).all()
-    assert rel(out, ref) < 1e-2
+    check_attention(L, qkv, d, what=f"attention jump {jump}")
 
 
 def test_attention_extreme_logits_stay_finite(L):
@@ -122,13 +108,7 @@ def test_attention_extreme_logits_stay_finite(L):
     qkv[:, :, 0] *= 40.0
     qkv[:, :, 1] *= 40.0
     qkv = qkv.bfloat16().contiguous()
-    out = torch.zeros(Bt, S, H, d, device="cuda", dtype=torch.bfloat16)
-    q, k, v = (qkv[:, :, i].float().transpose(1, 2) for i in range(3))
-    ref = torch.nn.functional.scaled_dot_product_attention(q, k, v).transpose(1, 2)
-    L.check(lib.tpdm_joint_attention(L.ptr(qkv), L.ptr(out), Bt, S, H, 64, d, 0, None))
-    torch.cuda.synchronize()
-    assert torch.isfinite(out.float()).all()
-    assert rel(out, ref) < 1e-2
+    check_attention(L, qkv, d, what="attention +-1e4 logits")
     # scores this far apart cannot be kept in range by the row-sum guard of the fast kernel: its CTAs must have been flagged and
     # recomputed by the exact kernel (per-chunk maxima)
     n_redo = lib.tpdm_attention_redo_count()
@@ -146,15 +126,10 @@ def test_attention_row_sum_guard_moves_the_reference(L, scale_k):
     qkv[:, :, 0] = qkv[:, :, 0].abs() * 2.0                     # q >= 0 ...
     qkv[:, :, 1] = qkv[:, :, 1].abs() * torch.linspace(0.05, scale_k, S, device="cuda").view(1, S, 1, 1)   # ... k >= 0 and growing
     qkv = qkv.bfloat16().contiguous()
-    out = torch.zeros(Bt, S, H, d, device="cuda", dtype=torch.bfloat16)
-    q, k, v = (qkv[:, :, i].float().transpose(1, 2) for i in range(3))
-    ref = torch.nn.functional.scaled_dot_product_attention(q, k, v).transpose(1, 2)
+    q, k = (qkv[:, :, i].float().transpose(1, 2) for i in range(2))
     spread = (q @ k.transpose(-1, -2) * (1.4427 / 8)).amax(-1) - (q @ k[:, :, :128].transpose(-1, -2) * (1.4427 / 8)).amax(-1)
     assert float(spread.max()) > 40.0       # log2 units above the first tile's maximum: the guard has to act
-    L.check(lib.tpdm_joint_attention(L.ptr(qkv), L.ptr(out), Bt, S, H, 64, d, 0, None))
-    torch.cuda.synchronize()
-    assert torch.isfinite(out.float()).all()
-    assert rel(out, ref) < 1e-2
+    check_attention(L, qkv, d, what=f"attention row-sum guard scale_k {scale_k}")
     n_redo = lib.tpdm_attention_redo_count()
     if scale_k <= 2.0:   # the guard of the eight-softmax-warp build acts every 4th tile; faster growth takes the exact pass (still exact)
         assert n_redo in (0, -1), n_redo
@@ -173,14 +148,7 @@ def test_attention_exact_pass_only_where_needed(L, d):
     qkv[:, :, 0, 1, :d] *= 40.0
     qkv[:, :, 1, 1, :d] *= 40.0
     qkv = qkv.bfloat16().contiguous()
-    out = torch.zeros(Bt, S, H, dp, device="cuda", dtype=torch.bfloat16)
-    q, k, v = (qkv[:, :, i, :, :d].float().transpose(1, 2) for i in range(3))
-    ref = torch.nn.functional.scaled_dot_product_attention(q, k, v).transpose(1, 2)
-    L.check(lib.tpdm_joint_attention(L.ptr(qkv), L.ptr(out), Bt, S, H, dp, d, 0, None))
-    torch.cuda.synchronize()
-    assert torch.isfinite(out.float()).all()
-    for h in range(H):
-        assert rel(out[:, :, h, :d], ref[:, :, h]) < 1e-2, h
+    check_attention(L, qkv, d, what=f"attention exact pass d={d}")   # every head and element; the failing index names the head
     n_redo = lib.tpdm_attention_redo_count()
     q_tiles = (S + 127) // 128
     assert n_redo == -1 or 0 < n_redo <= Bt * q_tiles, n_redo
@@ -195,9 +163,8 @@ def test_attention_cold_cache_no_deadlock(L):
     lib = L.load()
     Bt, S, H, d = 2, 4429, 24, 64
     qkv = torch.randn(Bt, S, 3, H, d, device="cuda").bfloat16().contiguous()
-    out = torch.zeros(Bt, S, H, d, device="cuda", dtype=torch.bfloat16)
-    q, k, v = (qkv[:, :, i].float().transpose(1, 2) for i in range(3))
-    ref = torch.nn.functional.scaled_dot_product_attention(q[:1, :4], k[:1, :4], v[:1, :4]).transpose(1, 2)
+    buf, out = attention_out(Bt, S, H, d)
+    before = buf.clone()
     flush = torch.empty(512 << 20, dtype=torch.uint8, device="cuda")
     big_a = torch.empty(1 << 30, dtype=torch.uint8, device="cuda")
     big_b = torch.empty(1 << 30, dtype=torch.uint8, device="cuda")
@@ -215,7 +182,7 @@ def test_attention_cold_cache_no_deadlock(L):
             first = out.clone()
         else:
             assert torch.equal(out, first)
-    assert rel(out[:1, :, :4], ref) < 6e-3
+    assert_attention(buf, before, out, qkv, d, what="attention cold cache")   # every launch returned this output
     assert lib.tpdm_attention_redo_count() in (0, -1)
 
 
@@ -290,11 +257,12 @@ def test_ln_modulate(L):
     B, rows, D = 2, 333, 1536
     x = torch.randn(B, rows, D, device="cuda") * 3 + 1
     mod = torch.randn(B, 4 * D, device="cuda")
-    out = torch.zeros(B, rows, D, device="cuda", dtype=torch.bfloat16)
+    buf, out = guarded((B, rows, D), torch.bfloat16)
+    before = buf.clone()
     L.check(lib.tpdm_ln_modulate(L.ptr(x), mod.data_ptr(), mod.data_ptr() + 4 * D, 4 * D, L.ptr(out), B, rows, D, None))
     torch.cuda.synchronize()
-    ref = torch.nn.functional.layer_norm(x, (D,), eps=1e-6) * (1 + mod[:, None, D:2 * D]) + mod[:, None, :D]
-    assert rel(out, ref) < 4e-3
+    ref, mag = ln_modulate_reference(x, mod[:, :D], mod[:, D:2 * D])
+    assert_launch(buf, before, [(out, ref, mag, None)], TAU_LN, "ln_modulate")
 
 
 def test_euler_step_matches_reference_fixture(golden):

@@ -146,6 +146,7 @@ EXPORTS = {
     "tpdm_conv3x3_nhwc": (C.c_int, [vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
     "tpdm_conv3x3_wgrad": (C.c_int, [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
     "tpdm_ln_modulate": (C.c_int, [vp, vp, vp, C.c_int, vp, C.c_int, C.c_int, C.c_int, vp]),
+    "tpdm_ln_modulate_pair": (C.c_int, [vp, vp, vp, vp, C.c_int, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
     "tpdm_quantize_fp8_rows": (C.c_int, [vp, C.c_int, C.c_int, vp, vp, vp]),
     "tpdm_ln_modulate_fp8": (C.c_int, [vp, vp, vp, C.c_int, vp, vp, C.c_int, C.c_int, C.c_int, vp]),
     "tpdm_gemm_fp8": (C.c_int, [vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp]),

@@ -1173,6 +1173,17 @@ int tpdm_ln_modulate(const float* x, const float* shift, const float* scale, int
   return k_ln_modulate(&seg, 1, D, static_cast<cudaStream_t>(stream));
 }
 
+int tpdm_ln_modulate_pair(const float* x0, const float* shift0, const float* scale0, void* out0_bf16, int rows0, const float* x1,
+                          const float* shift1, const float* scale1, void* out1_bf16, int rows1, int mod_stride, int batch, int D,
+                          void* stream) {
+  TPDM_CHECK(x0 && shift0 && scale0 && out0_bf16 && x1 && shift1 && scale1 && out1_bf16, TPDM_ERR_ARG,
+             "tpdm_ln_modulate_pair: null argument");
+  TPDM_CHECK(rows0 > 0 && rows1 > 0 && batch > 0, TPDM_ERR_SHAPE, "tpdm_ln_modulate_pair: rows %d / %d, batch %d", rows0, rows1, batch);
+  const LnSeg seg[2] = {LnSeg{x0, reinterpret_cast<bf16*>(out0_bf16), shift0, scale0, rows0, batch, mod_stride},
+                        LnSeg{x1, reinterpret_cast<bf16*>(out1_bf16), shift1, scale1, rows1, batch, mod_stride}};
+  return k_ln_modulate(seg, 2, D, static_cast<cudaStream_t>(stream));
+}
+
 int tpdm_quantize_fp8_rows(const float* x, int rows, int K, void* codes, float* scales, void* stream) {
   TPDM_CHECK(x && codes && scales, TPDM_ERR_ARG, "tpdm_quantize_fp8_rows: null argument");
   return k_quantize_fp8_rows(x, rows, K, static_cast<uint8_t*>(codes), scales, static_cast<cudaStream_t>(stream));
